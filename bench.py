@@ -2,6 +2,7 @@
 """bench.py — DOF-steps/s of the explicit FE time step on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--refine M] [--partition slabs|blocks|metis] [--impl native|reference]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is ONE explicit time step (one pass of Dynamic_solver.py:9-34 over the whole mesh): force K.u,
@@ -13,10 +14,12 @@ north star's ">= 80 % at 8 GPUs" is quoted on; it fits one B200 (38 GB).  config
 configs[2] (m = 65, ~20 M DOF) are measured in the same run and reported under `also`; configs[4] (m = 65,
 synchronization-avoiding mode) under `sync_avoiding` for N > 1.
 
-Timing protocol: set-up, graph instantiation (done inside the library at plan finalisation) and an untimed spin-up of
->= --spin-ms of steps come first; then R >= 5 repeats of EXACTLY --steps steps, each bracketed by barrier +
-synchronize and timed with CUDA events on the plan's stream, max over ranks per repeat; `value` is the MEDIAN
-repeat (min / max reported).  Inputs are larger than L2 (see config.l2).
+Timing protocol: set-up, graph instantiation (done inside the library at plan finalisation), --warmup steps from rest
+and an untimed spin-up of >= --spin-ms of steps come first; the spin-up's steps are then undone (the warm-up's state
+is put back), and EXACTLY --steps steps are timed, as --repeats back-to-back parts (default 5), each bracketed by
+barrier + synchronize and timed with CUDA events on the plan's stream, max over ranks per part; `value` is the MEDIAN
+part's rate (min / max reported).  The timed steps thus end in the state --warmup + --steps steps from rest reach,
+which --dump-outputs DIR writes out.  Inputs are larger than L2 (see config.l2).
 
 `value`   whole-job DOF-steps/s with the state resident in HBM.
 `e2e`     the same metric through the reference-facing call saa_step_host_ex — one parallel_explicit_solver_dis_pre
@@ -46,13 +49,13 @@ import numpy as np  # noqa: E402
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=0, help="timed time steps per repeat (0: 2000 for m <= 32, 500 for m <= 80, else 100)")
-    ap.add_argument("--warmup", type=int, default=10, help="untimed steps before the spin-up")
+    ap.add_argument("--steps", type=int, default=0, help="timed time steps (0: 2000 for m <= 32, 500 for m <= 80, else 100)")
+    ap.add_argument("--warmup", type=int, default=10, help="untimed steps from rest before the timed steps")
     ap.add_argument("--refine", "--m", dest="m", type=int, default=0,
                     help="cells per unit length of the 25x1x1 beam (0: 111 = the 104 M-DOF mesh); spell it --refine under torchrun")
     ap.add_argument("--impl", default="native", choices=["native", "reference"])
-    ap.add_argument("--repeats", type=int, default=0, help="timed repeats of --steps (0: at least 5, more until ~1 s is covered, at most 200)")
-    ap.add_argument("--spin-ms", type=float, default=300.0, help="untimed spin-up of steps before the timed repeats")
+    ap.add_argument("--repeats", type=int, default=0, help="back-to-back parts the timed steps run in, each timed on its own (0: min(5, steps))")
+    ap.add_argument("--spin-ms", type=float, default=300.0, help="untimed spin-up of steps after the warm-up; the state is put back afterwards")
     ap.add_argument("--e2e-steps", type=int, default=0, help="timed host-call steps (0: 200 for m <= 32, 60 for m <= 80, else 20)")
     ap.add_argument("--launch", default="auto", choices=["auto", "per_step", "graph", "persistent"])
     ap.add_argument("--setup", default="device", choices=["device", "host"], help="where the problem is assembled")
@@ -75,6 +78,9 @@ def parse():
     ap.add_argument("--filter-size", type=int, default=25, help="n_s of the LSTM refill (Online_predictor.py:57 uses 150; shortened so "
                     "that warm-up + three refill blocks fit the bench)")
     ap.add_argument("--train-epochs", type=int, default=20)
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the state they computed (d0, dn, tn of StepPlan.get_state) to DIR/<name>.npy; "
+                         "vectors longer than 2**21 / N values are a fixed, seeded sample")
     return ap.parse_args()
 
 
@@ -281,37 +287,64 @@ def run_reference(args, emit):
 
 
 # ---- timing ------------------------------------------------------------------------------------------------------
-def time_repeats(pl, torch, stream, steps, mode, launch, barrier, max_over_ranks, repeats, spin_ms, warmup, budget_s=1.0):
-    """spin-up, then `repeats` (0: adaptive) repeats of exactly `steps` steps -> (list of ms per repeat [max over ranks],
-    kernel launches of one repeat)."""
+def time_repeats(pl, torch, stream, steps, mode, launch, barrier, max_over_ranks, repeats, spin_ms, warmup):
+    """`warmup` steps, a spin-up of >= spin_ms, the state put back to where the warm-up left it, then exactly `steps`
+    timed steps in `repeats` (0: min(5, steps)) back-to-back parts -> (ms per step of each part [max over ranks],
+    kernel launches of all parts).  The timed steps thus always continue from the warm-up's state, whatever the
+    spin-up did, and the state they leave depends on the arguments alone."""
     if warmup > 0:
         pl.step(warmup, mode, launch)
+    repeats = min(repeats or 5, steps)
+    parts = [steps // repeats + (i < steps % repeats) for i in range(repeats)]
+    d0 = torch.empty(pl.n_dof, dtype=torch.float64, device="cuda")
+    dn = torch.empty_like(d0)
+    tn = pl.get_state_dev(d0.data_ptr(), dn.data_ptr())
     pl.synchronize()
     barrier()
     t0 = time.perf_counter()
     n_spin = 0
-    while True:                                   # the same call pattern as the timed repeats
-        pl.step(steps, mode, launch)
+    while True:                                   # the same call pattern as the timed parts
+        pl.step(parts[0], mode, launch)
         pl.synchronize()
         n_spin += 1
         if max_over_ranks(1.0 if (time.perf_counter() - t0) * 1e3 >= spin_ms else 0.0) >= 1.0 or n_spin >= 10000:
             break
-    est = (time.perf_counter() - t0) / n_spin
-    if repeats <= 0:
-        repeats = int(max_over_ranks(float(min(200, max(5, int(budget_s / max(est, 1e-6)))))))
-    out, launches = [], 0
-    for _ in range(repeats):
+    pl.set_state_dev(d0.data_ptr(), dn.data_ptr(), tn)
+    del d0, dn
+    out, l0 = [], pl.kernel_launches
+    for k in parts:
         barrier()
-        l0 = pl.kernel_launches
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(stream)
-        pl.step(steps, mode, launch)
+        pl.step(k, mode, launch)
         e1.record(stream)
         pl.synchronize()
         barrier()
-        launches = pl.kernel_launches - l0
-        out.append(max_over_ranks(e0.elapsed_time(e1)))
-    return out, launches
+        out.append(max_over_ranks(e0.elapsed_time(e1)) / k)
+    return out, pl.kernel_launches - l0
+
+
+DUMP_SAMPLE = 2 ** 21   # values per vector over all ranks: d0 + dn stay at 32 MB
+
+
+def dump_outputs(pl, torch, out_dir, rank, world):
+    """What a caller of the timed steps receives (StepPlan.get_state: d0, dn, tn) as float64 .npy files in out_dir,
+    suffixed _rank<r> for N > 1.  A vector longer than DUMP_SAMPLE / N is sampled at sorted indices drawn from a
+    generator seeded with its length, so that two builds of the project write the same entries."""
+    n = pl.n_dof
+    d0 = torch.empty(n, dtype=torch.float64, device="cuda")
+    dn = torch.empty_like(d0)
+    tn = pl.get_state_dev(d0.data_ptr(), dn.data_ptr())
+    k = DUMP_SAMPLE // world
+    idx = None if n <= k else np.unique(np.random.default_rng(n).integers(0, n, k))
+    os.makedirs(out_dir, exist_ok=True)
+    sfx = f"_rank{rank}" if world > 1 else ""
+    sel = (lambda v: v) if idx is None else (lambda v: v[torch.from_numpy(idx).to(v.device)])
+    for name, v in (("d0", sel(d0)), ("dn", sel(dn))):
+        np.save(os.path.join(out_dir, f"{name}{sfx}.npy"), v.cpu().numpy())
+    np.save(os.path.join(out_dir, f"tn{sfx}.npy"), np.float64(tn))
+    return {"dir": out_dir, "files": [f"{x}{sfx}.npy" for x in ("d0", "dn", "tn")], "n_dof_rank0": n,
+            "sampled_entries": n if idx is None else int(idx.size), "sample_seed": None if idx is None else n}
 
 
 def time_host_calls(pl, torch, dist, world, mode, dt, e2e_steps, barrier, max_over_ranks, n_dof_global):
@@ -564,8 +597,8 @@ def time_sync_avoiding(args, torch, dist, world, rank, local, barrier, max_over_
                             "error_vs_sync": {"rel_l2_displacement_at_block_ends": errs,
                                               "note": "all DOFs of all ranks (shared nodes counted once per holder) vs the fully synchronised run"}})
     # fully synchronised reference speed of the same mesh in the same run
-    ms, _ = time_repeats(pl, torch, stream, 500, splan.MODE_SYNC, splan.LAUNCH_AUTO, barrier, max_over_ranks, 5, 100.0, 10)
-    out["synchronised_every_step"] = {"value": n_dof_global * 500 / (float(np.median(ms)) * 1e-3), "ms_per_step": float(np.median(ms)) / 500}
+    ms, _ = time_repeats(pl, torch, stream, 2500, splan.MODE_SYNC, splan.LAUNCH_AUTO, barrier, max_over_ranks, 5, 100.0, 10)
+    out["synchronised_every_step"] = {"value": n_dof_global / (float(np.median(ms)) * 1e-3), "ms_per_step": float(np.median(ms))}
     pl.close()
     return out
 
@@ -583,6 +616,8 @@ def main():
         print(json.dumps(line), flush=True)
 
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs: the native implementation's timed steps only")
         run_reference(args, emit)
         return
     import torch
@@ -646,7 +681,7 @@ def main():
         if world > 1 and args.balance and args.partition == "slabs":
             from saa_b200 import device_setup
             st0 = torch.cuda.ExternalStream(pl.stream, device=torch.device("cuda", local))
-            ms0, _ = time_repeats(pl, torch, st0, 100, splan.MODE_LOCAL, splan.LAUNCH_AUTO, lambda: torch.cuda.synchronize(),
+            ms0, _ = time_repeats(pl, torch, st0, 300, splan.MODE_LOCAL, splan.LAUNCH_AUTO, lambda: torch.cuda.synchronize(),
                                   lambda x: float(x), 3, 50.0, 10)
             speed = torch.tensor([pl.n_dof / float(np.median(ms0))], dtype=torch.float64, device="cuda")
             allv = [torch.zeros_like(speed) for _ in range(world)]
@@ -697,10 +732,11 @@ def main():
     sampler = ClockSampler(local) if rank == 0 else None
     reps, launches = time_repeats(pl, torch, stream, steps, mode, launch, barrier, max_over_ranks, args.repeats, args.spin_ms, args.warmup)
     ms = float(np.median(reps))
+    dumped = dump_outputs(pl, torch, args.dump_outputs, rank, world) if args.dump_outputs else None
     ms_local = None
     if world > 1:   # the same shards stepped WITHOUT the exchange (MODEL=True arithmetic): what the halo costs per step
-        rl, _ = time_repeats(pl, torch, stream, steps, splan.MODE_LOCAL, launch, barrier, max_over_ranks, 5, 50.0, 0)
-        ms_local = float(np.median(rl)) / steps
+        rl, _ = time_repeats(pl, torch, stream, 5 * steps, splan.MODE_LOCAL, launch, barrier, max_over_ranks, 5, 50.0, 0)
+        ms_local = float(np.median(rl))
 
     # ---- end to end through the reference-facing host call -----------------------------------------
     e2e = time_host_calls(pl, torch, dist, world, mode, dtv, e2e_steps, barrier, max_over_ranks, n_dof_global)
@@ -718,7 +754,7 @@ def main():
     nnz = pl.nnz
     alg_bytes = max_over_ranks(float((pl.matfree_bytes if matfree else pl.matrix_bytes) + pl.vector_bytes))
     csr_bytes = max_over_ranks(float(nnz * 12 + (n_dof_local + 1) * 4 + 5 * 8 * n_dof_local))
-    step_s = ms * 1e-3 / steps
+    step_s = ms * 1e-3
     peak, peak_src = measured_peak()
     achieved = alg_bytes / step_s / 1e9
     traffic, traffic_src = None, None
@@ -749,14 +785,14 @@ def main():
                     multi.attach_transport(pl2, args.transport)
                 st2 = torch.cuda.ExternalStream(pl2.stream, device=torch.device("cuda", local))
                 md2 = splan.MODE_SYNC if w2 > 1 else splan.MODE_LOCAL
-                r2, _ = time_repeats(pl2, torch, st2, k2, md2, launch, barrier, max_over_ranks, 5, 200.0, 10)
+                r2, _ = time_repeats(pl2, torch, st2, 5 * k2, md2, launch, barrier, max_over_ranks, 5, 200.0, 10)
                 ms2 = float(np.median(r2))
                 b2 = max_over_ranks(float(pl2.matrix_bytes + pl2.vector_bytes))
                 e2 = time_host_calls(pl2, torch, dist, w2, md2, info2["dt"], 200 if m2 <= 32 else 60, barrier, max_over_ranks, 3 * info2["n_nodes"])
                 also.append({"workload": workload_name(m2, 3 * info2["n_nodes"], info2["n_elem"]), "n_gpus": w2, "steps": k2, "repeats": len(r2),
-                             "value": 3 * info2["n_nodes"] * k2 / (ms2 * 1e-3), "ms_per_step": ms2 / k2,
-                             "ms_per_step_min": min(r2) / k2, "ms_per_step_max": max(r2) / k2,
-                             "roofline_frac": b2 / (ms2 / k2 * 1e-3) / 1e9 / peak, "nnz_per_row": pl2.nnz / pl2.n_dof, "e2e": e2})
+                             "value": 3 * info2["n_nodes"] / (ms2 * 1e-3), "ms_per_step": ms2,
+                             "ms_per_step_min": min(r2), "ms_per_step_max": max(r2),
+                             "roofline_frac": b2 / (ms2 * 1e-3) / 1e9 / peak, "nnz_per_row": pl2.nnz / pl2.n_dof, "e2e": e2})
                 pl2.close()
                 del pl2
                 torch.cuda.empty_cache()
@@ -774,11 +810,12 @@ def main():
 
     if rank == 0:
         line = {
-            "metric": "DOF-steps/sec", "value": n_dof_global * steps / (ms * 1e-3), "unit": "DOF-steps/s",
-            "n_gpus": world, "steps": steps, "warmup": args.warmup, "ms_per_step": ms / steps,
+            "metric": "DOF-steps/sec", "value": n_dof_global / (ms * 1e-3), "unit": "DOF-steps/s",
+            "n_gpus": world, "steps": steps, "warmup": args.warmup, "ms_per_step": ms,
             "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
-            "timing": {"repeats": len(reps), "statistic": "median over repeats of `steps` steps, each repeat = max over ranks of CUDA-event time",
-                       "ms_per_step_min": min(reps) / steps, "ms_per_step_max": max(reps) / steps,
+            "timing": {"repeats": len(reps), "statistic": "median over the `repeats` back-to-back parts of the `steps` timed steps of ms per "
+                                                          "step, each part = max over ranks of CUDA-event time",
+                       "ms_per_step_min": min(reps), "ms_per_step_max": max(reps),
                        "spin_up_ms": args.spin_ms, "graphs": "instantiated at plan finalisation / transport attach, before any timing"},
             "config": {"workload": workload_name(m, n_dof_global, info["n_elem"]),
                        "partition": info["part"], "neighbours_rank0": nb_cnt, "shared_nodes_rank0": sh_cnt,
@@ -805,6 +842,8 @@ def main():
         if matfree:
             line["matfree"] = matfree
             line["config"]["kernel"] = "matfree (K5) — NOT the parity path; see line['matfree'].rel_l2_vs_assembled"
+        if dumped is not None:
+            line["dumped_outputs"] = dumped
         if parity is not None:
             line["parity"] = parity
         if also is not None:

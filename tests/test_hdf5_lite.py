@@ -1,9 +1,10 @@
 """hdf5_lite — the dependency-free HDF5 behind the result files (Data_prepare.py:243-246, Shared_extraction.py:32-40,
 Tools/DNN_tools.py:286-287) where h5py is not installed.
 
-Anchor: a file written by the HDF5 library itself — scipy ships MATLAB 7.3 test data, which is HDF5 behind a 512-byte
-user block.  The reader must decode it; the writer's structures are compared with that file's bytes one by one, checked
-against the consistency rules the library applies when it opens a file, and round-tripped through the reader."""
+Anchor: a file written by the HDF5 library itself — tests/golden/testhdf5_7.4_GLNX86.mat, MATLAB 7.3 test data from
+scipy's test suite (scipy/io/matlab/tests/data, BSD-licensed), which is HDF5 behind a 512-byte user block.  The reader
+must decode it; the writer's structures are compared with that file's bytes one by one, checked against the consistency
+rules the library applies when it opens a file, and round-tripped through the reader."""
 import os
 import struct
 import sys
@@ -14,17 +15,13 @@ import pytest
 
 import saa_b200  # noqa: F401
 from saa_b200 import hdf5_lite as h5
-from util import ROOT, bits_equal
+from util import GOLDEN, ROOT, bits_equal
 
 PKG = os.path.join(ROOT, "synchronization-avoiding-algorithms_b200")
 
 
 def _genuine():
-    import scipy.io
-    p = os.path.join(os.path.dirname(scipy.io.__file__), "matlab", "tests", "data", "testhdf5_7.4_GLNX86.mat")
-    if not os.path.isfile(p):
-        pytest.skip("scipy's MATLAB 7.3 (HDF5) test file is not installed")
-    return p
+    return os.path.join(GOLDEN, "testhdf5_7.4_GLNX86.mat")
 
 
 def _messages(buf, addr):

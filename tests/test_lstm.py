@@ -224,7 +224,8 @@ def test_reference_shared_extraction_script_runs_unchanged_on_this_package(tmp_p
     write_result(tmp_path / "Results" / "Dynamics" / "Local-rank-0.hdf5", D)
     env = dict(os.environ)
     env.pop("PYTHONPATH", None)
-    r = subprocess.run([sys.executable, os.path.join(PKG, "run_driver.py"), "/root/reference/Shared_extraction.py"], cwd=str(tmp_path),
+    script = os.path.join(os.environ["SAA_REFERENCE_ROOT"], "Shared_extraction.py")
+    r = subprocess.run([sys.executable, os.path.join(PKG, "run_driver.py"), script], cwd=str(tmp_path),
                        env=env, capture_output=True, text=True, timeout=300)
     assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
     out = read_result(tmp_path / "Results" / "sol_on_shared" / "rank=0-shared_dof.hdf5")
