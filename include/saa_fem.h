@@ -140,7 +140,8 @@ int saa_plan_destroy(saa_plan *plan);
 /* sizes / layout facts, e.g. for the roofline arithmetic of bench.py */
 int64_t saa_plan_n_dof(const saa_plan *plan);
 int64_t saa_plan_nnz(const saa_plan *plan);           /* stored entries of LocalK                         */
-int64_t saa_plan_padded_entries(const saa_plan *plan);/* entries streamed per step incl. slice padding    */
+int64_t saa_plan_padded_entries(const saa_plan *plan);/* 9 x block-lanes: entries of the 3x3 blocks incl. slice padding */
+int64_t saa_plan_value_planes(const saa_plan *plan);  /* value planes stored (32 fp64 each; at most padded_entries / 32) */
 int64_t saa_plan_kernel_launches(const saa_plan *plan);/* kernels launched by this plan so far            */
 int64_t saa_plan_matrix_bytes(const saa_plan *plan);  /* bytes of matrix storage streamed per step        */
 int64_t saa_plan_vector_bytes(const saa_plan *plan);  /* bytes of the vector streams of one step (d0, dn, d1, F, M; padded rows) */

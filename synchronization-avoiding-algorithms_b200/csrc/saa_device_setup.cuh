@@ -80,9 +80,42 @@ __global__ void saa_k_fin_slice_len(int64_t n_slices, const int32_t *__restrict_
     }
     cnt[s] = 32 * (int64_t)mx;
 }
-// one warp per slice: every lane writes the blocks of its node (stored order of each row kept), then pads with
+// one warp per slice: stored planes of every block-row = the union of the stored patterns of the 32 lanes (the pattern,
+// not the value bits, so that an explicitly stored 0.0 is kept; full: all nine planes), and the doubles the slice
+// takes in val
+__global__ void saa_k_fin_pmask(int64_t n_slices, const int64_t *__restrict__ slice_ptr, const int32_t *__restrict__ permn,
+                                const int64_t *__restrict__ indptr, const int32_t *__restrict__ indices, int full,
+                                uint16_t *__restrict__ pmask, int64_t *__restrict__ slice_vals)
+{
+    const int lane = threadIdx.x & 31;
+    const int64_t s = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (s >= n_slices) return;
+    const int64_t beg = slice_ptr[s];
+    const int L = (int)((slice_ptr[s + 1] - beg) >> 5);
+    const int32_t e = permn[s * 32 + lane];
+    SaaRowTriple t(indptr, e >= 0 ? e : 0);
+    int64_t planes = 0;
+    for (int j = 0; j < L; ++j) {
+        unsigned bits = 0;
+        if (e >= 0) {
+            const int32_t cn = t.next_col_node(indices);
+            if (cn != INT32_MAX)
+                for (int A = 0; A < 3; ++A)
+                    while (t.q[A] < t.qe[A] && indices[t.q[A]] / 3 == cn) {
+                        bits |= 1u << (3 * A + indices[t.q[A]] % 3);
+                        ++t.q[A];
+                    }
+        }
+        bits = full ? 0x1FFu : __reduce_or_sync(0xffffffffu, bits);
+        if (lane == 0) pmask[(beg >> 5) + j] = (uint16_t)bits;
+        planes += __popc(bits);
+    }
+    if (lane == 0) slice_vals[s] = 32 * planes;
+}
+// one warp per slice: every lane writes the stored planes of its blocks (stored order of each row kept), then pads with
 // blocks 0.0 * d0[own node]
-__global__ void saa_k_fin_fill(int64_t n_slices, const int64_t *__restrict__ slice_ptr, const int32_t *__restrict__ permn,
+__global__ void saa_k_fin_fill(int64_t n_slices, const int64_t *__restrict__ slice_ptr, const int64_t *__restrict__ val_ptr,
+                               const uint16_t *__restrict__ pmask, const int32_t *__restrict__ permn,
                                const int32_t *__restrict__ iperm, const int64_t *__restrict__ indptr,
                                const int32_t *__restrict__ indices, const double *__restrict__ data, double *__restrict__ val,
                                int32_t *__restrict__ col)
@@ -92,10 +125,18 @@ __global__ void saa_k_fin_fill(int64_t n_slices, const int64_t *__restrict__ sli
     if (s >= n_slices) return;
     const int64_t beg = slice_ptr[s];
     const int L = (int)((slice_ptr[s + 1] - beg) >> 5);
-    double *vs = val + 9 * beg + lane;
+    double *vs = val + val_ptr[s] + lane;
+    const uint16_t *ms = pmask + (beg >> 5);
     int32_t *cs = col + beg + lane;
     const int64_t inode = s * 32 + lane;
     const int32_t e = permn[inode];
+    int64_t off = 0;                                   // planes stored for the blocks before j
+    auto store = [&](int j, const double (&a)[9]) {
+        const unsigned m = ms[j];
+        for (int k = 0; k < 9; ++k)
+            if (m & (1u << k)) vs[32 * (off + __popc(m & ((1u << k) - 1u)))] = a[k];
+        off += __popc(m);
+    };
     int j = 0;
     if (e >= 0) {
         SaaRowTriple t(indptr, e);
@@ -109,12 +150,13 @@ __global__ void saa_k_fin_fill(int64_t n_slices, const int64_t *__restrict__ sli
                     a[3 * A + indices[t.q[A]] % 3] = data[t.q[A]];
                     ++t.q[A];
                 }
-            for (int k = 0; k < 9; ++k) vs[32 * (9 * (int64_t)j + k)] = a[k];
+            store(j, a);
             cs[32 * (int64_t)j] = iperm[3 * (int64_t)cn] / 3;
         }
     }
+    const double z[9] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
     for (; j < L; ++j) {
-        for (int k = 0; k < 9; ++k) vs[32 * (9 * (int64_t)j + k)] = 0.0;
+        store(j, z);
         cs[32 * (int64_t)j] = (int32_t)inode;
     }
 }
@@ -244,11 +286,20 @@ static int finalize_device(saa_plan *p)
     CK(cudaMemcpy(&lanes, p->d_slice_ptr + p->n_slices, sizeof(int64_t), cudaMemcpyDeviceToHost));
     p->padded_entries = 9 * lanes;
 
-    // 5. matrix in node-block sliced-ELL order, vectors, Dirichlet mask
-    CK(cudaMalloc((void **)&p->d_val, std::max<int64_t>(9 * lanes, 1) * sizeof(double)));
+    // 5. plane masks and value offsets; matrix in plane-masked node-block sliced-ELL order (val allocated at its exact
+    //    size), vectors, Dirichlet mask
+    CK(cudaMalloc((void **)&p->d_pmask, std::max<int64_t>(lanes / 32, 1) * sizeof(uint16_t)));
+    saa_k_fin_pmask<<<nblk(p->n_slices, 8), 256>>>(p->n_slices, p->d_slice_ptr, permn, p->in_indptr, p->in_indices,
+                                                   p->plane_mask ? 0 : 1, p->d_pmask, cnt);   // cnt[n_slices] is still 0
+    CK(cudaMalloc((void **)&p->d_val_ptr, (p->n_slices + 1) * sizeof(int64_t)));
+    thrust::exclusive_scan(thrust::device, cnt, cnt + p->n_slices + 1, p->d_val_ptr);
+    int64_t n_val = 0;
+    CK(cudaMemcpy(&n_val, p->d_val_ptr + p->n_slices, sizeof(int64_t), cudaMemcpyDeviceToHost));
+    p->value_planes = n_val / 32;
+    CK(cudaMalloc((void **)&p->d_val, std::max<int64_t>(n_val, 1) * sizeof(double)));
     CK(cudaMalloc((void **)&p->d_col, std::max<int64_t>(lanes, 1) * sizeof(int32_t)));
-    saa_k_fin_fill<<<nblk(p->n_slices, 8), 256>>>(p->n_slices, p->d_slice_ptr, permn, p->d_iperm, p->in_indptr, p->in_indices,
-                                                  p->in_data, p->d_val, p->d_col);
+    saa_k_fin_fill<<<nblk(p->n_slices, 8), 256>>>(p->n_slices, p->d_slice_ptr, p->d_val_ptr, p->d_pmask, permn, p->d_iperm,
+                                                  p->in_indptr, p->in_indices, p->in_data, p->d_val, p->d_col);
     CK(cudaMalloc((void **)&p->d_M, p->n_rows * sizeof(double)));
     CK(cudaMalloc((void **)&p->d_F, p->n_rows * sizeof(double)));
     saa_k_fin_vectors<<<nblk(p->n_rows, 256), 256>>>(p->n_rows, permn, p->in_M, p->in_F, p->d_M, p->d_F);

@@ -110,12 +110,15 @@ struct saa_plan {
     std::vector<int32_t> nb_rank, holders_rank;
     // layout
     int64_t nnz = 0, padded_entries = 0, n_rows = 0, n_slices = 0, sh_slices = 0;
+    int64_t value_planes = 0;              // stored value planes (32 fp64 each)
+    bool plane_mask = true;                // false: all nine planes of every block stored (SAA_PLANE_MASK=0, or the cp.async variant)
     std::vector<int32_t> iperm_h;          // external local DOF -> internal row
     std::vector<int32_t> node_order;       // optional base order of the nodes (saa_plan_set_node_order); empty = ascending
     // device
     SaaDev D{};
     SaaHaloDev H{};
-    int64_t *d_slice_ptr = nullptr;
+    int64_t *d_slice_ptr = nullptr, *d_val_ptr = nullptr;
+    uint16_t *d_pmask = nullptr;
     double *d_val = nullptr, *d_M = nullptr, *d_F = nullptr;
     int32_t *d_col = nullptr, *d_iperm = nullptr;
     uint32_t *d_dir = nullptr;
@@ -323,6 +326,12 @@ extern "C" int saa_plan_finalize(saa_plan *p)
 {
     if (!p) return fail("saa_plan_finalize: null plan");
     if (p->finalized) return 0;
+    if (const char *kv = getenv("SAA_KVARIANT")) p->kvariant = atoi(kv);
+    {   // value planes that are zero in every lane of a slice are not stored (SAA_PLANE_MASK=0 stores all nine); the
+        // cp.async variant walks the values by block-row arithmetic and gets the full-plane layout
+        const char *pm = getenv("SAA_PLANE_MASK");
+        p->plane_mask = !(pm && pm[0] == '0') && p->kvariant < 6;
+    }
     if (p->dev_input) return finalize_device(p);
     CK(cudaSetDevice(p->device));
     const int64_t n = p->n_dof, nn = n / 3;
@@ -386,7 +395,7 @@ extern "C" int saa_plan_finalize(saa_plan *p)
         if (permn[i] >= 0)
             for (int c = 0; c < 3; ++c) p->iperm_h[3 * permn[i] + c] = (int32_t)(3 * i + c);
 
-    // 3. node-block sliced ELL
+    // 3. plane-masked node-block sliced ELL
     std::vector<int64_t> slice_ptr(p->n_slices + 1, 0);
     for (int64_t s = 0; s < p->n_slices; ++s) {
         int32_t mx = 0;
@@ -398,11 +407,26 @@ extern "C" int saa_plan_finalize(saa_plan *p)
     }
     const int64_t lanes = slice_ptr[p->n_slices];
     p->padded_entries = 9 * lanes;
-    std::vector<double> val((size_t)(9 * lanes), 0.0);
+    // visits the stored entries of node e in stored order: fn(block j, plane 3A+B, entry k)
+    auto for_each_entry = [&](int64_t e, auto &&fn) {
+        int32_t q[3] = {p->indptr[3 * e], p->indptr[3 * e + 1], p->indptr[3 * e + 2]};
+        const int32_t qe[3] = {p->indptr[3 * e + 1], p->indptr[3 * e + 2], p->indptr[3 * e + 3]};
+        for (int64_t j = 0; j < nblk[e]; ++j) {
+            const int32_t cn = bcol[bptr[e] + j];
+            for (int A = 0; A < 3; ++A)
+                while (q[A] < qe[A] && p->indices[q[A]] / 3 == cn) {
+                    fn(j, 3 * A + p->indices[q[A]] % 3, q[A]);
+                    ++q[A];
+                }
+        }
+    };
+    // stored planes of every block-row: the union of the stored patterns of its 32 lanes (the pattern, not the value
+    // bits, so that an explicitly stored 0.0 is kept), and the column-node ids
+    std::vector<uint16_t> pmask((size_t)(lanes / 32), p->plane_mask ? 0 : 0x1FF);
     std::vector<int32_t> col((size_t)lanes);
     for (int64_t s = 0; s < p->n_slices; ++s) {
         const int64_t L = (slice_ptr[s + 1] - slice_ptr[s]) / 32;
-        double *vs = val.data() + 9 * slice_ptr[s];
+        uint16_t *ms = pmask.data() + slice_ptr[s] / 32;
         int32_t *cs = col.data() + slice_ptr[s];
         for (int l = 0; l < 32; ++l) {
             const int64_t inode = s * 32 + l;
@@ -410,20 +434,33 @@ extern "C" int saa_plan_finalize(saa_plan *p)
             int64_t cnt = 0;
             if (e >= 0) {
                 cnt = nblk[e];
-                int32_t q[3] = {p->indptr[3 * e], p->indptr[3 * e + 1], p->indptr[3 * e + 2]};
-                const int32_t qe[3] = {p->indptr[3 * e + 1], p->indptr[3 * e + 2], p->indptr[3 * e + 3]};
-                for (int64_t j = 0; j < cnt; ++j) {
-                    const int32_t cn = bcol[bptr[e] + j];
-                    for (int A = 0; A < 3; ++A)          // stored order kept: entries of a row in ascending column
-                        while (q[A] < qe[A] && p->indices[q[A]] / 3 == cn) {
-                            vs[(9 * j + 3 * A + p->indices[q[A]] % 3) * 32 + l] = p->data[q[A]];
-                            ++q[A];
-                        }
-                    cs[32 * j + l] = p->iperm_h[3 * (int64_t)cn] / 3;
-                }
+                for_each_entry(e, [&](int64_t j, int b, int32_t) { ms[j] |= (uint16_t)(1u << b); });
+                for (int64_t j = 0; j < cnt; ++j) cs[32 * j + l] = p->iperm_h[3 * (int64_t)bcol[bptr[e] + j]] / 3;
             }
             // padding blocks: 0.0 * d0[own node] at the end of the rows leaves the sums unchanged
             for (int64_t j = cnt; j < L; ++j) cs[32 * j + l] = (int32_t)inode;
+        }
+    }
+    std::vector<int64_t> val_ptr(p->n_slices + 1, 0);
+    for (int64_t s = 0; s < p->n_slices; ++s) {
+        int64_t planes = 0;
+        for (int64_t r = slice_ptr[s] / 32; r < slice_ptr[s + 1] / 32; ++r) planes += __builtin_popcount(pmask[r]);
+        val_ptr[s + 1] = val_ptr[s] + 32 * planes;
+    }
+    p->value_planes = val_ptr[p->n_slices] / 32;
+    std::vector<double> val((size_t)val_ptr[p->n_slices], 0.0);
+    for (int64_t s = 0; s < p->n_slices; ++s) {
+        const int64_t L = (slice_ptr[s + 1] - slice_ptr[s]) / 32;
+        const uint16_t *ms = pmask.data() + slice_ptr[s] / 32;
+        std::vector<int64_t> off(L + 1, 0);              // planes stored for the blocks before j
+        for (int64_t j = 0; j < L; ++j) off[j + 1] = off[j] + __builtin_popcount(ms[j]);
+        double *vs = val.data() + val_ptr[s];
+        for (int l = 0; l < 32; ++l) {
+            const int64_t e = permn[s * 32 + l];
+            if (e >= 0)
+                for_each_entry(e, [&](int64_t j, int b, int32_t k) {
+                    vs[32 * (off[j] + __builtin_popcount(ms[j] & ((1u << b) - 1u))) + l] = p->data[k];
+                });
         }
     }
     std::vector<double> M(p->n_rows, 1.0), F(p->n_rows, 0.0);
@@ -434,7 +471,8 @@ extern "C" int saa_plan_finalize(saa_plan *p)
         dir[i >> 5] |= (1u << (i & 31));
     }
 
-    if (upload(&p->d_slice_ptr, slice_ptr) || upload(&p->d_val, val) || upload(&p->d_col, col) ||
+    if (upload(&p->d_slice_ptr, slice_ptr) || upload(&p->d_val_ptr, val_ptr) || upload(&p->d_pmask, pmask) ||
+        upload(&p->d_val, val) || upload(&p->d_col, col) ||
         upload(&p->d_M, M) || upload(&p->d_F, F) || upload(&p->d_dir, dir) || upload(&p->d_iperm, p->iperm_h))
         return -1;
     const int64_t sh_pad = 3 * sh_padn;
@@ -460,7 +498,7 @@ static int finalize_tail(saa_plan *p, int64_t sh_pad)
     CK(cudaStreamCreateWithFlags(&p->stream, cudaStreamNonBlocking));
 
     p->D.n_rows = p->n_rows; p->D.n_slices = p->n_slices; p->D.sh_slices = p->sh_slices;
-    p->D.slice_ptr = p->d_slice_ptr; p->D.val = p->d_val; p->D.col = p->d_col; p->D.dir_mask = p->d_dir;
+    p->D.slice_ptr = p->d_slice_ptr; p->D.val_ptr = p->d_val_ptr; p->D.pmask = p->d_pmask; p->D.val = p->d_val; p->D.col = p->d_col; p->D.dir_mask = p->d_dir;
     p->D.M = p->d_M; p->D.F = p->d_F;
     {   // one mass value per node when every node's three DOFs hold the same bits (SAA_NODE_MASS=0 keeps the per-DOF stream)
         const char *nm = getenv("SAA_NODE_MASS");
@@ -560,10 +598,10 @@ static int finalize_tail(saa_plan *p, int64_t sh_pad)
     std::vector<int32_t>().swap(p->indptr); std::vector<int32_t>().swap(p->indices);
     std::vector<double>().swap(p->data); std::vector<double>().swap(p->F); std::vector<double>().swap(p->M);
     CK(cudaDeviceSynchronize());   // set-up work ran on the default stream; the plan's stream is non-blocking
-    if (const char *kv = getenv("SAA_KVARIANT")) p->kvariant = atoi(kv);
-    // measured on B200 (profiles/r1/kernel_variants.md, re-measured in round 2 after the mass-stream change, profiles/r2/
-    // kernel_variants_r2.md): the column-prefetching schedule with 4 blocks per SM wins at 1 M, 21 M and 104 M DOF
-    if (p->kvariant < 0) p->kvariant = 4;
+    // measured on B200 (profiles/r1/kernel_variants.md, profiles/r2/kernel_variants_r2.md, and after the plane-masked
+    // layout profiles/plane_mask/variants.md): the column-prefetching schedule with 3 blocks per SM (85-register cap; the
+    // predicated value loads spill under the 64-register cap of 4 blocks per SM) wins at 1.1 M and 104 M DOF
+    if (p->kvariant < 0) p->kvariant = 5;
     p->finalized = true;
     return prepare_graphs(p, false);
 }
@@ -580,7 +618,7 @@ extern "C" int saa_plan_destroy(saa_plan *p)
         }
         for (void *m : p->peer_mapped) cudaIpcCloseMemHandle(m);
         for (auto &g : p->step_graphs) cudaGraphExecDestroy(g.exec);
-        void *ptrs[] = {p->d_slice_ptr, p->d_val, p->d_col, p->d_M, p->d_F, p->d_dir, p->d_iperm, p->d_buf[0], p->d_buf[1],
+        void *ptrs[] = {p->d_slice_ptr, p->d_val_ptr, p->d_pmask, p->d_val, p->d_col, p->d_M, p->d_F, p->d_dir, p->d_iperm, p->d_buf[0], p->d_buf[1],
                         p->d_clk, p->d_stage, p->d_xbuf, p->d_send, p->d_dst_ptr, p->d_dst_pos, p->d_src_ptr, p->d_src_pos,
                         p->d_recv, p->d_done, p->d_own_ready, p->d_dst_nb, p->d_dst_pos_peer, p->d_peer_recv, p->d_peer_stride, p->d_peer_flag,
                         p->d_hist_rows, p->d_hist, p->d_pred_rows, p->d_force, p->d_hook,
@@ -608,10 +646,14 @@ extern "C" int64_t saa_plan_vector_bytes(const saa_plan *p)
     // fp64 streams of one step: d0 and dn read, d1 written, F read (one value per row each) + the lumped mass (per row, or per node)
     return p ? 4 * 8 * p->n_rows + 8 * (p->D.node_mass ? p->n_rows / 3 : p->n_rows) : -1;
 }
+extern "C" int64_t saa_plan_value_planes(const saa_plan *p) { return p ? p->value_planes : -1; }
 extern "C" int64_t saa_plan_matrix_bytes(const saa_plan *p)
 {
-    // 9 values + one column-node id per stored block, slice offsets, Dirichlet mask words
-    return p ? (p->padded_entries / 9) * 76 + (p->n_slices + 1) * 8 + (p->n_rows / 32) * 4 : -1;
+    // stored value planes (32 fp64 each), one column-node id per block-lane, one plane mask per block-row, slice and
+    // value offsets, Dirichlet mask words
+    if (!p) return -1;
+    const int64_t lanes = p->padded_entries / 9;
+    return p->value_planes * 256 + lanes * 4 + (lanes / 32) * 2 + 2 * (p->n_slices + 1) * 8 + (p->n_rows / 32) * 4;
 }
 extern "C" void *saa_plan_stream(saa_plan *p) { return p ? (void *)plan_stream(p) : nullptr; }
 

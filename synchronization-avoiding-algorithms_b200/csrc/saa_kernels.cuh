@@ -10,17 +10,23 @@
 // which nvcc never contracts into FMA, and the row sum runs over the stored entries in order starting
 // from 0.0 — the same sequence of roundings scipy/numpy perform, hence bit-identical results.
 //
-// Storage (HBM): node-block sliced ELL.  The stiffness of 3-D elasticity is made of 3x3 node blocks, so one
-// thread owns one NODE (its three DOF rows) and one warp owns a slice of 32 nodes.  Block j of the node of
-// lane l in slice s is stored as nine value planes and one column-node id (slice_ptr counts block-lanes):
-//     value (A,B) of block j :  val[9*slice_ptr[s] + (9*j + 3*A + B)*32 + l]
-//     column node of block j :  col[  slice_ptr[s] + j*32 + l]
-// so every warp-wide load is a fully coalesced, aligned 256-B (values) or 128-B (ids) request, and the column
-// id is shared by the nine entries of a block: 76 B per block instead of 108 B as scalar CSR.  Entries the
-// reference dropped as exact zeros (csr_matrix(dense), Mat_construction.py:150) are stored as 0.0 inside
-// their block; adding 0.0*x leaves a finite row sum bit-identical (the sum starts at +0.0 and can never
-// become -0.0).  Within a row the blocks are in ascending column order and inside a block B = 0,1,2, i.e.
-// exactly the stored order of the CSR row, which is the summation order of csr_matvec.
+// Storage (HBM): plane-masked node-block sliced ELL.  The stiffness of 3-D elasticity is made of 3x3 node blocks, so
+// one thread owns one NODE (its three DOF rows) and one warp owns a slice of 32 nodes.  Block j of the node of lane l in
+// slice s has one column-node id and up to nine value planes (plane (A,B) = entry (A,B) of block j in all 32 lanes);
+// slice_ptr counts block-lanes, the block-row of block j is r = slice_ptr[s]/32 + j:
+//     column node of block j  :  col[slice_ptr[s] + j*32 + l]
+//     stored planes of block j:  bit 3A+B of pmask[r]
+//     value (A,B) of block j  :  val[val_ptr[s] + 32*(off_j + popc(pmask[r] & ((1 << (3A+B)) - 1))) + l]  if that bit is set
+// where off_j is the number of planes stored for blocks 0..j-1 of the slice.  A plane is stored iff at least one lane
+// of the slice has a stored CSR entry there; a plane that is not stored is 0.0 in every lane, and the kernel puts 0.0
+// in the register instead of loading it, so the arithmetic is the same as with all nine planes.  On structured meshes
+// the 32 nodes of a slice share their stencil, so whole planes are zero in every lane (DESIGN.md §3).  Every warp-wide
+// load stays a fully coalesced, aligned 256-B (values) or 128-B (ids) request, and the column id is shared by the
+// entries of a block.  Entries the reference dropped as exact zeros (csr_matrix(dense), Mat_construction.py:150) in a
+// stored plane are 0.0; adding 0.0*x leaves a finite row sum bit-identical (the sum starts at +0.0 and can never
+// become -0.0).  Within a row the blocks are in ascending column order and inside a block B = 0,1,2, i.e. exactly the
+// stored order of the CSR row, which is the summation order of csr_matvec.  SAA_PLANE_MASK=0 at finalisation stores
+// all nine planes of every block (pmask = 0x1FF, val_ptr[s] = 9*slice_ptr[s]).
 // Nodes are ordered boundary-first (nodes of the partition interface, then interior) and, inside windows of
 // SIGMA nodes, by decreasing block count, so slices are almost padding-free; all vectors (d0, dn, M, F) live
 // in that internal order (row = 3*node + component) and are streamed.  The only non-streaming access is the
@@ -36,7 +42,7 @@ namespace cg = cooperative_groups;
 #define SAA_DOT_MODE 0
 #endif
 #ifndef SAA_UNROLL
-#define SAA_UNROLL 2          // blocks whose loads are in flight together per thread (2 x 76 B x 32 lanes per warp)
+#define SAA_UNROLL 2          // blocks whose loads are in flight together per thread (2 x at most 76 B x 32 lanes per warp)
 #endif
 
 struct SaaDev {
@@ -44,7 +50,9 @@ struct SaaDev {
     int64_t n_slices;          // slices of 32 nodes
     int64_t sh_slices;         // slices [0, sh_slices) hold the shared (interface) nodes
     const int64_t *slice_ptr;  // [n_slices + 1] offsets in block-lanes (multiples of 32)
-    const double *val;         // block values, nine planes per block (see above)
+    const int64_t *val_ptr;    // [n_slices + 1] offsets of the slices in val, in doubles
+    const uint16_t *pmask;     // [block-rows] stored value planes of each block-row (see above)
+    const double *val;         // stored value planes
     const int32_t *col;        // internal column NODE ids
     const uint32_t *dir_mask;  // bit (row & 31) of word (row >> 5) set: row is a Dirichlet DOF
     const double *M;           // lumped mass, internal row order — or one value per NODE when node_mass is set (all three
@@ -185,39 +193,57 @@ __device__ __forceinline__ void saa_block_madd(const double (&a)[9], const doubl
         for (int b = 0; b < 3; ++b) s[A] = __dadd_rn(s[A], __dmul_rn(a[3 * A + b], xv[b]));
 }
 
+// Value planes of one block: plane e is loaded iff bit e of the block's plane mask m is set (m is warp-uniform, so the
+// predicate is too); otherwise a[e] = 0.0, the value every lane would have loaded from a full-plane layout.  v points
+// at the block's first stored plane (of this lane); the stored planes follow each other in bit order.
+__device__ __forceinline__ double ld_stream_f64_if(const double *p, unsigned pred)
+{
+    double v;
+    asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %2, 0;\n\tmov.b64 %0, 0d0000000000000000;\n\t"
+                 "@q ld.global.nc.L1::no_allocate.f64 %0, [%1];\n\t}"
+                 : "=&d"(v) : "l"(p), "r"(pred));
+    return v;
+}
+__device__ __forceinline__ void saa_load_block(const double *v, unsigned m, double (&a)[9])
+{
+#pragma unroll
+    for (int e = 0; e < 9; ++e) a[e] = ld_stream_f64_if(v + 32 * __popc(m & ((1u << e) - 1u)), m & (1u << e));
+}
+
 template <int UNROLL, bool NC_X>
 __device__ __forceinline__ void saa_node_dot_pipe(const SaaDev &P, int64_t slice, int lane, const double *x, double (&s)[3])
 {
     static_assert(UNROLL == 2, "the software pipeline below is written for two blocks per batch");
     const int64_t beg = P.slice_ptr[slice];
     const int len = (int)((P.slice_ptr[slice + 1] - beg) >> 5);
-    const double *v = P.val + 9 * beg + lane;
+    const double *v = P.val + P.val_ptr[slice] + lane;
     const int32_t *c = P.col + beg + lane;
+    const uint16_t *mk = P.pmask + (beg >> 5);
     s[0] = 0.0; s[1] = 0.0; s[2] = 0.0;
-    // column ids run one batch ahead of the values, so that the gathers of a batch are issued together with its
-    // value loads instead of after a first round trip
+    // column ids and plane masks run one batch ahead of the values, so that the gathers of a batch are issued together
+    // with its value loads instead of after a first round trip
     int32_t k0 = 0, k1 = 0;
-    if (len > 0) k0 = ld_stream_s32(c);
-    if (len > 1) k1 = ld_stream_s32(c + 32);
+    unsigned m0 = 0, m1 = 0;
+    if (len > 0) { k0 = ld_stream_s32(c); m0 = __ldg(mk); }
+    if (len > 1) { k1 = ld_stream_s32(c + 32); m1 = __ldg(mk + 1); }
     int j = 0;
     for (; j + 2 <= len; j += 2) {
         double a0[9], a1[9], x0[3], x1[3];
-#pragma unroll
-        for (int e = 0; e < 9; ++e) a0[e] = ld_stream_f64(v + 32 * (9 * j + e));
-#pragma unroll
-        for (int e = 0; e < 9; ++e) a1[e] = ld_stream_f64(v + 32 * (9 * (j + 1) + e));
+        saa_load_block(v, m0, a0);
+        v += 32 * __popc(m0);
+        saa_load_block(v, m1, a1);
+        v += 32 * __popc(m1);
         saa_gather3<NC_X>(x, k0, x0);
         saa_gather3<NC_X>(x, k1, x1);
-        if (j + 2 < len) k0 = ld_stream_s32(c + 32 * (j + 2));
-        if (j + 3 < len) k1 = ld_stream_s32(c + 32 * (j + 3));
+        if (j + 2 < len) { k0 = ld_stream_s32(c + 32 * (j + 2)); m0 = __ldg(mk + j + 2); }
+        if (j + 3 < len) { k1 = ld_stream_s32(c + 32 * (j + 3)); m1 = __ldg(mk + j + 3); }
         SAA_FENCE9(a0); SAA_FENCE9(a1); SAA_FENCE3(x0); SAA_FENCE3(x1);
         saa_block_madd(a0, x0, s);              // blocks in ascending column order: the order of the CSR row
         saa_block_madd(a1, x1, s);
     }
     if (j < len) {
         double a0[9], x0[3];
-#pragma unroll
-        for (int e = 0; e < 9; ++e) a0[e] = ld_stream_f64(v + 32 * (9 * j + e));
+        saa_load_block(v, m0, a0);
         saa_gather3<NC_X>(x, k0, x0);
         saa_block_madd(a0, x0, s);
     }
@@ -229,19 +255,25 @@ __device__ __forceinline__ void saa_node_dot_simple(const SaaDev &P, int64_t sli
 {
     const int64_t beg = P.slice_ptr[slice];
     const int len = (int)((P.slice_ptr[slice + 1] - beg) >> 5);
-    const double *v = P.val + 9 * beg + lane;
+    const double *v = P.val + P.val_ptr[slice] + lane;
     const int32_t *c = P.col + beg + lane;
+    const uint16_t *mk = P.pmask + (beg >> 5);
     s[0] = 0.0; s[1] = 0.0; s[2] = 0.0;
     int j = 0;
     for (; j + UNROLL <= len; j += UNROLL) {
         double a[UNROLL][9];
         int32_t k[UNROLL];
+        unsigned m[UNROLL];
         double xv[UNROLL][3];
 #pragma unroll
         for (int u = 0; u < UNROLL; ++u) {
             k[u] = ld_stream_s32(c + 32 * (j + u));
+            m[u] = __ldg(mk + j + u);
+        }
 #pragma unroll
-            for (int e = 0; e < 9; ++e) a[u][e] = ld_stream_f64(v + 32 * (9 * (j + u) + e));
+        for (int u = 0; u < UNROLL; ++u) {
+            saa_load_block(v, m[u], a[u]);
+            v += 32 * __popc(m[u]);
         }
 #pragma unroll
         for (int u = 0; u < UNROLL; ++u) {
@@ -258,9 +290,10 @@ __device__ __forceinline__ void saa_node_dot_simple(const SaaDev &P, int64_t sli
     }
     for (; j < len; ++j) {
         const int32_t k = ld_stream_s32(c + 32 * j);
+        const unsigned m = __ldg(mk + j);
         double a[9];
-#pragma unroll
-        for (int e = 0; e < 9; ++e) a[e] = ld_stream_f64(v + 32 * (9 * j + e));
+        saa_load_block(v, m, a);
+        v += 32 * __popc(m);
         const double *xp = x + 3 * (int64_t)k;
         double xv[3];
 #pragma unroll
@@ -555,6 +588,8 @@ __global__ void __launch_bounds__(256, MINB) saa_k_step(SaaDev P, SaaHaloDev H, 
 // of the block-lanes, i.e. one contiguous stream of the value / id arrays, which it pulls through a ring of
 // STAGES buffers of two block-rows (2 x (2304 B values + 128 B ids)) each.  The d0 gathers of a stage are issued
 // one stage ahead.  Same arithmetic in the same order as saa_node_dot / saa_finish_node — same bits.
+// It addresses val by block-row arithmetic, so it needs the full-plane layout (all nine planes of every block stored);
+// finalisation builds that layout when this variant is selected.
 #define SAA_STREAM_STAGE_BYTES(BR) ((BR) * (2304 + 128))
 __device__ __forceinline__ void saa_cp_async16(void *smem_dst, const void *gmem_src)
 {

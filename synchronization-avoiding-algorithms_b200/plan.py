@@ -47,6 +47,7 @@ ABI = {
     "saa_plan_n_dof": (_i64, [_vp]),
     "saa_plan_nnz": (_i64, [_vp]),
     "saa_plan_padded_entries": (_i64, [_vp]),
+    "saa_plan_value_planes": (_i64, [_vp]),
     "saa_plan_kernel_launches": (_i64, [_vp]),
     "saa_plan_matrix_bytes": (_i64, [_vp]),
     "saa_plan_vector_bytes": (_i64, [_vp]),
@@ -251,6 +252,11 @@ class StepPlan:
     @property
     def padded_entries(self):
         return int(lib().saa_plan_padded_entries(self.h))
+
+    @property
+    def value_planes(self):
+        """value planes the step kernel streams (32 fp64 each); padded_entries / 32 when every plane is stored"""
+        return int(lib().saa_plan_value_planes(self.h))
 
     @property
     def matrix_bytes(self):
