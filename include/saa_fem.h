@@ -237,6 +237,34 @@ int saa_plan_read_history(saa_plan *plan, int64_t first, int64_t count, double *
 int saa_plan_read_history_dev(saa_plan *plan, int64_t first, int64_t count, double *out_dev);
 
 /*
+ * Energy monitor: while armed, every step of the plan also evaluates the terms of the central-difference scheme's
+ * discrete energy balance  E_{n+1/2} = E_{n-1/2} + dW_n - dD_n  (DESIGN.md §7a) and keeps the running sums of external
+ * and damping work on the device.  Every `every`-th step (step_idx % every == 0) writes one record of
+ * SAA_ENERGY_FIELDS doubles per rank into a device ring of `capacity` records:
+ *   0 step            step index n (the plan's step counter)
+ *   1 tn              t_n
+ *   2 kinetic_half    T_{n-1/2} = 1/2 sum m (d_n - d_{n-1})^2 / dt^2            over owned rows
+ *   3 coupling        1/2 sum d_{n-1,i} f_i,  f = this rank's own LocalK d_n    over all local rows
+ *   4 strain          U_n = 1/2 sum d_{n,i} f_i                                 over all local rows
+ *   5 kinetic         T_n = 1/2 sum m (d_{n+1} - d_{n-1})^2 / (4 dt^2)           over owned rows
+ *   6 work_external   sum of dW_k = F ramp(t_k) . (d_{k+1} - d_{k-1}) / 2 over arm <= k < n, owned rows
+ *   7 work_damping    sum of dD_k = alpha dt 2 T_k over arm <= k < n, owned rows
+ *   8 energy_at_arm   kinetic_half + coupling of the arming step (constant)
+ * Owned rows: non-shared rows, and a shared row on its lowest-rank holder only.  Fields 2-8 are additive over the ranks
+ * of a partition; the global residual  sum_r (kinetic_half + coupling - energy_at_arm - work_external + work_damping)
+ * is 0 in exact arithmetic (a PREDICT step's overwrite shows up in it).  Records are bit-identical run to run.
+ * capacity <= 0 disarms; every >= 1.  Arming resets the work sums; set_state keeps them.  All ranks of a partition
+ * must arm at the same step with the same `every`.  Not available with the persistent loop or SAA_OPT_MATFREE; with
+ * the peer transport, armed synchronised steps run as three kernels instead of the fused one.
+ */
+#define SAA_ENERGY_FIELDS 9
+int saa_plan_set_energy(saa_plan *plan, int64_t capacity, int64_t every);
+/* records written since arming */
+int64_t saa_plan_energy_count(const saa_plan *plan);
+/* copy records [first, first+count) to host memory (count x SAA_ENERGY_FIELDS doubles); fails for overwritten ones */
+int saa_plan_read_energy(saa_plan *plan, int64_t first, int64_t count, double *out_host);
+
+/*
  * Synchronization-avoiding mode (Online_predictor.py:280-301): `table` holds n_rows predictions of the
  * shared DOFs, row-major (n_rows, 3*n_shared_ref) in the order of the reference's loc_dof_shared
  * (`dofs`, local DOF ids, Online_predictor.py:129).  A SAA_MODE_PREDICT step overwrites those DOFs of d1

@@ -5,6 +5,7 @@
 // Reference semantics restated here (paths under /root/reference): Tools/Dynamic_solver.py:9-34,
 // Tools/Distributed_tools.py:77-92, Data_prepare.py:223-240, Online_predictor.py:251-318.
 #include "saa_kernels.cuh"
+#include "saa_energy.cuh"
 #include "saa_matfree.cuh"
 
 #include <dlfcn.h>
@@ -157,11 +158,21 @@ struct saa_plan {
     int32_t *d_pred_rows = nullptr;
     const double *d_pred_table = nullptr;
     int64_t pred_n = 0, pred_rows = 0, pred_next = 0;
+    std::vector<int32_t> pred_rows_h;       // internal rows of the predicted DOFs
     SaaHookDev hook_h{};                    // host mirror of the device-resident hook state
     SaaHookDev *d_hook = nullptr;
     int64_t hook_epoch = 0;                 // bumped when the hook configuration (not just the table) changes
     struct StepGraph { int mode, cur; int64_t epoch; cudaGraphExec_t exec; int launches; };
     std::vector<StepGraph> step_graphs;     // two-step graphs of steps with hooks
+    // energy monitor (saa_plan_set_energy): per-slice / per-unit partials [slices | units of 256 shared rows], the
+    // reduction's block sums and ticket, accumulators + ring; PREDICT steps: skipped-row mask, stashed d_{n-1}, partials
+    int64_t energy_cap = 0, energy_every = 1, energy_count = 0;
+    int64_t epart_n = 0, epred_n = 0;       // partials per field (stride) of the step and of the prediction scatter
+    int energy_grid = 0;                    // blocks of the reduction (fixed per plan: fixed summation order)
+    double *d_epart = nullptr, *d_estage = nullptr, *d_ering = nullptr, *d_epred = nullptr, *d_pred_stash = nullptr;
+    unsigned int *d_eticket = nullptr;
+    uint32_t *d_pred_skip = nullptr;
+    SaaEnergyDev *d_energy = nullptr;
     // execution
     cudaStream_t stream = nullptr;
     cudaGraphExec_t graph_exec[2] = {nullptr, nullptr};   // LOCAL-mode two-step graphs captured at cur = 0 / 1
@@ -622,6 +633,7 @@ extern "C" int saa_plan_destroy(saa_plan *p)
                         p->d_clk, p->d_stage, p->d_xbuf, p->d_send, p->d_dst_ptr, p->d_dst_pos, p->d_src_ptr, p->d_src_pos,
                         p->d_recv, p->d_done, p->d_own_ready, p->d_dst_nb, p->d_dst_pos_peer, p->d_peer_recv, p->d_peer_stride, p->d_peer_flag,
                         p->d_hist_rows, p->d_hist, p->d_pred_rows, p->d_force, p->d_hook,
+                        p->d_epart, p->d_estage, p->d_ering, p->d_epred, p->d_pred_stash, p->d_eticket, p->d_pred_skip, p->d_energy,
                         p->d_mf_slice_ptr, p->d_mf_inc, p->d_mf_cells, p->d_mf_X};
         for (void *q : ptrs)
             if (q) cudaFree(q);
@@ -733,6 +745,80 @@ extern "C" int saa_plan_get_state_dev(saa_plan *p, double *d0, double *dn, doubl
     return 0;
 }
 
+// ---- energy monitor --------------------------------------------------------------------------------------
+// PREDICT steps with the monitor on: K1E skips the d_{n+1} terms of the predicted rows (mask) and stashes their d_{n-1};
+// the prediction scatter adds those terms after the overwrite, one partial per block of 256 predicted rows
+static int energy_prepare_predict(saa_plan *p)
+{
+    CK(cudaStreamSynchronize(plan_stream(p)));       // earlier steps may still read the buffers replaced here
+    for (void *q : {(void *)p->d_pred_skip, (void *)p->d_pred_stash, (void *)p->d_epred})
+        if (q) cudaFree(q);
+    p->d_pred_skip = nullptr; p->d_pred_stash = nullptr; p->d_epred = nullptr; p->epred_n = 0;
+    if (p->pred_n <= 0) return 0;
+    std::vector<uint32_t> skip(p->n_rows / 32, 0u);
+    for (int32_t r : p->pred_rows_h) skip[r >> 5] |= 1u << (r & 31);
+    if (upload(&p->d_pred_skip, skip)) return -1;
+    CK(cudaMalloc((void **)&p->d_pred_stash, p->n_rows * sizeof(double)));
+    p->epred_n = nblk(p->pred_n, 256);
+    CK(cudaMalloc((void **)&p->d_epred, SAA_ENERGY_PARTS * p->epred_n * sizeof(double)));
+    return 0;
+}
+
+extern "C" int saa_plan_set_energy(saa_plan *p, int64_t capacity, int64_t every)
+{
+    NEED_FINAL(p, "saa_plan_set_energy");
+    if (capacity > 0 && every < 1) return fail("saa_plan_set_energy: every must be >= 1 (got %lld)", (long long)every);
+    if (capacity > 0 && p->matfree)
+        return fail("saa_plan_set_energy: the matrix-free kernel (SAA_OPT_MATFREE) computes a different force; the energy monitor needs the assembled-matrix step");
+    CK(cudaSetDevice(p->device));
+    CK(cudaStreamSynchronize(plan_stream(p)));
+    if (p->d_ering) { cudaFree(p->d_ering); p->d_ering = nullptr; }
+    p->energy_cap = p->energy_count = 0;
+    p->hook_epoch++;
+    if (capacity <= 0) return 0;
+    if (!p->d_epart) {                               // layout-sized buffers: allocated once per plan
+        const int64_t n_units = nblk(p->H.sh_rows, 256);
+        p->epart_n = p->n_slices + n_units;
+        p->energy_grid = (int)std::min<int64_t>(296, std::max<int64_t>(1, nblk(p->epart_n, 2048)));
+        CK(cudaMalloc((void **)&p->d_epart, SAA_ENERGY_PARTS * p->epart_n * sizeof(double)));
+        CK(cudaMemset(p->d_epart, 0, SAA_ENERGY_PARTS * p->epart_n * sizeof(double)));
+        CK(cudaMalloc((void **)&p->d_estage, SAA_ENERGY_PARTS * p->energy_grid * sizeof(double)));
+        CK(cudaMalloc((void **)&p->d_eticket, sizeof(unsigned int)));
+        CK(cudaMemset(p->d_eticket, 0, sizeof(unsigned int)));
+        CK(cudaMalloc((void **)&p->d_energy, sizeof(SaaEnergyDev)));
+    }
+    CK(cudaMalloc((void **)&p->d_ering, (size_t)capacity * SAA_ENERGY_FIELDS * sizeof(double)));
+    SaaEnergyDev e{};
+    e.arm = 1;
+    e.every = every;
+    e.first = (p->step_index + every - 1) / every;   // first recorded step is the next multiple of every
+    e.cap = capacity;
+    e.ring = p->d_ering;
+    CK(cudaMemcpy(p->d_energy, &e, sizeof e, cudaMemcpyHostToDevice));
+    p->energy_cap = capacity;
+    p->energy_every = every;
+    if (energy_prepare_predict(p)) return -1;
+    return 0;
+}
+extern "C" int64_t saa_plan_energy_count(const saa_plan *p) { return p ? p->energy_count : -1; }
+extern "C" int saa_plan_read_energy(saa_plan *p, int64_t first, int64_t count, double *out)
+{
+    NEED_FINAL(p, "saa_plan_read_energy");
+    if (first < 0 || count < 0 || first + count > p->energy_count) return fail("saa_plan_read_energy: range out of bounds");
+    if (first < p->energy_count - p->energy_cap) return fail("saa_plan_read_energy: records already overwritten");
+    if (count > 0 && !out) return fail("saa_plan_read_energy: null output");
+    CK(cudaSetDevice(p->device));
+    CK(cudaStreamSynchronize(plan_stream(p)));
+    for (int64_t s = 0; s < count;) {               // contiguous runs of the ring
+        const int64_t slot = (first + s) % p->energy_cap;
+        const int64_t run = std::min(count - s, p->energy_cap - slot);
+        CK(cudaMemcpy(out + s * SAA_ENERGY_FIELDS, p->d_ering + slot * SAA_ENERGY_FIELDS, run * SAA_ENERGY_FIELDS * sizeof(double),
+                      cudaMemcpyDeviceToHost));
+        s += run;
+    }
+    return 0;
+}
+
 // ---- history / prediction ------------------------------------------------------------------------------
 extern "C" int saa_plan_set_history(saa_plan *p, const int64_t *dofs, int64_t n_dofs, int64_t capacity, int64_t save_every)
 {
@@ -806,6 +892,8 @@ extern "C" int saa_plan_set_prediction(saa_plan *p, const int64_t *dofs, int64_t
         }
         if (upload(&p->d_pred_rows, rows)) return -1;
         p->pred_n = n_dofs;
+        p->pred_rows_h = rows;
+        if (p->energy_cap > 0 && energy_prepare_predict(p)) return -1;
     } else if (n_dofs != p->pred_n) {
         return fail("saa_plan_set_prediction: n_dofs changed without a DOF list");
     }
@@ -822,12 +910,27 @@ extern "C" int saa_plan_set_prediction(saa_plan *p, const int64_t *dofs, int64_t
 static void enqueue_hooks(saa_plan *p, cudaStream_t st, int mode)
 {
     const SaaClock *clk_old = p->d_clk + (p->cur ^ 1);
+    const bool energy = p->energy_cap > 0;
     if (mode == SAA_MODE_PREDICT && p->pred_n > 0) {                         // Online_predictor.py:298
-        saa_k_hook_scatter<<<nblk(p->pred_n, 256), 256, 0, st>>>(p->pred_n, p->d_pred_rows, p->d_hook, clk_old, p->d_buf[p->cur]);
+        if (energy)
+            saa_k_hook_scatter_energy<<<nblk(p->pred_n, 256), 256, 0, st>>>(p->D, p->H, p->pred_n, p->d_pred_rows, p->d_hook, clk_old,
+                                                                            p->d_buf[p->cur], p->d_pred_stash, p->d_epred, p->epred_n);
+        else
+            saa_k_hook_scatter<<<nblk(p->pred_n, 256), 256, 0, st>>>(p->pred_n, p->d_pred_rows, p->d_hook, clk_old, p->d_buf[p->cur]);
         p->launches++;
     }
     if (p->hist_cap > 0 && p->hist_n > 0) {                                  // Data_prepare.py:238-240
         saa_k_hook_gather<<<nblk(p->hist_n, 256), 256, 0, st>>>(p->hist_n, p->d_hist_rows, p->d_hook, clk_old, p->d_buf[p->cur], p->d_hist);
+        p->launches++;
+    }
+    if (energy) {
+        // partials this step wrote: synchronised steps K1E over the interior slices + K3E units (contiguous), other
+        // steps K1E over every slice (+ the prediction scatter's blocks)
+        const bool sync = mode == SAA_MODE_SYNC && p->size > 1;
+        const int64_t a0 = sync ? p->sh_slices : 0, na = (sync ? p->epart_n : p->n_slices) - a0;
+        const bool pred = mode == SAA_MODE_PREDICT && p->pred_n > 0;
+        saa_k_energy_reduce<<<p->energy_grid, 256, 0, st>>>(p->d_epart, p->epart_n, a0, na, p->d_epred, p->epred_n, 0, pred ? p->epred_n : 0,
+                                                            p->d_estage, p->d_eticket, p->d_energy, clk_old, p->dt, p->dt2, p->alpha);
         p->launches++;
     }
 }
@@ -835,6 +938,7 @@ static void count_step(saa_plan *p, int mode)
 {
     if (mode == SAA_MODE_PREDICT) p->pred_next++;
     if (p->hist_cap > 0 && (p->step_index % p->hist_every) == 0) p->hist_count++;
+    if (p->energy_cap > 0 && (p->step_index % p->energy_every) == 0) p->energy_count++;
     p->step_index++;
 }
 static int check_prediction(saa_plan *p, int mode, int64_t n_steps)
@@ -880,11 +984,21 @@ static void launch_stream(saa_plan *p, cudaStream_t st, const SaaDev &D, int64_t
     p->launches++;
 }
 // K1 only: slices [slice_begin, n_slices) as interior rows (no interface handling inside the kernel)
-static void launch_interior(saa_plan *p, cudaStream_t st, int64_t slice_begin, unsigned count_sync, bool advance_clock, int64_t slice_end = -1)
+static void launch_interior(saa_plan *p, cudaStream_t st, int64_t slice_begin, unsigned count_sync, bool advance_clock, int64_t slice_end = -1,
+                            bool predict = false)
 {
     SaaDev D = p->D;
     D.sh_slices = 0;
     if (slice_end < 0) slice_end = p->n_slices;
+    if (p->energy_cap > 0) {       // K1E (also for the cp.async variant: its full-plane layout is a layout with pmask = 0x1FF)
+        const unsigned n_main = std::max(1u, nblk(slice_end - slice_begin, SAA_WARPS_PER_BLOCK));
+        const bool skip = predict && p->pred_n > 0;
+        saa_k_step_energy<1><<<n_main, 256, 0, st>>>(D, p->H, p->d_buf[p->cur], p->d_buf[p->cur ^ 1], p->d_clk + p->cur,
+                                                     advance_clock ? p->d_clk + (p->cur ^ 1) : nullptr, slice_begin, count_sync,
+                                                     p->d_epart, p->epart_n, skip ? p->d_pred_skip : nullptr, p->d_pred_stash);
+        p->launches++;
+        return;
+    }
     if (p->kvariant >= 6 && p->n_slices > slice_begin) {       // cp.async streaming kernels, persistent grid
         launch_stream<3, 24, 1>(p, st, D, slice_begin, count_sync, advance_clock);   // the fastest streaming configuration measured
         return;
@@ -896,7 +1010,7 @@ static void launch_interior(saa_plan *p, cudaStream_t st, int64_t slice_begin, u
     p->launches++;
 }
 
-static void launch_local_step(saa_plan *p, cudaStream_t st)
+static void launch_local_step(saa_plan *p, cudaStream_t st, bool predict = false)
 {
     if (p->matfree) {
         const unsigned g = std::max(1u, nblk(p->n_slices, SAA_WARPS_PER_BLOCK));
@@ -909,19 +1023,19 @@ static void launch_local_step(saa_plan *p, cudaStream_t st)
         }
         p->launches++;
     } else {
-        launch_interior(p, st, 0, 0u, true);
+        launch_interior(p, st, 0, 0u, true, -1, predict);
     }
     p->cur ^= 1;
 }
 
-static bool needs_hooks(const saa_plan *p, int mode) { return mode == SAA_MODE_PREDICT || p->hist_cap > 0; }
+static bool needs_hooks(const saa_plan *p, int mode) { return mode == SAA_MODE_PREDICT || p->hist_cap > 0 || p->energy_cap > 0; }
 
 // one step of `mode` (local / predict / peer-synchronised) with its hooks: kernels only
 static void launch_peer_step(saa_plan *p, cudaStream_t st);
 static void enqueue_step_with_hooks(saa_plan *p, cudaStream_t st, int mode)
 {
     if (mode == SAA_MODE_SYNC) launch_peer_step(p, st);
-    else launch_local_step(p, st);
+    else launch_local_step(p, st, mode == SAA_MODE_PREDICT);
     enqueue_hooks(p, st, mode);
 }
 // steps with history / prediction hooks, replayed two at a time from a CUDA graph (the hooks take their row / slot
@@ -976,6 +1090,8 @@ static int capture_two_steps(saa_plan *p, bool peer)
     cudaGraphExec_t *slot = peer ? &p->graph_peer[p->cur] : &p->graph_exec[p->cur];
     if (*slot) return 0;
     cudaGraph_t g;
+    const int64_t energy_cap = p->energy_cap;
+    p->energy_cap = 0;                               // these graphs run only while no hook is set: never the monitor's kernels
     CK(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
     const int64_t l0 = p->launches;
     for (int i = 0; i < 2; ++i) {
@@ -983,6 +1099,7 @@ static int capture_two_steps(saa_plan *p, bool peer)
         else launch_local_step(p, st);
     }
     p->launches = l0;
+    p->energy_cap = energy_cap;
     CK(cudaStreamEndCapture(st, &g));
     CK(cudaGraphInstantiate(slot, g, 0));
     CK(cudaGraphDestroy(g));
@@ -1005,6 +1122,8 @@ static int step_local(saa_plan *p, int64_t n_steps, int mode, int launch)
     cudaStream_t st = p->stream;
     const bool hooks = needs_hooks(p, mode);
     if (launch == SAA_LAUNCH_AUTO) launch = (n_steps >= 2 ? SAA_LAUNCH_GRAPH : SAA_LAUNCH_PER_STEP);   // graphs exist since finalize
+    if (p->energy_cap > 0 && launch == SAA_LAUNCH_PERSISTENT)
+        return fail("saa_plan_step: the energy monitor is not available in the persistent loop (disarm it, or use per-step or graph launches)");
     if (hooks && launch == SAA_LAUNCH_PERSISTENT) return fail("history / prediction hooks are not available in the persistent loop");
     if (p->matfree && launch == SAA_LAUNCH_PERSISTENT) return fail("the matrix-free kernel has no persistent form");
     if (check_prediction(p, mode, n_steps)) return -1;
@@ -1037,7 +1156,7 @@ static int step_local(saa_plan *p, int64_t n_steps, int mode, int launch)
         p->step_index += done;
     }
     for (; done < n_steps; ++done) {
-        launch_local_step(p, st);
+        launch_local_step(p, st, mode == SAA_MODE_PREDICT);
         enqueue_hooks(p, st, mode);
         count_step(p, mode);
     }
@@ -1065,7 +1184,14 @@ static void sync_phase_interior(saa_plan *p, cudaStream_t st)
 static void sync_phase_shared(saa_plan *p, cudaStream_t st)
 {
     if (p->sh_slices > 0) {
-        if (use_peer(p))
+        if (p->energy_cap > 0) {   // K3E: partials of the units of 256 shared rows after the slices' ones
+            if (use_peer(p))
+                saa_k_shared_update_energy<true><<<nblk(p->H.sh_rows, 256), 256, 0, st>>>(p->D, p->Hp, p->d_buf[p->cur], p->d_buf[p->cur ^ 1], p->d_clk + p->cur,
+                                                                                         p->d_epart, p->epart_n, p->n_slices);
+            else
+                saa_k_shared_update_energy<false><<<nblk(p->H.sh_rows, 256), 256, 0, st>>>(p->D, p->H, p->d_buf[p->cur], p->d_buf[p->cur ^ 1], p->d_clk + p->cur,
+                                                                                          p->d_epart, p->epart_n, p->n_slices);
+        } else if (use_peer(p))
             saa_k_shared_update<true><<<nblk(p->H.sh_rows, 256), 256, 0, st>>>(p->D, p->Hp, p->d_buf[p->cur], p->d_buf[p->cur ^ 1], p->d_clk + p->cur);
         else
             saa_k_shared_update<false><<<nblk(p->H.sh_rows, 256), 256, 0, st>>>(p->D, p->H, p->d_buf[p->cur], p->d_buf[p->cur ^ 1], p->d_clk + p->cur);
@@ -1107,7 +1233,7 @@ static int step_sync_nccl(saa_plan *p, int64_t n_steps)
 // peer transport: three stream-ordered kernels per step, no host involvement -> replayed from a two-step graph
 static void launch_peer_step(saa_plan *p, cudaStream_t st)
 {
-    if (p->peer_fused && p->sh_slices > 0) {
+    if (p->peer_fused && p->sh_slices > 0 && p->energy_cap == 0) {     // the monitor has no fused form: three kernels
         // n_main slice blocks + one tail block per unit of 256 shared rows; at most one WAITING tail block per SM (every
         // schedule variant keeps >= 3 blocks per SM resident), so blocks that have not started always find a slot
         const unsigned n_main = nblk(p->n_slices, SAA_WARPS_PER_BLOCK);
@@ -1127,11 +1253,13 @@ static void launch_peer_step(saa_plan *p, cudaStream_t st)
 static int step_sync_peer(saa_plan *p, int64_t n_steps, int launch)
 {
     cudaStream_t st = p->stream;
-    const bool hooks = p->hist_cap > 0;
+    const bool hooks = p->hist_cap > 0 || p->energy_cap > 0;
     int64_t done = 0;
     if (launch == SAA_LAUNCH_PERSISTENT) {
         // one cooperative launch for all n_steps synchronised steps (small shards: no launch per step); every rank must
         // make the same call, like any synchronised step
+        if (p->energy_cap > 0)
+            return fail("saa_plan_step: the energy monitor is not available in the persistent loop (disarm it, or use per-step or graph launches)");
         if (hooks) return fail("history hooks are not available in the persistent loop");
         if (p->coop_blocks_sync <= 0) return fail("cooperative launch not available");
         if (p->sh_slices == 0) return fail("saa_plan_step: the persistent synchronised loop needs an interface (this rank has none)");
@@ -1202,6 +1330,8 @@ extern "C" int saa_plan_set_option(saa_plan *p, int option, int value)
         return p->peer ? prepare_graphs(p, true) : 0;
     }
     if (option == SAA_OPT_MATFREE) {
+        if (value && p->energy_cap > 0)
+            return fail("saa_plan_set_option: the energy monitor is armed; the matrix-free kernel (SAA_OPT_MATFREE) computes a different force and has no energy form");
         if (value && !p->d_mf_inc) return fail("saa_plan_set_option: SAA_OPT_MATFREE needs saa_plan_set_matfree_dev first");
         if (!value && !p->d_val) return fail("saa_plan_set_option: the assembled matrix of this plan was released (SAA_OPT_MATFREE = 2)");
         if (value == 2 && p->d_val) {                    // release the assembled matrix: the plan is matrix-free for good
@@ -1651,7 +1781,7 @@ extern "C" int saa_group_step(saa_group *g, int64_t n_steps, int mode, int launc
             }
         } else {
             for (saa_plan *p : g->plans) {
-                launch_local_step(p, st);
+                launch_local_step(p, st, mode == SAA_MODE_PREDICT);
                 if (after_step(p, st, mode == SAA_MODE_SYNC ? SAA_MODE_LOCAL : mode)) return -1;
             }
         }

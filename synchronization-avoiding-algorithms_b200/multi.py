@@ -52,3 +52,13 @@ def attach_transport(pl, transport="peer"):
     elif transport != "host":
         raise ValueError(f"unknown transport {transport!r}")
     return transport
+
+
+def gather_energy(pl, first=0, count=None):
+    """Global energy balance of a partition stepped one process per rank: every rank's energy records
+    (StepPlan.read_energy) all-gathered through `torch.distributed` and combined by plan.energy_balance.
+    Collective; all ranks get the same array."""
+    import torch.distributed as dist
+    recs = [None] * dist.get_world_size()
+    dist.all_gather_object(recs, (pl.rank, pl.read_energy(first, count)))
+    return _plan.energy_balance([r for _, r in sorted(recs, key=lambda t: t[0])])

@@ -71,6 +71,9 @@ ABI = {
     "saa_plan_read_history": (_int, [_vp, _i64, _i64, _vp]),
     "saa_plan_read_history_dev": (_int, [_vp, _i64, _i64, _vp]),
     "saa_plan_set_prediction": (_int, [_vp, _vp, _i64, _vp, _i64]),
+    "saa_plan_set_energy": (_int, [_vp, _i64, _i64]),
+    "saa_plan_energy_count": (_i64, [_vp]),
+    "saa_plan_read_energy": (_int, [_vp, _i64, _i64, _vp]),
     "saa_plan_halo_layout": (_int, [_vp, _vp, _vp, _vp, _int]),
     "saa_plan_step_begin_host": (_int, [_vp, _vp]),
     "saa_plan_step_end_host": (_int, [_vp, _vp]),
@@ -89,6 +92,34 @@ ABI = {
 
 class SaaError(RuntimeError):
     pass
+
+
+# one energy record (include/saa_fem.h, SAA_ENERGY_FIELDS): fields 2-8 are additive over the ranks of a partition
+ENERGY_FIELDS = ("step", "tn", "kinetic_half", "coupling", "strain", "kinetic", "work_external", "work_damping",
+                 "energy_at_arm")
+ENERGY_DTYPE = np.dtype([("step", np.int64)] + [(f, np.float64) for f in ENERGY_FIELDS[1:]])
+BALANCE_DTYPE = np.dtype(ENERGY_DTYPE.descr + [("total", np.float64), ("residual", np.float64)])
+
+
+def energy_balance(records_per_rank):
+    """Global energy balance of a partition from the per-rank records of the same steps (read_energy of every rank,
+    in rank order): the additive fields summed in ascending rank order, plus
+      total    = kinetic_half + coupling                      (E_{n-1/2} = T_{n-1/2} + S_{n-1/2})
+      residual = total - energy_at_arm - work_external + work_damping   (0 in exact arithmetic).
+    Raises ValueError when the ranks' records are not of the same steps."""
+    recs = [np.asarray(r) for r in records_per_rank]
+    if not recs:
+        raise ValueError("energy_balance: no records")
+    out = np.zeros(recs[0].shape, dtype=BALANCE_DTYPE)
+    out["step"], out["tn"] = recs[0]["step"], recs[0]["tn"]
+    for q, r in enumerate(recs):
+        if r.shape != out.shape or not np.array_equal(r["step"], out["step"]) or not np.array_equal(r["tn"], out["tn"]):
+            raise ValueError(f"energy_balance: the records of rank {q} are not of the same steps as rank 0's (step / tn differ)")
+        for f in ENERGY_FIELDS[2:]:
+            out[f] += r[f]
+    out["total"] = out["kinetic_half"] + out["coupling"]
+    out["residual"] = out["total"] - out["energy_at_arm"] - out["work_external"] + out["work_damping"]
+    return out
 
 
 PINNED_POOL = 4
@@ -410,6 +441,27 @@ class StepPlan:
         n = self._pred_n if d is None else d.size
         self._pred_n = n
         _check(lib().saa_plan_set_prediction(self.h, _p(d), n, table_dev_ptr, int(n_rows)), "saa_plan_set_prediction")
+
+    # ---- energy monitor ----------------------------------------------------------------------------
+    def set_energy(self, capacity, every=1):
+        """Arm the on-device energy monitor with a ring of `capacity` records, one every `every` steps (capacity 0
+        disarms).  Every rank of a partition must arm at the same step with the same `every`."""
+        _check(lib().saa_plan_set_energy(self.h, int(capacity), int(every)), "saa_plan_set_energy")
+
+    @property
+    def energy_count(self):
+        return int(lib().saa_plan_energy_count(self.h))
+
+    def read_energy(self, first=0, count=None):
+        """Records [first, first + count) as a structured array of ENERGY_DTYPE (this rank's share; energy_balance
+        combines the ranks)."""
+        count = self.energy_count - first if count is None else count
+        raw = np.empty((max(int(count), 0), len(ENERGY_FIELDS)))
+        _check(lib().saa_plan_read_energy(self.h, int(first), int(count), _p(raw)), "saa_plan_read_energy")
+        out = np.empty(raw.shape[0], dtype=ENERGY_DTYPE)
+        for k, f in enumerate(ENERGY_FIELDS):
+            out[f] = raw[:, k]
+        return out
 
     # ---- caller-provided transport (messages through host memory) -----------------------------------
     def halo_layout(self):
