@@ -33,6 +33,30 @@ struct SaaRowTriple {
         return cn;
     }
 };
+// the checks saa_plan_create / saa_plan_finalize make on a host CSR, one thread per row; sets bits of *bad:
+//   1 indptr[0] != 0, 2 indptr decreases, 4 a column index outside [0, n_rows), 8 columns of a row not strictly increasing.
+// A row reads indices only inside [0, nnz), so a malformed indptr cannot make the check itself read out of bounds.
+#define SAA_CSR_BAD_START 1u
+#define SAA_CSR_BAD_INDPTR 2u
+#define SAA_CSR_BAD_COLUMN 4u
+#define SAA_CSR_BAD_ORDER 8u
+__global__ void saa_k_fin_check_csr(int64_t n_rows, int64_t nnz, const int64_t *__restrict__ indptr,
+                                    const int32_t *__restrict__ indices, unsigned int *__restrict__ bad)
+{
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_rows) return;
+    const int64_t a = indptr[i], b = indptr[i + 1];
+    unsigned int f = 0u;
+    if (i == 0 && a != 0) f |= SAA_CSR_BAD_START;
+    if (b < a) f |= SAA_CSR_BAD_INDPTR;
+    if (a >= 0 && a <= b && b <= nnz)
+        for (int64_t k = a; k < b; ++k) {
+            const int32_t c = indices[k];
+            if (c < 0 || c >= n_rows) f |= SAA_CSR_BAD_COLUMN;
+            if (k > a && c <= indices[k - 1]) f |= SAA_CSR_BAD_ORDER;
+        }
+    if (f) atomicOr(bad, f);
+}
 __global__ void saa_k_fin_nblk(int64_t n_nodes, const int64_t *__restrict__ indptr, const int32_t *__restrict__ indices, int32_t *__restrict__ nblk)
 {
     const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -213,6 +237,21 @@ static int finalize_device(saa_plan *p)
     const int64_t n_sh = (int64_t)p->shared_pos.size();
     CK(cudaMemcpy(&p->nnz, p->in_indptr + n, sizeof(int64_t), cudaMemcpyDeviceToHost));
     auto pad32 = [](int64_t v) { return (v + 31) / 32 * 32; };
+
+    // 0. the CSR must be what the host path accepts: every kernel below indexes by its column ids
+    {
+        DevBuf b_bad;
+        if (b_bad.alloc(sizeof(unsigned int))) return -1;
+        CK(cudaMemset(b_bad.p, 0, sizeof(unsigned int)));
+        saa_k_fin_check_csr<<<nblk(n, 256), 256>>>(n, p->nnz, p->in_indptr, p->in_indices, b_bad.as<unsigned int>());
+        CK(cudaGetLastError());
+        unsigned int bad = 0;
+        CK(cudaMemcpy(&bad, b_bad.p, sizeof(unsigned int), cudaMemcpyDeviceToHost));
+        if (bad & SAA_CSR_BAD_START) return fail("saa_plan_finalize: indptr[0] is not 0");
+        if (bad & SAA_CSR_BAD_INDPTR) return fail("saa_plan_finalize: indptr not monotone");
+        if (bad & SAA_CSR_BAD_COLUMN) return fail("saa_plan_finalize: column index out of range");
+        if (bad & SAA_CSR_BAD_ORDER) return fail("saa_plan_finalize: LocalK must have sorted, duplicate-free column indices");
+    }
 
     // 1. block counts, shared flags, the two regions in their starting order
     DevBuf b_nblk, b_flag, b_sh, b_in, b_key;
