@@ -185,6 +185,30 @@ int saa_plan_set_option(saa_plan *plan, int option, int value);
 int saa_plan_set_matfree_dev(saa_plan *plan, int64_t n_elem, const int32_t *cells_dev, const double *coords_dev,
                              double lmd, double mu);
 int64_t saa_plan_matfree_bytes(const saa_plan *plan); /* bytes K5 streams per step besides the vector streams     */
+
+/*
+ * Stress recovery (DESIGN.md §7b) from the plan's current displacement d0, i.e. d_n at the plan's tn, after all work
+ * enqueued on the plan so far.  Both need the element geometry attached by saa_plan_set_matfree_dev (attaching it does
+ * not enable the matrix-free step) and work with any SAA_OPT_MATFREE value and any transport.  They change no state,
+ * clock, hook or energy sum.
+ *
+ * saa_plan_element_stress_dev: out_dev (n_elem x SAA_STRESS_FIELDS doubles, device) receives per element, in the
+ *   order of the cells handed to saa_plan_set_matfree_dev:
+ *     0-5  sigma = D B u_e in Voigt order  sxx syy szz syz sxz sxy  (B of Mat_construction.py:99-104, D of
+ *          commons.py:25-31; constant over a linear tetrahedron)
+ *     6    von Mises  sqrt(0.5 ((sxx-syy)^2 + (syy-szz)^2 + (szz-sxx)^2) + 3 (syz^2 + sxz^2 + sxy^2))
+ *     7    weight V_e = detJ / 6, the factor of B^T D B in the element stiffness
+ *   An element's values depend only on its four corners in connectivity order: the same element gives the same bits
+ *   whatever the partition, node order or set-up path.  out_dev must be 16-byte aligned.  Returns after the plan's stream has finished the work; fails
+ *   when an element has detJ <= 0 (its row is zero then).
+ * saa_plan_nodal_stress_dev: from element rows elem_dev (the output above), out_dev (n_nodes x 7 doubles, device,
+ *   Local_nodal_list order) receives this rank's partial sums  sum_e V_e sigma_e (6) and sum_e V_e (1) over the local
+ *   elements incident to the node, added in ascending element order (elem_dev 16-byte aligned).  Shared nodes need the sum over their holders
+ *   before the division (plan.nodal_stress).  Enqueued on the plan's stream; saa_plan_synchronize waits for it.
+ */
+#define SAA_STRESS_FIELDS 8   /* sxx syy szz syz sxz sxy von_mises weight(detJ/6) */
+int saa_plan_element_stress_dev(saa_plan *plan, double *out_dev);
+int saa_plan_nodal_stress_dev(saa_plan *plan, const double *elem_dev, double *out_dev);
 /* the cudaStream_t the plan enqueues on (as void*), so that callers can record events on it */
 void *saa_plan_stream(saa_plan *plan);
 

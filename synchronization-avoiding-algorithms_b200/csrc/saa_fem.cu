@@ -7,6 +7,7 @@
 #include "saa_kernels.cuh"
 #include "saa_energy.cuh"
 #include "saa_matfree.cuh"
+#include "saa_stress.cuh"
 
 #include <dlfcn.h>
 
@@ -204,6 +205,9 @@ struct saa_plan {
     int64_t mf_elems = 0, mf_lanes = 0;
     int mf_minb = 3;                        // SAA_MF_MINB: minimum resident blocks per SM of the matrix-free kernel (register cap)
     bool matfree = false;                   // SAA_OPT_MATFREE: local steps evaluate B^T D B u_e instead of streaming the matrix
+    // stress recovery (saa_plan_element_stress_dev / saa_plan_nodal_stress_dev), allocated on first use
+    int32_t *d_st_ext = nullptr;            // external position of every internal node (-1: slice padding)
+    unsigned long long *d_st_bad = nullptr; // lowest element index with detJ <= 0 of the last element call, ~0 if none
 };
 
 struct saa_group {
@@ -634,7 +638,7 @@ extern "C" int saa_plan_destroy(saa_plan *p)
                         p->d_recv, p->d_done, p->d_own_ready, p->d_dst_nb, p->d_dst_pos_peer, p->d_peer_recv, p->d_peer_stride, p->d_peer_flag,
                         p->d_hist_rows, p->d_hist, p->d_pred_rows, p->d_force, p->d_hook,
                         p->d_epart, p->d_estage, p->d_ering, p->d_epred, p->d_pred_stash, p->d_eticket, p->d_pred_skip, p->d_energy,
-                        p->d_mf_slice_ptr, p->d_mf_inc, p->d_mf_cells, p->d_mf_X};
+                        p->d_mf_slice_ptr, p->d_mf_inc, p->d_mf_cells, p->d_mf_X, p->d_st_ext, p->d_st_bad};
         for (void *q : ptrs)
             if (q) cudaFree(q);
         if (p->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(p->comm);
@@ -1944,4 +1948,50 @@ extern "C" int64_t saa_plan_matfree_bytes(const saa_plan *p)
 {
     if (!p || !p->d_mf_inc) return -1;
     return 16 * p->mf_elems + 4 * p->mf_lanes + 24 * (p->n_rows / 3) + (p->n_slices + 1) * 8 + (p->n_rows / 32) * 4;
+}
+
+// ---- stress recovery (saa_stress.cuh) --------------------------------------------------------------------------
+extern "C" int saa_plan_element_stress_dev(saa_plan *p, double *out_dev)
+{
+    NEED_FINAL(p, "saa_plan_element_stress_dev");
+    if (!p->d_mf_inc) return fail("saa_plan_element_stress_dev: no element geometry attached; call saa_plan_set_matfree_dev first");
+    if (!out_dev) return fail("saa_plan_element_stress_dev: null output");
+    if ((uintptr_t)out_dev % 16) return fail("saa_plan_element_stress_dev: out_dev must be 16-byte aligned");
+    CK(cudaSetDevice(p->device));
+    const cudaStream_t st = plan_stream(p);
+    if (!p->d_st_bad) CK(cudaMalloc((void **)&p->d_st_bad, sizeof(unsigned long long)));
+    CK(cudaMemsetAsync(p->d_st_bad, 0xff, sizeof(unsigned long long), st));
+    saa_k_stress_elem<<<nblk(p->mf_elems, 256), 256, 0, st>>>(p->mf_elems, p->MF.cells, p->MF.X, p->d_buf[p->cur], p->MF.lmd, p->MF.mu,
+                                                             out_dev, p->d_st_bad);
+    CK(cudaGetLastError());
+    p->launches++;
+    unsigned long long bad = 0;
+    CK(cudaMemcpyAsync(&bad, p->d_st_bad, sizeof bad, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    if (bad != ~0ull)
+        return fail("saa_plan_element_stress_dev: element %llu (in the order given to saa_plan_set_matfree_dev) has detJ <= 0: "
+                    "inverted or degenerate tetrahedron", bad);
+    return 0;
+}
+
+extern "C" int saa_plan_nodal_stress_dev(saa_plan *p, const double *elem_dev, double *out_dev)
+{
+    NEED_FINAL(p, "saa_plan_nodal_stress_dev");
+    if (!p->d_mf_inc) return fail("saa_plan_nodal_stress_dev: no element geometry attached; call saa_plan_set_matfree_dev first");
+    if (!elem_dev || !out_dev) return fail("saa_plan_nodal_stress_dev: null argument");
+    if ((uintptr_t)elem_dev % 16) return fail("saa_plan_nodal_stress_dev: elem_dev must be 16-byte aligned");
+    CK(cudaSetDevice(p->device));
+    const cudaStream_t st = plan_stream(p);
+    if (!p->d_st_ext) {
+        CK(cudaMalloc((void **)&p->d_st_ext, (p->n_rows / 3) * sizeof(int32_t)));
+        CK(cudaMemsetAsync(p->d_st_ext, 0xff, (p->n_rows / 3) * sizeof(int32_t), st));
+        saa_k_hp_inverse<<<nblk(p->n_dof / 3, 256), 256, 0, st>>>(p->n_dof / 3, p->d_iperm, p->d_st_ext);
+        CK(cudaGetLastError());
+        p->launches++;
+    }
+    saa_k_stress_node<<<nblk(p->n_slices, SAA_WARPS_PER_BLOCK), 32 * SAA_WARPS_PER_BLOCK, 0, st>>>(p->n_slices, p->MF.slice_ptr, p->MF.inc,
+                                                                                                   p->d_st_ext, elem_dev, out_dev);
+    CK(cudaGetLastError());
+    p->launches++;
+    return 0;
 }

@@ -62,3 +62,17 @@ def gather_energy(pl, first=0, count=None):
     recs = [None] * dist.get_world_size()
     dist.all_gather_object(recs, (pl.rank, pl.read_energy(first, count)))
     return _plan.energy_balance([r for _, r in sorted(recs, key=lambda t: t[0])])
+
+
+def gather_nodal_stress(pl, halo=None):
+    """Averaged nodal stresses (n_nodes, 7) of this rank's nodes for a partition stepped one process per rank: the
+    partial sums of the shared nodes travel to their other holders (device_setup.dist_exchange) and are summed in
+    ascending rank order.  Collective when pl.size > 1; `halo` is this rank's maps.halo_plan."""
+    from . import device_setup, stress
+    part = pl.nodal_stress_partial()
+    if pl.size == 1:
+        return stress.nodal_stress(part)
+    if halo is None:
+        raise _plan.SaaError("gather_nodal_stress: a partition of size > 1 needs this rank's halo (maps.halo_plan)")
+    recv = device_setup.dist_exchange(stress.shared_message(part, halo))
+    return stress.nodal_stress(part, halo, pl.rank, recv)

@@ -60,6 +60,8 @@ ABI = {
     "saa_plan_set_option": (_int, [_vp, _int, _int]),
     "saa_plan_set_matfree_dev": (_int, [_vp, _i64, _vp, _vp, _f64, _f64]),
     "saa_plan_matfree_bytes": (_i64, [_vp]),
+    "saa_plan_element_stress_dev": (_int, [_vp, _vp]),
+    "saa_plan_nodal_stress_dev": (_int, [_vp, _vp, _vp]),
     "saa_plan_stream": (_vp, [_vp]),
     "saa_step_host": (_int, [_vp, _vp, _vp, _f64, _int, _vp]),
     "saa_step_host_ex": (_int, [_vp, _vp, _vp, _f64, _int, _vp, _int]),
@@ -99,6 +101,9 @@ ENERGY_FIELDS = ("step", "tn", "kinetic_half", "coupling", "strain", "kinetic", 
                  "energy_at_arm")
 ENERGY_DTYPE = np.dtype([("step", np.int64)] + [(f, np.float64) for f in ENERGY_FIELDS[1:]])
 BALANCE_DTYPE = np.dtype(ENERGY_DTYPE.descr + [("total", np.float64), ("residual", np.float64)])
+
+# one element row of StepPlan.element_stress (include/saa_fem.h, SAA_STRESS_FIELDS)
+STRESS_FIELDS = ("sxx", "syy", "szz", "syz", "sxz", "sxy", "von_mises", "weight")
 
 
 def energy_balance(records_per_rank):
@@ -360,10 +365,47 @@ class StepPlan:
         torch.cuda.synchronize(dev)
         _check(lib().saa_plan_set_matfree_dev(self.h, c.shape[0], c.data_ptr(), x.data_ptr(), float(lmd), float(mu)),
                "saa_plan_set_matfree_dev")
+        self.n_elem = int(c.shape[0])
 
     @property
     def matfree_bytes(self):
         return int(lib().saa_plan_matfree_bytes(self.h))
+
+    # ---- stress recovery ---------------------------------------------------------------------------
+    def element_stress(self, out=None):
+        """(n_elem, 8) float64 CUDA tensor of the current d0, one row per element in the order of the cells given to
+        set_matfree: sigma in Voigt order (xx yy zz yz xz xy), von Mises, weight V = detJ/6 (STRESS_FIELDS).  Needs
+        the geometry of set_matfree (the matrix-free step need not be enabled).  Raises SaaError for an element with
+        detJ <= 0.  The values are complete when it returns."""
+        import torch
+        if not hasattr(self, "n_elem"):
+            _check(lib().saa_plan_element_stress_dev(self.h, None), "saa_plan_element_stress_dev")
+        dev = torch.device("cuda", self.device)
+        if out is None:
+            out = torch.empty((self.n_elem, 8), dtype=torch.float64, device=dev)
+        elif out.shape != (self.n_elem, 8) or out.dtype != torch.float64 or out.device != dev or not out.is_contiguous():
+            raise SaaError(f"element_stress: out must be a contiguous float64 ({self.n_elem}, 8) tensor on {dev}")
+        torch.cuda.current_stream(dev).synchronize()          # torch's pending work on `out` precedes the plan's stream
+        _check(lib().saa_plan_element_stress_dev(self.h, out.data_ptr()), "saa_plan_element_stress_dev")
+        return out
+
+    def nodal_stress_partial(self, elem=None):
+        """(n_nodes, 7) float64 CUDA tensor, Local_nodal_list order: this rank's sums of V_e sigma_e (6) and V_e (1)
+        over its elements incident to each node, added in ascending element order.  `elem` is an element_stress
+        result (computed here when not given).  stress.nodal_stress turns it into averaged nodal stresses."""
+        import torch
+        if not hasattr(self, "n_elem"):
+            _check(lib().saa_plan_nodal_stress_dev(self.h, None, None), "saa_plan_nodal_stress_dev")
+        dev = torch.device("cuda", self.device)
+        if elem is None:
+            elem = self.element_stress()
+        elif elem.shape != (self.n_elem, 8) or elem.dtype != torch.float64 or elem.device != dev or not elem.is_contiguous():
+            raise SaaError(f"nodal_stress_partial: elem must be a contiguous float64 ({self.n_elem}, 8) tensor on {dev}")
+        out = torch.empty((self.n_dof // 3, 7), dtype=torch.float64, device=dev)
+        torch.cuda.current_stream(dev).synchronize()
+        _check(lib().saa_plan_nodal_stress_dev(self.h, elem.data_ptr(), out.data_ptr()), "saa_plan_nodal_stress_dev")
+        self.synchronize()
+        return out
 
     def _host_out(self):
         """The array a host call returns d1 in.  From 1 MiB per vector on it is a view of page-locked memory
