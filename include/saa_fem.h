@@ -209,6 +209,44 @@ int64_t saa_plan_matfree_bytes(const saa_plan *plan); /* bytes K5 streams per st
 #define SAA_STRESS_FIELDS 8   /* sxx syy szz syz sxz sxy von_mises weight(detJ/6) */
 int saa_plan_element_stress_dev(saa_plan *plan, double *out_dev);
 int saa_plan_nodal_stress_dev(saa_plan *plan, const double *elem_dev, double *out_dev);
+
+/*
+ * Static solve on the resident stiffness (DESIGN.md §7c).  Both calls read the assembled matrix (refused after
+ * SAA_OPT_MATFREE = 2; any other SAA_OPT_MATFREE value is fine), run after all work enqueued on the plan so far, return
+ * when their results are complete and change no state, clock, hook, history ring, prediction table or energy sum.
+ * Vectors are device memory in local DOF order (Local_nodal_list, 3 per node), n_dof doubles per plan.
+ *
+ * saa_plan_apply_stiffness_dev: y = LocalK x, each row summed over its stored entries in CSR order from 0.0 without FMA
+ *   (a host-built plan gives scipy's LocalK @ x bit for bit).  Shared rows get this rank's partial.
+ * saa_group_apply_stiffness_dev: the same on every plan of a group (x_dev[i], y_dev[i] of rank i), the shared rows then
+ *   hold the sum over their holders in ascending rank order, i.e. f_global[dofs_local] of syn_cpus.
+ *
+ * saa_plan_solve_static_dev: the system of Steady_Elasticity_solver (Tools/Steady_solvers.py:13-22),
+ *     A x = b,   A = S K S + (I - S),   b = S F,
+ *   S keeping the non-Dirichlet DOFs and F the plan's un-ramped load, by conjugate gradients with a 3x3 node-block
+ *   Jacobi preconditioner (the inverse of every node's diagonal block, clamped rows and columns replaced by the
+ *   identity; a block that is not positive definite is refused, naming the rank and local node).
+ *   x0_dev: start vector (NULL: 0; its Dirichlet entries are taken as 0).  x_dev receives the iterate of the first
+ *   iteration with ||r_k||_2 <= rtol ||b||_2, or of iteration max_iter (*converged = 0 then; not an error).
+ *   The host reads the device-resident flags every check_every iterations; a chunk of check_every iterations is one
+ *   CUDA graph (environment SAA_STATIC_GRAPH=0: launched one by one); the result bits depend on neither.
+ *   hist_dev (NULL ok, max_iter doubles): ||r_k||_2 after iteration k = 1, 2, ... at hist_dev[k - 1].
+ *   *iters: iterations run; *rel_res: recurrence ||r|| / ||b||; *rel_res_true: ||b - A x|| / ||b|| from one more apply
+ *   (absolute norms when b = 0).  Fails with the iteration index on a breakdown (p.Ap <= 0, r.z <= 0 before
+ *   convergence, or a non-finite value); never returns non-finite values.  Work vectors (about 64 B per DOF) are
+ *   allocated by the call and released before it returns.  Dot products are summed with fixed trees: repeated calls
+ *   give the same bits.  A plan of a partition with size > 1 is refused here: use the group form.
+ * saa_group_solve_static_dev: the same for the P plans of a group (x0_dev may be NULL or hold NULL entries; x_dev[i]
+ *   of rank i); shared DOFs of x are bit-identical on all their holders.
+ */
+int saa_plan_apply_stiffness_dev(saa_plan *plan, const double *x_dev, double *y_dev);
+int saa_group_apply_stiffness_dev(saa_group *grp, const double *const *x_dev, double *const *y_dev);
+int saa_plan_solve_static_dev(saa_plan *plan, const double *x0_dev, double *x_dev, double rtol, int64_t max_iter,
+                              int64_t check_every, double *hist_dev, int64_t *iters, double *rel_res, double *rel_res_true,
+                              int *converged);
+int saa_group_solve_static_dev(saa_group *grp, const double *const *x0_dev, double *const *x_dev, double rtol,
+                               int64_t max_iter, int64_t check_every, double *hist_dev, int64_t *iters, double *rel_res,
+                               double *rel_res_true, int *converged);
 /* the cudaStream_t the plan enqueues on (as void*), so that callers can record events on it */
 void *saa_plan_stream(saa_plan *plan);
 

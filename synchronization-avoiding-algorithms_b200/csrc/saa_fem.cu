@@ -8,13 +8,16 @@
 #include "saa_energy.cuh"
 #include "saa_matfree.cuh"
 #include "saa_stress.cuh"
+#include "saa_static.cuh"
 
 #include <dlfcn.h>
 
 #include <algorithm>
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <memory>
 #include <numeric>
 #include <string>
 #include <vector>
@@ -1994,4 +1997,315 @@ extern "C" int saa_plan_nodal_stress_dev(saa_plan *p, const double *elem_dev, do
     CK(cudaGetLastError());
     p->launches++;
     return 0;
+}
+
+// ---- static solve on the resident stiffness (saa_static.cuh, DESIGN.md §7c) ------------------------------------
+// Work vectors of one plan for the duration of one call: one allocation, released when the call returns.  H is the
+// plan's halo description with the pack and receive buffers pointed at the call's own scratch, so no buffer of the
+// step path is written.
+struct CgWork {
+    saa_plan *p = nullptr;
+    DevBuf mem;
+    double *x = nullptr, *r = nullptr, *pv = nullptr, *q = nullptr, *z = nullptr, *binv = nullptr, *part = nullptr,
+           *stage = nullptr, *recv = nullptr;
+    uint32_t *free_mask = nullptr;
+    int32_t *ext = nullptr;
+    unsigned int *ticket = nullptr;
+    SaaHaloDev H{};
+    int64_t n_nodes = 0, n_blk = 0, n_units = 0, n_parts = 0;   // blocks of the slice / node kernels, shared-row units
+};
+#define SAA_CG_REDUCE_BLOCKS 256
+
+static int cg_alloc(CgWork &w, saa_plan *p, bool solve, cudaStream_t st)
+{
+    const int64_t n = p->n_rows;
+    w.p = p;
+    w.H = p->H;
+    w.n_nodes = n / 3;
+    w.n_blk = nblk(p->n_slices, 8);                  // = blocks of 256 nodes
+    w.n_units = nblk(p->H.sh_rows, 256);
+    w.n_parts = w.n_blk + w.n_units;
+    size_t off = 0;
+    auto take = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
+    const size_t ox = take(8 * n), oq = take(8 * n);
+    size_t orr = 0, op = 0, oz = 0, ob = 0, opart = 0, ost = 0, ofm = 0, oext = 0, otk = 0;
+    if (solve) {
+        orr = take(8 * n); op = take(8 * n); oz = take(8 * n); ob = take(48 * w.n_nodes); opart = take(16 * w.n_parts);
+        ost = take(16 * SAA_CG_REDUCE_BLOCKS); ofm = take(4 * (n / 32)); oext = take(4 * w.n_nodes); otk = take(4);
+    }
+    const size_t oxb = take(8 * p->H.sh_rows), osend = take(8 * p->total_msg), orecv = take(8 * p->total_msg);
+    if (w.mem.alloc(off)) return -1;
+    char *b = (char *)w.mem.p;
+    w.x = (double *)(b + ox); w.q = (double *)(b + oq);
+    if (solve) {
+        w.r = (double *)(b + orr); w.pv = (double *)(b + op); w.z = (double *)(b + oz); w.binv = (double *)(b + ob);
+        w.part = (double *)(b + opart); w.stage = (double *)(b + ost); w.free_mask = (uint32_t *)(b + ofm);
+        w.ext = (int32_t *)(b + oext); w.ticket = (unsigned int *)(b + otk);
+        CK(cudaMemsetAsync(w.ticket, 0, sizeof(unsigned int), st));   // ordered before the first reduction
+    }
+    w.recv = (double *)(b + orecv);
+    w.H.xbuf = (double *)(b + oxb); w.H.sendbuf = (double *)(b + osend); w.H.recv = w.recv;
+    return 0;
+}
+
+// syn_cpus on vector v of every plan of a group: pack the partial values of the shared rows, move the messages by
+// device copies (as saa_group_step does); saa_k_sum_forces / saa_k_cg_shared then add them in ascending rank order
+static int cg_exchange(CgWork *W, int P, double *CgWork::*v, cudaStream_t st)
+{
+    for (int i = 0; i < P; ++i)
+        if (W[i].H.sh_rows > 0) saa_k_pack_forces<<<nblk(W[i].H.sh_rows, 256), 256, 0, st>>>(W[i].H, W[i].*v);
+    for (int i = 0; i < P; ++i) {
+        const saa_plan *a = W[i].p;
+        for (size_t k = 0; k < a->nb_rank.size(); ++k) {
+            const CgWork &b = W[a->nb_rank[k]];
+            const size_t kk = std::find(b.p->nb_rank.begin(), b.p->nb_rank.end(), (int32_t)i) - b.p->nb_rank.begin();
+            CK(cudaMemcpyAsync(W[i].recv + a->msg_off[k], b.H.sendbuf + b.p->msg_off[kk],
+                               (a->msg_off[k + 1] - a->msg_off[k]) * sizeof(double), cudaMemcpyDeviceToDevice, st));
+        }
+    }
+    CK(cudaGetLastError());
+    return 0;
+}
+
+// out = S K in (DOT, with p.q partials) or b - S K in (RES, with r.r and b.b partials) on every plan, shared rows summed
+template <int MODE>
+static int cg_apply(CgWork *W, int P, double *CgWork::*in, double *CgWork::*out, cudaStream_t st, const long long *gate)
+{
+    for (int i = 0; i < P; ++i)
+        saa_k_cg_apply<MODE><<<W[i].n_blk, 256, 0, st>>>(W[i].p->D, W[i].*in, W[i].*out, W[i].free_mask, W[i].part, W[i].n_parts, gate);
+    if (P > 1) {
+        if (cg_exchange(W, P, out, st)) return -1;
+        for (int i = 0; i < P; ++i)
+            if (W[i].n_units > 0)
+                saa_k_cg_shared<MODE><<<W[i].n_units, 256, 0, st>>>(W[i].p->D, W[i].H, W[i].*in, W[i].*out, W[i].free_mask, W[i].part,
+                                                                    W[i].n_parts, W[i].n_blk, gate);
+    }
+    CK(cudaGetLastError());
+    return 0;
+}
+
+// the partials of the last apply (all n_parts) or update (n_blk, stride n_blk) of every plan -> rank slots rk[f * P + rank]
+template <int NF>
+static void cg_reduce(CgWork *W, int P, bool of_apply, double *rk, cudaStream_t st, const long long *gate)
+{
+    for (int i = 0; i < P; ++i) {
+        const int64_t n = of_apply ? W[i].n_parts : W[i].n_blk;
+        const unsigned G = std::min<unsigned>(nblk(n, 2048), SAA_CG_REDUCE_BLOCKS);
+        saa_k_cg_reduce<NF><<<G, 256, 0, st>>>(W[i].part, n, n, W[i].stage, W[i].ticket, rk + i, P, gate);
+    }
+}
+
+struct GraphExecGuard {
+    cudaGraphExec_t e = nullptr;
+    ~GraphExecGuard() { if (e) cudaGraphExecDestroy(e); }
+};
+
+static int cg_solve(saa_plan *const *plans, int P, const char *name, const double *const *x0, double *const *xout, double rtol,
+                    int64_t max_iter, int64_t check_every, double *hist, int64_t *iters, double *rel_res, double *rel_res_true,
+                    int *converged)
+{
+    if (!(rtol >= 0.0) || !std::isfinite(rtol)) return fail("%s: rtol must be finite and >= 0", name);
+    if (max_iter < 0) return fail("%s: max_iter < 0", name);
+    if (check_every < 1) return fail("%s: check_every must be >= 1", name);
+    for (int i = 0; i < P; ++i) {
+        if (!xout || !xout[i]) return fail("%s: null output", name);
+        if (!plans[i]->d_val) return fail("%s: the assembled matrix of this plan was released (SAA_OPT_MATFREE = 2)", name);
+    }
+    saa_plan *p0 = plans[0];
+    CK(cudaSetDevice(p0->device));
+    for (int i = 0; i < P; ++i) CK(cudaStreamSynchronize(plans[i]->stream));   // earlier work on a plan's own stream
+    const cudaStream_t st = plan_stream(p0);
+    std::unique_ptr<CgWork[]> W(new CgWork[P]);
+    for (int i = 0; i < P; ++i)
+        if (cg_alloc(W[i], plans[i], true, st)) return -1;
+    DevBuf sbuf;                                     // state, rank slots [2][P], bad node per plan
+    if (sbuf.alloc(sizeof(SaaCgState) + 2 * P * sizeof(double) + P * sizeof(unsigned long long))) return -1;
+    SaaCgState *S = sbuf.as<SaaCgState>();
+    double *rk = (double *)(S + 1);
+    unsigned long long *bad = (unsigned long long *)(rk + 2 * P);
+    SaaCgState hs{};
+    hs.rtol = rtol;
+    hs.max_iter = max_iter;
+    CK(cudaMemcpyAsync(S, &hs, sizeof hs, cudaMemcpyHostToDevice, st));
+    CK(cudaMemsetAsync(bad, 0xff, P * sizeof(unsigned long long), st));
+
+    // preconditioner: free rows, diagonal blocks (summed over the holders of a shared node), their inverses
+    for (int i = 0; i < P; ++i) {
+        CgWork &w = W[i];
+        saa_plan *p = w.p;
+        CK(cudaMemsetAsync(w.ext, 0xff, w.n_nodes * sizeof(int32_t), st));
+        saa_k_hp_inverse<<<nblk(p->n_dof / 3, 256), 256, 0, st>>>(p->n_dof / 3, p->d_iperm, w.ext);
+        saa_k_cg_free_mask<<<nblk(p->n_rows / 32, 256), 256, 0, st>>>(p->n_rows / 32, p->d_dir, w.ext, w.free_mask);
+        saa_k_cg_diag<<<w.n_blk, 256, 0, st>>>(p->D, w.x, w.r, w.z);
+    }
+    if (P > 1)
+        for (double *CgWork::*c : {&CgWork::x, &CgWork::r, &CgWork::z}) {
+            if (cg_exchange(W.get(), P, c, st)) return -1;
+            for (int i = 0; i < P; ++i) {
+                saa_k_sum_forces<<<nblk(W[i].p->n_rows, 256), 256, 0, st>>>(W[i].p->n_rows, W[i].H, W[i].*c, W[i].q);
+                CK(cudaMemcpyAsync(W[i].*c, W[i].q, W[i].p->n_rows * sizeof(double), cudaMemcpyDeviceToDevice, st));
+            }
+        }
+    for (int i = 0; i < P; ++i)
+        saa_k_cg_binv<<<nblk(W[i].n_nodes, 256), 256, 0, st>>>(W[i].n_nodes, W[i].x, W[i].r, W[i].z, W[i].free_mask, W[i].ext,
+                                                               W[i].binv, bad + i);
+    CK(cudaGetLastError());
+    std::vector<unsigned long long> bad_h(P);
+    CK(cudaMemcpyAsync(bad_h.data(), bad, P * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    for (int i = 0; i < P; ++i)
+        if (bad_h[i] != ~0ull)
+            return fail("%s: rank %d, local node %llu: its diagonal 3x3 block (clamped rows and columns replaced by the identity) "
+                        "is not positive definite, Cholesky fails", name, plans[i]->rank, bad_h[i]);
+
+    // x = S x0, r = b - A x, z = B^-1 r, p = z
+    for (int i = 0; i < P; ++i) {
+        CgWork &w = W[i];
+        CK(cudaMemsetAsync(w.x, 0, w.p->n_rows * sizeof(double), st));
+        if (x0 && x0[i]) {
+            saa_k_scatter_to_internal<<<nblk(w.p->n_dof, 256), 256, 0, st>>>(w.p->n_dof, w.p->d_iperm, x0[i], w.x);
+            saa_k_cg_mask<<<nblk(w.p->n_rows, 256), 256, 0, st>>>(w.p->n_rows, w.free_mask, w.x);
+        }
+    }
+    if (cg_apply<SAA_APPLY_RES>(W.get(), P, &CgWork::x, &CgWork::r, st, nullptr)) return -1;
+    cg_reduce<2>(W.get(), P, true, rk, st, nullptr);
+    saa_k_cg_scalar<<<1, 32, 0, st>>>(S, rk, P, SAA_CG_RES0, hist);
+    for (int i = 0; i < P; ++i)
+        saa_k_cg_update<true><<<W[i].n_blk, 256, 0, st>>>(W[i].n_nodes, W[i].H, S, W[i].x, W[i].r, W[i].pv, W[i].q, W[i].z, W[i].binv,
+                                                          W[i].free_mask, W[i].part, W[i].n_blk);
+    cg_reduce<2>(W.get(), P, false, rk, st, nullptr);
+    saa_k_cg_scalar<<<1, 32, 0, st>>>(S, rk, P, SAA_CG_INIT, hist);
+    CK(cudaGetLastError());
+
+    const long long *gate = &S->done;
+    auto iteration = [&]() -> int {
+        if (cg_apply<SAA_APPLY_DOT>(W.get(), P, &CgWork::pv, &CgWork::q, st, gate)) return -1;
+        cg_reduce<1>(W.get(), P, true, rk, st, gate);
+        saa_k_cg_scalar<<<1, 32, 0, st>>>(S, rk, P, SAA_CG_ALPHA, hist);
+        for (int i = 0; i < P; ++i)
+            saa_k_cg_update<false><<<W[i].n_blk, 256, 0, st>>>(W[i].n_nodes, W[i].H, S, W[i].x, W[i].r, W[i].pv, W[i].q, W[i].z,
+                                                               W[i].binv, W[i].free_mask, W[i].part, W[i].n_blk);
+        cg_reduce<2>(W.get(), P, false, rk, st, gate);
+        saa_k_cg_scalar<<<1, 32, 0, st>>>(S, rk, P, SAA_CG_BETA, hist);
+        for (int i = 0; i < P; ++i)
+            saa_k_cg_direction<<<nblk(W[i].p->n_rows, 256), 256, 0, st>>>(W[i].p->n_rows, S, W[i].z, W[i].pv);
+        CK(cudaGetLastError());
+        return 0;
+    };
+    // a chunk of check_every iterations, replayed from one CUDA graph (SAA_STATIC_GRAPH=0: launched one by one)
+    const int64_t chunk = std::min<int64_t>(check_every, std::max<int64_t>(max_iter, 1));
+    const char *ge = getenv("SAA_STATIC_GRAPH");
+    GraphExecGuard exec;
+    if (max_iter > 0 && !(ge && ge[0] == '0')) {
+        cudaGraph_t g;
+        CK(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
+        int rc = 0;
+        for (int64_t c = 0; c < chunk && rc == 0; ++c) rc = iteration();
+        CK(cudaStreamEndCapture(st, &g));
+        if (rc) { cudaGraphDestroy(g); return -1; }
+        const cudaError_t e = cudaGraphInstantiate(&exec.e, g, 0);
+        cudaGraphDestroy(g);
+        CK(e);
+    }
+    auto read_state = [&]() -> int {
+        CK(cudaMemcpyAsync(&hs, S, sizeof hs, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        return 0;
+    };
+    if (read_state()) return -1;
+    for (int64_t launched = 0; !hs.done && launched < max_iter; launched += chunk) {
+        if (exec.e) {
+            CK(cudaGraphLaunch(exec.e, st));
+        } else {
+            for (int64_t c = 0; c < chunk; ++c)
+                if (iteration()) return -1;
+        }
+        if (read_state()) return -1;
+    }
+    if (hs.fail) {
+        const char *what = hs.fail == 1 ? "p.Ap <= 0 or not finite (A is not positive definite on the free DOFs)"
+                         : hs.fail == 2 ? "r.z <= 0 or not finite before convergence" : "non-finite residual";
+        return fail("%s: breakdown at iteration %lld: %s", name, hs.fail_it, what);
+    }
+    // the true residual b - A x of the returned iterate, and x in local DOF order
+    if (cg_apply<SAA_APPLY_RES>(W.get(), P, &CgWork::x, &CgWork::q, st, nullptr)) return -1;
+    cg_reduce<2>(W.get(), P, true, rk, st, nullptr);
+    saa_k_cg_scalar<<<1, 32, 0, st>>>(S, rk, P, SAA_CG_TRUE, hist);
+    for (int i = 0; i < P; ++i)
+        saa_k_gather_to_external<<<nblk(W[i].p->n_dof, 256), 256, 0, st>>>(W[i].p->n_dof, W[i].p->d_iperm, W[i].x, xout[i]);
+    CK(cudaGetLastError());
+    if (read_state()) return -1;
+    const double bn = std::sqrt(hs.bb);
+    if (iters) *iters = hs.it;
+    if (rel_res) *rel_res = bn > 0.0 ? std::sqrt(hs.rr) / bn : std::sqrt(hs.rr);
+    if (rel_res_true) *rel_res_true = bn > 0.0 ? std::sqrt(hs.rr_true) / bn : std::sqrt(hs.rr_true);
+    if (converged) *converged = (int)hs.converged;
+    return 0;
+}
+
+extern "C" int saa_plan_solve_static_dev(saa_plan *p, const double *x0_dev, double *x_dev, double rtol, int64_t max_iter,
+                                         int64_t check_every, double *hist_dev, int64_t *iters, double *rel_res,
+                                         double *rel_res_true, int *converged)
+{
+    NEED_FINAL(p, "saa_plan_solve_static_dev");
+    if (p->size > 1)
+        return fail("saa_plan_solve_static_dev: this plan is rank %d of a partition of size %d; solve all ranks together with "
+                    "saa_group_solve_static_dev (the peer, NCCL and host-staged transports are not supported by the static solve)",
+                    p->rank, p->size);
+    return cg_solve(&p, 1, "saa_plan_solve_static_dev", &x0_dev, &x_dev, rtol, max_iter, check_every, hist_dev, iters, rel_res,
+                    rel_res_true, converged);
+}
+
+extern "C" int saa_group_solve_static_dev(saa_group *g, const double *const *x0_dev, double *const *x_dev, double rtol,
+                                          int64_t max_iter, int64_t check_every, double *hist_dev, int64_t *iters,
+                                          double *rel_res, double *rel_res_true, int *converged)
+{
+    if (!g) return fail("saa_group_solve_static_dev: null group");
+    return cg_solve(g->plans.data(), (int)g->plans.size(), "saa_group_solve_static_dev", x0_dev, x_dev, rtol, max_iter,
+                    check_every, hist_dev, iters, rel_res, rel_res_true, converged);
+}
+
+// y = LocalK x of every plan (local DOF order); with `sum`, the shared rows hold the rank-ordered holder sums
+static int apply_stiffness(saa_plan *const *plans, int P, const char *name, const double *const *x, double *const *y, bool sum)
+{
+    for (int i = 0; i < P; ++i) {
+        if (!x || !y || !x[i] || !y[i]) return fail("%s: null argument", name);
+        if (!plans[i]->d_val) return fail("%s: the assembled matrix of this plan was released (SAA_OPT_MATFREE = 2)", name);
+    }
+    CK(cudaSetDevice(plans[0]->device));
+    for (int i = 0; i < P; ++i) CK(cudaStreamSynchronize(plans[i]->stream));
+    const cudaStream_t st = plan_stream(plans[0]);
+    std::unique_ptr<CgWork[]> W(new CgWork[P]);
+    for (int i = 0; i < P; ++i) {
+        CgWork &w = W[i];
+        saa_plan *p = plans[i];
+        if (cg_alloc(w, p, false, st)) return -1;
+        CK(cudaMemsetAsync(w.x, 0, p->n_rows * sizeof(double), st));   // slice padding: finite, multiplied by 0.0
+        saa_k_scatter_to_internal<<<nblk(p->n_dof, 256), 256, 0, st>>>(p->n_dof, p->d_iperm, x[i], w.x);
+        saa_k_cg_apply<SAA_APPLY_RAW><<<w.n_blk, 256, 0, st>>>(p->D, w.x, w.q, nullptr, nullptr, 0, nullptr);
+    }
+    double *CgWork::*res = &CgWork::q;
+    if (sum) {
+        if (cg_exchange(W.get(), P, &CgWork::q, st)) return -1;
+        for (int i = 0; i < P; ++i)
+            saa_k_sum_forces<<<nblk(W[i].p->n_rows, 256), 256, 0, st>>>(W[i].p->n_rows, W[i].H, W[i].q, W[i].x);
+        res = &CgWork::x;
+    }
+    for (int i = 0; i < P; ++i)
+        saa_k_gather_to_external<<<nblk(plans[i]->n_dof, 256), 256, 0, st>>>(plans[i]->n_dof, plans[i]->d_iperm, W[i].*res, y[i]);
+    CK(cudaGetLastError());
+    CK(cudaStreamSynchronize(st));
+    return 0;
+}
+
+extern "C" int saa_plan_apply_stiffness_dev(saa_plan *p, const double *x_dev, double *y_dev)
+{
+    NEED_FINAL(p, "saa_plan_apply_stiffness_dev");
+    return apply_stiffness(&p, 1, "saa_plan_apply_stiffness_dev", &x_dev, &y_dev, false);
+}
+
+extern "C" int saa_group_apply_stiffness_dev(saa_group *g, const double *const *x_dev, double *const *y_dev)
+{
+    if (!g) return fail("saa_group_apply_stiffness_dev: null group");
+    return apply_stiffness(g->plans.data(), (int)g->plans.size(), "saa_group_apply_stiffness_dev", x_dev, y_dev, true);
 }

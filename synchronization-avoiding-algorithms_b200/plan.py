@@ -62,6 +62,10 @@ ABI = {
     "saa_plan_matfree_bytes": (_i64, [_vp]),
     "saa_plan_element_stress_dev": (_int, [_vp, _vp]),
     "saa_plan_nodal_stress_dev": (_int, [_vp, _vp, _vp]),
+    "saa_plan_apply_stiffness_dev": (_int, [_vp, _vp, _vp]),
+    "saa_group_apply_stiffness_dev": (_int, [_vp, _vp, _vp]),
+    "saa_plan_solve_static_dev": (_int, [_vp, _vp, _vp, _f64, _i64, _i64, _vp, _vp, _vp, _vp, _vp]),
+    "saa_group_solve_static_dev": (_int, [_vp, _vp, _vp, _f64, _i64, _i64, _vp, _vp, _vp, _vp, _vp]),
     "saa_plan_stream": (_vp, [_vp]),
     "saa_step_host": (_int, [_vp, _vp, _vp, _f64, _int, _vp]),
     "saa_step_host_ex": (_int, [_vp, _vp, _vp, _f64, _int, _vp, _int]),
@@ -125,6 +129,60 @@ def energy_balance(records_per_rank):
     out["total"] = out["kinetic_half"] + out["coupling"]
     out["residual"] = out["total"] - out["energy_at_arm"] - out["work_external"] + out["work_damping"]
     return out
+
+
+class StaticResult:
+    """Result of StepPlan.solve_static / PlanGroup.solve_static.
+    x                  solution in local DOF order: a float64 CUDA tensor, or a list of them (one per plan of a group)
+    iterations         CG iterations run
+    rel_residual       ||r|| / ||b|| of the CG recurrence at the returned iterate
+    rel_residual_true  ||b - A x|| / ||b|| from one more stiffness apply
+    converged          rel_residual <= rtol was reached within max_iter
+    history            float64 CUDA tensor (iterations,): ||r_k|| after iteration k = 1, 2, ..."""
+
+    def __init__(self, x, iterations, rel_residual, rel_residual_true, converged, history):
+        self.x, self.iterations, self.history = x, iterations, history
+        self.rel_residual, self.rel_residual_true, self.converged = rel_residual, rel_residual_true, converged
+
+    def __repr__(self):
+        return (f"StaticResult(iterations={self.iterations}, rel_residual={self.rel_residual:.3e}, "
+                f"rel_residual_true={self.rel_residual_true:.3e}, converged={self.converged})")
+
+
+def _dev_vector(t, n, device, what):
+    """t checked as a contiguous float64 CUDA tensor of n entries on `device`"""
+    import torch
+    dev = torch.device("cuda", device)
+    if not isinstance(t, torch.Tensor) or t.dtype != torch.float64 or t.device != dev or t.numel() != n or not t.is_contiguous():
+        raise SaaError(f"{what}: need a contiguous float64 tensor of {n} entries on {dev}")
+    return t
+
+
+# default iteration cap of solve_static: the history takes max_iter doubles on the device during the call (8 MB here)
+MAX_ITER_DEFAULT = 1_000_000
+
+
+def _solve_static(fn, handle, plans, rtol, max_iter, x0, check_every):
+    import torch
+    dev = torch.device("cuda", plans[0].device)
+    max_iter = min(10 * sum(pl.n_dof for pl in plans), MAX_ITER_DEFAULT) if max_iter is None else int(max_iter)
+    x0 = [None] * len(plans) if x0 is None else list(x0)
+    if len(x0) != len(plans):
+        raise SaaError(f"solve_static: x0 needs one vector per plan ({len(plans)})")
+    x0 = [None if v is None else _dev_vector(v, pl.n_dof, pl.device, "solve_static: x0") for v, pl in zip(x0, plans)]
+    xs = [torch.empty(pl.n_dof, dtype=torch.float64, device=dev) for pl in plans]
+    hist = torch.empty(max(max_iter, 1), dtype=torch.float64, device=dev)
+    ptrs = lambda ts: (ctypes.c_void_p * len(ts))(*[None if t is None else t.data_ptr() for t in ts])
+    it, rel, rel_true, conv = ctypes.c_int64(0), ctypes.c_double(0), ctypes.c_double(0), ctypes.c_int(0)
+    torch.cuda.current_stream(dev).synchronize()              # torch's pending work on x0 precedes the plans' stream
+    args = (float(rtol), max_iter, int(check_every), hist.data_ptr(), ctypes.byref(it), ctypes.byref(rel),
+            ctypes.byref(rel_true), ctypes.byref(conv))
+    if handle is None:
+        _check(fn(plans[0].h, None if x0[0] is None else x0[0].data_ptr(), xs[0].data_ptr(), *args), "saa_plan_solve_static_dev")
+    else:
+        _check(fn(handle, ptrs(x0), ptrs(xs), *args), "saa_group_solve_static_dev")
+    return StaticResult(xs[0] if handle is None else xs, int(it.value), rel.value, rel_true.value, bool(conv.value),
+                        hist[:int(it.value)].clone())        # the max_iter-long buffer is released
 
 
 PINNED_POOL = 4
@@ -407,6 +465,26 @@ class StepPlan:
         self.synchronize()
         return out
 
+    # ---- static solve ------------------------------------------------------------------------------
+    def apply_stiffness(self, x):
+        """y = LocalK x (float64 CUDA tensors of n_dof, local DOF order), bit for bit scipy's LocalK @ x on a host-built
+        plan.  Shared rows of a partition hold this rank's partial (PlanGroup.apply_stiffness sums them)."""
+        import torch
+        x = _dev_vector(x, self.n_dof, self.device, "apply_stiffness: x")
+        y = torch.empty_like(x)
+        torch.cuda.current_stream(x.device).synchronize()
+        _check(lib().saa_plan_apply_stiffness_dev(self.h, x.data_ptr(), y.data_ptr()), "saa_plan_apply_stiffness_dev")
+        return y
+
+    def solve_static(self, rtol=1e-10, max_iter=None, x0=None, check_every=50):
+        """Solve the steady system of Steady_Elasticity_solver, (S K S + I - S) x = S F, on the device by block-Jacobi
+        preconditioned CG (DESIGN.md §7c).  max_iter defaults to 10 n_dof, at most MAX_ITER_DEFAULT (CG in floating
+        point needs more than n_dof iterations on an ill-conditioned system); x0: start tensor (None: 0).  Returns a
+        StaticResult; not converging within max_iter is not an error (converged=False).  A plan of a partition with
+        size > 1 is solved through PlanGroup.solve_static."""
+        return _solve_static(lib().saa_plan_solve_static_dev, None, [self], rtol, max_iter, None if x0 is None else [x0],
+                             check_every)
+
     def _host_out(self):
         """The array a host call returns d1 in.  From 1 MiB per vector on it is a view of page-locked memory
         (saa_host_alloc), so that this download and — once the caller has rotated it into d_0 / d_n
@@ -604,6 +682,24 @@ class PlanGroup:
 
     def synchronize(self):
         _check(lib().saa_group_synchronize(self.h), "saa_group_synchronize")
+
+    def apply_stiffness(self, xs):
+        """[LocalK_r x_r] of every plan with the shared rows summed over their holders in ascending rank order
+        (f_global[dofs_local] of syn_cpus): list of float64 CUDA tensors, local DOF order."""
+        import torch
+        if len(xs) != len(self.plans):
+            raise SaaError(f"apply_stiffness: need one vector per plan ({len(self.plans)})")
+        xs = [_dev_vector(x, pl.n_dof, pl.device, "apply_stiffness: x") for x, pl in zip(xs, self.plans)]
+        ys = [torch.empty_like(x) for x in xs]
+        ptrs = lambda ts: (ctypes.c_void_p * len(ts))(*[t.data_ptr() for t in ts])
+        torch.cuda.current_stream(xs[0].device).synchronize()
+        _check(lib().saa_group_apply_stiffness_dev(self.h, ptrs(xs), ptrs(ys)), "saa_group_apply_stiffness_dev")
+        return ys
+
+    def solve_static(self, rtol=1e-10, max_iter=None, x0=None, check_every=50):
+        """StepPlan.solve_static over all partitions of the group; x0 and the result's x are lists, one per plan.
+        max_iter defaults to 10 times the sum of the plans' n_dof, at most MAX_ITER_DEFAULT."""
+        return _solve_static(lib().saa_group_solve_static_dev, self.h, self.plans, rtol, max_iter, x0, check_every)
 
     def close(self):
         if getattr(self, "h", None):
