@@ -35,6 +35,7 @@ extern "C" {
 typedef struct saa_plan saa_plan;     /* one partition's device-resident problem + state */
 typedef struct saa_group saa_group;   /* several plans of ONE process stepped together (halo exchange by
                                          device copies) — used to run a P-way partition on fewer GPUs */
+typedef struct saa_mg saa_mg;         /* multigrid hierarchy over plans of nested meshes (saa_mg_create) */
 
 /* step modes (MODEL / size arguments of Dynamic_solver.py:9-10,22,25) */
 #define SAA_MODE_LOCAL 0      /* size == 1, or MODEL=True: no exchange, F_int = LocalK.dot(d0)            */
@@ -247,6 +248,41 @@ int saa_plan_solve_static_dev(saa_plan *plan, const double *x0_dev, double *x_de
 int saa_group_solve_static_dev(saa_group *grp, const double *const *x0_dev, double *const *x_dev, double rtol,
                                int64_t max_iter, int64_t check_every, double *hist_dev, int64_t *iters, double *rel_res,
                                double *rel_res_true, int *converged);
+
+/*
+ * Geometric multigrid preconditioner for the static solve (DESIGN.md §7d): one V-cycle per CG iteration over a hierarchy
+ * of nested meshes, each level a finalized plan of size 1 (levels[0] the fine plan, then ever coarser ones) whose
+ * stiffness is the Galerkin operator P^T K P of the level above.  Only size-1 plans with their assembled matrix
+ * (not SAA_OPT_MATFREE = 2), all on one device, are accepted.
+ *
+ * saa_mg_create: p_ptr[l], p_col[l], p_w[l] (device memory, l = 0 .. n_levels - 2) is the prolongation from level l + 1
+ *   to level l as a node CSR in the plans' external local node numbering: fine node e of level l gets
+ *   sum_k p_w[l][k] x_c(p_col[l][k]) for k in [p_ptr[l][e], p_ptr[l][e + 1]), the same weight on all three components
+ *   (p_ptr[l]: n_dof_l / 3 + 1 int64, p_col[l]: int32).  coarse_inv_dev is A^-1 of the coarsest level, dense, row-major,
+ *   in its external DOF order (n_dof x n_dof doubles, copied; at most coarsest_max_dof DOF).  Smoothing is Chebyshev of
+ *   `degree` (>= 1) on [0.3, 1.1] x lambda with the level's 3x3 node-block Jacobi, before and after the coarse
+ *   correction; lambda estimates lambda_max(B^-1 A) by power_iters (>= 1) power steps from a fixed start vector.  The
+ *   set-up is bit-reproducible.  A diagonal block that is not positive definite is refused, naming the level and node.
+ * saa_mg_info: lambda[l] of every level (n_levels doubles, NULL ok) and the device bytes the hierarchy holds itself
+ *   (NULL ok; the plans' own memory not included).
+ * saa_plan_solve_static_mg_dev: saa_plan_solve_static_dev on levels[0], preconditioned by the V-cycle instead of the
+ *   block-Jacobi step; same arguments, contract and determinism.  Its work vectors (5 per DOF of the fine plan) are
+ *   allocated by the call and released before it returns; no state, clock, hook, history ring, prediction table or
+ *   energy sum of any level changes.
+ * saa_mg_vcycle_dev, saa_mg_prolong_dev, saa_mg_restrict_dev (external local DOF order, device memory):
+ *   z = V r on the free DOFs of levels[0];  x_f = S_f P x_c and b_c = S_c P^T r_f between levels `level` (fine) and
+ *   `level` + 1 (S: the level's free DOFs).  They return when the result is complete.
+ */
+int saa_mg_create(saa_mg **out, saa_plan *const *levels, int n_levels, const int64_t *const *p_ptr, const int32_t *const *p_col,
+                  const double *const *p_w, const double *coarse_inv_dev, int degree, int power_iters, int64_t coarsest_max_dof);
+int saa_mg_destroy(saa_mg *mg);
+int saa_mg_info(const saa_mg *mg, double *lambda, int64_t *bytes);
+int saa_plan_solve_static_mg_dev(saa_mg *mg, const double *x0_dev, double *x_dev, double rtol, int64_t max_iter,
+                                 int64_t check_every, double *hist_dev, int64_t *iters, double *rel_res, double *rel_res_true,
+                                 int *converged);
+int saa_mg_vcycle_dev(saa_mg *mg, const double *r_dev, double *z_dev);
+int saa_mg_prolong_dev(saa_mg *mg, int level, const double *xc_dev, double *xf_dev);
+int saa_mg_restrict_dev(saa_mg *mg, int level, const double *rf_dev, double *bc_dev);
 /* the cudaStream_t the plan enqueues on (as void*), so that callers can record events on it */
 void *saa_plan_stream(saa_plan *plan);
 

@@ -9,6 +9,7 @@
 #include "saa_matfree.cuh"
 #include "saa_stress.cuh"
 #include "saa_static.cuh"
+#include "saa_multigrid.cuh"
 
 #include <dlfcn.h>
 
@@ -2100,6 +2101,50 @@ struct GraphExecGuard {
     ~GraphExecGuard() { if (e) cudaGraphExecDestroy(e); }
 };
 
+// The iterations of a solve: chunks of check_every iterations, each replayed from one CUDA graph (SAA_STATIC_GRAPH=0:
+// launched one by one), until the device-resident flags say done; hs then holds the final state.  A breakdown fails
+// the call with its iteration index.
+template <class Iteration>
+static int cg_iterate(Iteration &iteration, const char *name, cudaStream_t st, SaaCgState *S, SaaCgState &hs, int64_t max_iter,
+                      int64_t check_every)
+{
+    const int64_t chunk = std::min<int64_t>(check_every, std::max<int64_t>(max_iter, 1));
+    const char *ge = getenv("SAA_STATIC_GRAPH");
+    GraphExecGuard exec;
+    if (max_iter > 0 && !(ge && ge[0] == '0')) {
+        cudaGraph_t g;
+        CK(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
+        int rc = 0;
+        for (int64_t c = 0; c < chunk && rc == 0; ++c) rc = iteration();
+        CK(cudaStreamEndCapture(st, &g));
+        if (rc) { cudaGraphDestroy(g); return -1; }
+        const cudaError_t e = cudaGraphInstantiate(&exec.e, g, 0);
+        cudaGraphDestroy(g);
+        CK(e);
+    }
+    auto read_state = [&]() -> int {
+        CK(cudaMemcpyAsync(&hs, S, sizeof hs, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        return 0;
+    };
+    if (read_state()) return -1;
+    for (int64_t launched = 0; !hs.done && launched < max_iter; launched += chunk) {
+        if (exec.e) {
+            CK(cudaGraphLaunch(exec.e, st));
+        } else {
+            for (int64_t c = 0; c < chunk; ++c)
+                if (iteration()) return -1;
+        }
+        if (read_state()) return -1;
+    }
+    if (hs.fail) {
+        const char *what = hs.fail == 1 ? "p.Ap <= 0 or not finite (A is not positive definite on the free DOFs)"
+                         : hs.fail == 2 ? "r.z <= 0 or not finite before convergence" : "non-finite residual";
+        return fail("%s: breakdown at iteration %lld: %s", name, hs.fail_it, what);
+    }
+    return 0;
+}
+
 static int cg_solve(saa_plan *const *plans, int P, const char *name, const double *const *x0, double *const *xout, double rtol,
                     int64_t max_iter, int64_t check_every, double *hist, int64_t *iters, double *rel_res, double *rel_res_true,
                     int *converged)
@@ -2192,41 +2237,12 @@ static int cg_solve(saa_plan *const *plans, int P, const char *name, const doubl
         CK(cudaGetLastError());
         return 0;
     };
-    // a chunk of check_every iterations, replayed from one CUDA graph (SAA_STATIC_GRAPH=0: launched one by one)
-    const int64_t chunk = std::min<int64_t>(check_every, std::max<int64_t>(max_iter, 1));
-    const char *ge = getenv("SAA_STATIC_GRAPH");
-    GraphExecGuard exec;
-    if (max_iter > 0 && !(ge && ge[0] == '0')) {
-        cudaGraph_t g;
-        CK(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-        int rc = 0;
-        for (int64_t c = 0; c < chunk && rc == 0; ++c) rc = iteration();
-        CK(cudaStreamEndCapture(st, &g));
-        if (rc) { cudaGraphDestroy(g); return -1; }
-        const cudaError_t e = cudaGraphInstantiate(&exec.e, g, 0);
-        cudaGraphDestroy(g);
-        CK(e);
-    }
+    if (cg_iterate(iteration, name, st, S, hs, max_iter, check_every)) return -1;
     auto read_state = [&]() -> int {
         CK(cudaMemcpyAsync(&hs, S, sizeof hs, cudaMemcpyDeviceToHost, st));
         CK(cudaStreamSynchronize(st));
         return 0;
     };
-    if (read_state()) return -1;
-    for (int64_t launched = 0; !hs.done && launched < max_iter; launched += chunk) {
-        if (exec.e) {
-            CK(cudaGraphLaunch(exec.e, st));
-        } else {
-            for (int64_t c = 0; c < chunk; ++c)
-                if (iteration()) return -1;
-        }
-        if (read_state()) return -1;
-    }
-    if (hs.fail) {
-        const char *what = hs.fail == 1 ? "p.Ap <= 0 or not finite (A is not positive definite on the free DOFs)"
-                         : hs.fail == 2 ? "r.z <= 0 or not finite before convergence" : "non-finite residual";
-        return fail("%s: breakdown at iteration %lld: %s", name, hs.fail_it, what);
-    }
     // the true residual b - A x of the returned iterate, and x in local DOF order
     if (cg_apply<SAA_APPLY_RES>(W.get(), P, &CgWork::x, &CgWork::q, st, nullptr)) return -1;
     cg_reduce<2>(W.get(), P, true, rk, st, nullptr);
@@ -2308,4 +2324,387 @@ extern "C" int saa_group_apply_stiffness_dev(saa_group *g, const double *const *
 {
     if (!g) return fail("saa_group_apply_stiffness_dev: null group");
     return apply_stiffness(g->plans.data(), (int)g->plans.size(), "saa_group_apply_stiffness_dev", x_dev, y_dev, true);
+}
+
+// ---- geometric multigrid preconditioner (saa_multigrid.cuh, DESIGN.md §7d) -------------------------------------------
+// One level: its plan, the block-Jacobi inverse and free rows (w: the fields cg_apply / cg_reduce use, w.x / w.q point
+// at r / d for the power iteration), the level's vectors and the tables that connect it to its neighbours.
+struct MgLevel {
+    saa_plan *p = nullptr;
+    DevBuf mem, tab, ttab;
+    CgWork w;
+    double *x = nullptr, *b = nullptr, *r = nullptr, *d = nullptr, *slot = nullptr;   // x, b: coarse levels only
+    double lam = 0.0;
+    std::vector<double> c1, c2;                                         // Chebyshev step k: d = c1 d + c2 B^-1 r
+    int64_t *p_ptr = nullptr; int32_t *p_cnode = nullptr; double *p_w = nullptr;    // prolongation from level + 1
+    int64_t *t_ptr = nullptr; int32_t *t_fnode = nullptr; double *t_w = nullptr;    // restriction from level - 1
+};
+struct saa_mg {
+    int n = 0;
+    std::unique_ptr<MgLevel[]> L;
+    DevBuf cinv;                                                        // A^-1 of the coarsest level, internal order
+    int64_t bytes = 0;
+};
+
+// Chebyshev polynomial of `degree` steps on [0.3, 1.1] x lam (the smoother of PETSc's PCMG default): step 0 is
+// d = B^-1 r / theta, step k > 0 d = rho_k rho_{k-1} d + 2 rho_k / delta B^-1 r with rho_k = 1 / (2 sigma - rho_{k-1})
+static void mg_chebyshev(MgLevel &l, int degree)
+{
+    const double hi = 1.1 * l.lam, lo = 0.3 * l.lam, theta = 0.5 * (hi + lo), delta = 0.5 * (hi - lo), sigma = theta / delta;
+    double rho = 1.0 / sigma;
+    l.c1.assign(degree, 0.0);
+    l.c2.assign(degree, 1.0 / theta);
+    for (int k = 1; k < degree; ++k) {
+        const double rn = 1.0 / (2.0 * sigma - rho);
+        l.c1[k] = rn * rho;
+        l.c2[k] = 2.0 * rn / delta;
+        rho = rn;
+    }
+}
+
+// x = V b on level l (b, x: level vectors in internal order, b zero on non-free rows)
+static void mg_vcycle(saa_mg *mg, int l, const double *b, double *x, cudaStream_t st, const long long *gate)
+{
+    MgLevel &L = mg->L[l];
+    const SaaDev &D = L.p->D;
+    const int64_t nn = L.w.n_nodes;
+    const unsigned gs = (unsigned)L.w.n_blk, gn = nblk(nn, 256);
+    if (l == mg->n - 1) {
+        saa_k_mg_coarse<<<nblk(L.p->n_rows, 8), 256, 0, st>>>(L.p->n_rows, mg->cinv.as<double>(), b, x, L.w.free_mask, gate);
+        return;
+    }
+    const int deg = (int)L.c2.size();
+    auto residual = [&]() { saa_k_mg_residual<<<gs, 256, 0, st>>>(D, x, b, L.r, L.w.free_mask, gate); };
+    auto next_steps = [&]() {
+        for (int k = 1; k < deg; ++k) {
+            residual();
+            saa_k_mg_cheb<SAA_MG_CHEB_NEXT><<<gn, 256, 0, st>>>(nn, L.r, L.d, x, L.w.binv, L.w.free_mask, L.c1[k], L.c2[k], gate);
+        }
+    };
+    saa_k_mg_cheb<SAA_MG_CHEB_FIRST_ZERO><<<gn, 256, 0, st>>>(nn, b, L.d, x, L.w.binv, L.w.free_mask, 0.0, L.c2[0], gate);
+    next_steps();
+    residual();
+    MgLevel &C = mg->L[l + 1];
+    saa_k_mg_restrict<<<nblk(C.w.n_nodes, 256), 256, 0, st>>>(C.w.n_nodes, C.w.ext, C.t_ptr, C.t_fnode, C.t_w, L.r, C.b,
+                                                              C.w.free_mask, gate);
+    mg_vcycle(mg, l + 1, C.b, C.x, st, gate);
+    saa_k_mg_prolong<<<gn, 256, 0, st>>>(nn, L.w.ext, L.p_ptr, L.p_cnode, L.p_w, C.x, x, L.w.free_mask, gate);
+    residual();
+    saa_k_mg_cheb<SAA_MG_CHEB_FIRST><<<gn, 256, 0, st>>>(nn, L.r, L.d, x, L.w.binv, L.w.free_mask, 0.0, L.c2[0], gate);
+    next_steps();
+}
+
+// level l's memory, free rows, block-Jacobi inverse and lambda_max(B^-1 A)
+static int mg_level_setup(saa_mg *mg, int l, saa_plan *p, int power_iters, cudaStream_t st)
+{
+    MgLevel &L = mg->L[l];
+    CgWork &w = L.w;
+    const int64_t n = p->n_rows;
+    L.p = w.p = p;
+    w.H = p->H;
+    w.n_nodes = n / 3;
+    w.n_blk = nblk(p->n_slices, 8);
+    w.n_units = 0;
+    w.n_parts = w.n_blk;
+    size_t off = 0;
+    auto take = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
+    const bool own_xb = l > 0;
+    const size_t ox = own_xb ? take(8 * n) : 0, ob = own_xb ? take(8 * n) : 0, orr = take(8 * n), od = take(8 * n);
+    const size_t obinv = take(48 * w.n_nodes), opart = take(16 * w.n_parts), ost = take(16 * SAA_CG_REDUCE_BLOCKS);
+    const size_t ofm = take(4 * (n / 32)), oext = take(4 * w.n_nodes), otk = take(4), osl = take(16), obad = take(8);
+    if (L.mem.alloc(off)) return -1;
+    mg->bytes += off;
+    char *base = (char *)L.mem.p;
+    if (own_xb) { L.x = (double *)(base + ox); L.b = (double *)(base + ob); }
+    L.r = (double *)(base + orr); L.d = (double *)(base + od);
+    w.binv = (double *)(base + obinv); w.part = (double *)(base + opart); w.stage = (double *)(base + ost);
+    w.free_mask = (uint32_t *)(base + ofm); w.ext = (int32_t *)(base + oext); w.ticket = (unsigned int *)(base + otk);
+    L.slot = (double *)(base + osl);
+    unsigned long long *bad = (unsigned long long *)(base + obad);
+    w.x = L.r; w.q = L.d;
+    CK(cudaMemsetAsync(w.ticket, 0, sizeof(unsigned int), st));
+    CK(cudaMemsetAsync(bad, 0xff, sizeof(unsigned long long), st));
+    CK(cudaMemsetAsync(w.ext, 0xff, w.n_nodes * sizeof(int32_t), st));
+    saa_k_hp_inverse<<<nblk(p->n_dof / 3, 256), 256, 0, st>>>(p->n_dof / 3, p->d_iperm, w.ext);
+    saa_k_cg_free_mask<<<nblk(n / 32, 256), 256, 0, st>>>(n / 32, p->d_dir, w.ext, w.free_mask);
+    {
+        DevBuf cols;                                   // the diagonal blocks' three columns
+        if (cols.alloc(3 * 8 * n)) return -1;
+        double *c = cols.as<double>();
+        saa_k_cg_diag<<<w.n_blk, 256, 0, st>>>(p->D, c, c + n, c + 2 * n);
+        saa_k_cg_binv<<<nblk(w.n_nodes, 256), 256, 0, st>>>(w.n_nodes, c, c + n, c + 2 * n, w.free_mask, w.ext, w.binv, bad);
+        CK(cudaGetLastError());
+        unsigned long long bad_h = 0;
+        CK(cudaMemcpyAsync(&bad_h, bad, sizeof bad_h, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        if (bad_h != ~0ull)
+            return fail("saa_mg_create: level %d, local node %llu: its diagonal 3x3 block (clamped rows and columns replaced by the "
+                        "identity) is not positive definite, Cholesky fails", l, bad_h);
+    }
+    // power iteration of B^-1 A, Rayleigh quotient in the A inner product: lam = (A x)^T B^-1 (A x) / x^T A x
+    saa_k_mg_start<<<nblk(w.n_nodes, 256), 256, 0, st>>>(w.n_nodes, w.ext, w.free_mask, w.x);
+    for (int it = 0; it < power_iters; ++it) {
+        if (cg_apply<SAA_APPLY_DOT>(&w, 1, &CgWork::x, &CgWork::q, st, nullptr)) return -1;
+        cg_reduce<1>(&w, 1, true, L.slot, st, nullptr);
+        saa_k_mg_power<<<w.n_blk, 256, 0, st>>>(w.n_nodes, w.q, w.x, w.binv, w.free_mask, L.slot, w.part, w.n_blk);
+        cg_reduce<1>(&w, 1, false, L.slot + 1, st, nullptr);
+    }
+    CK(cudaGetLastError());
+    double s[2];
+    CK(cudaMemcpyAsync(s, L.slot, sizeof s, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    L.lam = s[1] / s[0];
+    if (!(L.lam > 0.0) || !std::isfinite(L.lam))
+        return fail("saa_mg_create: level %d: the estimate of lambda_max(B^-1 A) is %g (A is not positive definite on the free DOFs)",
+                    l, L.lam);
+    return 0;
+}
+
+// the prolongation from level l + 1 to level l (stored on level l) and its transpose (stored on level l + 1)
+static int mg_tables(saa_mg *mg, int l, const int64_t *ptr, const int32_t *col, const double *wt, cudaStream_t st)
+{
+    MgLevel &F = mg->L[l], &C = mg->L[l + 1];
+    const int64_t nf = F.p->n_dof / 3, nc = C.p->n_dof / 3;
+    DevBuf badb;
+    if (badb.alloc(8)) return -1;
+    CK(cudaMemsetAsync(badb.p, 0xff, 8, st));
+    saa_k_mg_check_table<<<nblk(nf, 256), 256, 0, st>>>(nf, nc, ptr, col, badb.as<unsigned long long>());
+    CK(cudaGetLastError());
+    unsigned long long bad = 0;
+    int64_t nnz = 0;
+    CK(cudaMemcpyAsync(&bad, badb.p, 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    if (bad != ~0ull)
+        return fail("saa_mg_create: prolongation %d -> %d, fine node %llu: p_ptr is not a CSR offset table over the %lld nodes of "
+                    "level %d, or a column is outside the %lld nodes of level %d", l + 1, l, bad, (long long)nf, l, (long long)nc, l + 1);
+    CK(cudaMemcpyAsync(&nnz, ptr + nf, 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    if (nnz >= INT32_MAX) return fail("saa_mg_create: prolongation %d -> %d has 2^31 or more entries", l + 1, l);
+    const size_t b_ptr = 8 * (nf + 1), b_col = 4 * std::max<int64_t>(nnz, 1), b_w = 8 * std::max<int64_t>(nnz, 1);
+    const size_t bt_ptr = 8 * (nc + 1);
+    if (F.tab.alloc(b_ptr + b_col + b_w + 64) || C.ttab.alloc(bt_ptr + b_col + b_w + 64)) return -1;
+    mg->bytes += b_ptr + b_col + b_w + bt_ptr + b_col + b_w;
+    F.p_ptr = F.tab.as<int64_t>(); F.p_w = (double *)(F.p_ptr + nf + 1); F.p_cnode = (int32_t *)(F.p_w + std::max<int64_t>(nnz, 1));
+    C.t_ptr = C.ttab.as<int64_t>(); C.t_w = (double *)(C.t_ptr + nc + 1); C.t_fnode = (int32_t *)(C.t_w + std::max<int64_t>(nnz, 1));
+    CK(cudaMemcpyAsync(F.p_ptr, ptr, b_ptr, cudaMemcpyDeviceToDevice, st));
+    CK(cudaMemcpyAsync(F.p_w, wt, 8 * nnz, cudaMemcpyDeviceToDevice, st));
+    DevBuf scratch;                                    // entry row, sort keys, sorted entries
+    if (scratch.alloc(12 * std::max<int64_t>(nnz, 1))) return -1;
+    int32_t *row_of = scratch.as<int32_t>(), *keys = row_of + nnz, *entry = keys + nnz;
+    saa_k_mg_table_rows<<<nblk(nf, 256), 256, 0, st>>>(nf, ptr, col, C.p->d_iperm, row_of, F.p_cnode);
+    CK(cudaMemcpyAsync(keys, col, 4 * nnz, cudaMemcpyDeviceToDevice, st));
+    CK(cudaGetLastError());
+    // transpose: entries stably sorted by coarse node keep their ascending fine-node order
+    thrust::sequence(thrust::cuda::par.on(st), entry, entry + nnz);
+    thrust::stable_sort_by_key(thrust::cuda::par.on(st), keys, keys + nnz, entry);
+    thrust::lower_bound(thrust::cuda::par.on(st), keys, keys + nnz, thrust::counting_iterator<int32_t>(0),
+                        thrust::counting_iterator<int32_t>((int32_t)nc + 1), C.t_ptr);
+    saa_k_mg_table_transpose<<<nblk(nnz, 256), 256, 0, st>>>(nnz, entry, row_of, wt, F.p->d_iperm, C.t_fnode, C.t_w);
+    CK(cudaGetLastError());
+    CK(cudaStreamSynchronize(st));
+    return 0;
+}
+
+extern "C" int saa_mg_create(saa_mg **out, saa_plan *const *levels, int n_levels, const int64_t *const *p_ptr, const int32_t *const *p_col,
+                             const double *const *p_w, const double *coarse_inv_dev, int degree, int power_iters, int64_t coarsest_max_dof)
+{
+    if (!out) return fail("saa_mg_create: null output");
+    *out = nullptr;
+    if (!levels || n_levels < 2) return fail("saa_mg_create: a hierarchy needs at least two levels (got %d)", n_levels);
+    if (degree < 1 || power_iters < 1) return fail("saa_mg_create: degree and power_iters must be >= 1");
+    if (!p_ptr || !p_col || !p_w || !coarse_inv_dev) return fail("saa_mg_create: null prolongation table or coarse inverse");
+    for (int l = 0; l < n_levels; ++l) {
+        saa_plan *p = levels[l];
+        if (!p) return fail("saa_mg_create: level %d: null plan", l);
+        if (!p->finalized) return fail("saa_mg_create: level %d: plan not finalized", l);
+        if (p->size > 1)
+            return fail("saa_mg_create: level %d is rank %d of a partition of size %d; the multigrid preconditioner needs size-1 plans",
+                        l, p->rank, p->size);
+        if (!p->d_val) return fail("saa_mg_create: level %d: the assembled matrix of this plan was released (SAA_OPT_MATFREE = 2)", l);
+        if (p->device != levels[0]->device)
+            return fail("saa_mg_create: level %d is on device %d, level 0 on device %d", l, p->device, levels[0]->device);
+        if (l < n_levels - 1 && (!p_ptr[l] || !p_col[l] || !p_w[l])) return fail("saa_mg_create: null prolongation table %d", l);
+    }
+    const saa_plan *pc = levels[n_levels - 1];
+    if (pc->n_dof > coarsest_max_dof)
+        return fail("saa_mg_create: the coarsest level has %lld DOF, above coarsest_max_dof = %lld (its dense inverse would take %.2f GB)",
+                    (long long)pc->n_dof, (long long)coarsest_max_dof, 8.0 * pc->n_rows * pc->n_rows / 1e9);
+    CK(cudaSetDevice(levels[0]->device));
+    for (int l = 0; l < n_levels; ++l) CK(cudaStreamSynchronize(levels[l]->stream));
+    const cudaStream_t st = plan_stream(levels[0]);
+    std::unique_ptr<saa_mg> mg(new saa_mg);
+    mg->n = n_levels;
+    mg->L.reset(new MgLevel[n_levels]);
+    for (int l = 0; l < n_levels; ++l) {
+        if (mg_level_setup(mg.get(), l, levels[l], power_iters, st)) return -1;
+        mg_chebyshev(mg->L[l], degree);
+    }
+    for (int l = 0; l + 1 < n_levels; ++l)
+        if (mg_tables(mg.get(), l, p_ptr[l], p_col[l], p_w[l], st)) return -1;
+    const int64_t ne = pc->n_dof, ni = pc->n_rows;
+    if (mg->cinv.alloc(8 * ni * ni)) return -1;
+    mg->bytes += 8 * ni * ni;
+    CK(cudaMemsetAsync(mg->cinv.p, 0, 8 * ni * ni, st));
+    saa_k_mg_coarse_permute<<<nblk(ne * ne, 256), 256, 0, st>>>(ne, ni, pc->d_iperm, coarse_inv_dev, mg->cinv.as<double>());
+    CK(cudaGetLastError());
+    CK(cudaStreamSynchronize(st));
+    *out = mg.release();
+    return 0;
+}
+
+extern "C" int saa_mg_destroy(saa_mg *mg)
+{
+    if (!mg) return 0;
+    cudaSetDevice(mg->L[0].p->device);
+    delete mg;
+    return 0;
+}
+
+extern "C" int saa_mg_info(const saa_mg *mg, double *lambda, int64_t *bytes)
+{
+    if (!mg) return fail("saa_mg_info: null hierarchy");
+    if (lambda)
+        for (int l = 0; l < mg->n; ++l) lambda[l] = mg->L[l].lam;
+    if (bytes) *bytes = mg->bytes;
+    return 0;
+}
+
+static int mg_check(saa_mg *mg, const char *name)
+{
+    if (!mg) return fail("%s: null hierarchy", name);
+    for (int l = 0; l < mg->n; ++l)
+        if (!mg->L[l].p->d_val) return fail("%s: level %d: the assembled matrix of this plan was released (SAA_OPT_MATFREE = 2)", name, l);
+    CK(cudaSetDevice(mg->L[0].p->device));
+    for (int l = 0; l < mg->n; ++l) CK(cudaStreamSynchronize(mg->L[l].p->stream));
+    return 0;
+}
+
+extern "C" int saa_plan_solve_static_mg_dev(saa_mg *mg, const double *x0, double *xout, double rtol, int64_t max_iter,
+                                            int64_t check_every, double *hist, int64_t *iters, double *rel_res, double *rel_res_true,
+                                            int *converged)
+{
+    const char *name = "saa_plan_solve_static_mg_dev";
+    if (!(rtol >= 0.0) || !std::isfinite(rtol)) return fail("%s: rtol must be finite and >= 0", name);
+    if (max_iter < 0) return fail("%s: max_iter < 0", name);
+    if (check_every < 1) return fail("%s: check_every must be >= 1", name);
+    if (!xout) return fail("%s: null output", name);
+    if (mg_check(mg, name)) return -1;
+    MgLevel &F = mg->L[0];
+    saa_plan *p = F.p;
+    const cudaStream_t st = plan_stream(p);
+    // the outer iteration's vectors; preconditioner, free rows and partials are the fine level's
+    CgWork w;
+    w.p = p; w.H = F.w.H; w.n_nodes = F.w.n_nodes; w.n_blk = F.w.n_blk; w.n_units = 0; w.n_parts = F.w.n_parts;
+    w.binv = F.w.binv; w.part = F.w.part; w.stage = F.w.stage; w.free_mask = F.w.free_mask; w.ext = F.w.ext; w.ticket = F.w.ticket;
+    const int64_t n = p->n_rows;
+    if (w.mem.alloc(5 * 8 * n)) return -1;
+    w.x = w.mem.as<double>(); w.r = w.x + n; w.pv = w.r + n; w.q = w.pv + n; w.z = w.q + n;
+    DevBuf sbuf;
+    if (sbuf.alloc(sizeof(SaaCgState) + 2 * sizeof(double))) return -1;
+    SaaCgState *S = sbuf.as<SaaCgState>();
+    double *rk = (double *)(S + 1);
+    SaaCgState hs{};
+    hs.rtol = rtol;
+    hs.max_iter = max_iter;
+    CK(cudaMemcpyAsync(S, &hs, sizeof hs, cudaMemcpyHostToDevice, st));
+    CK(cudaMemsetAsync(w.x, 0, n * sizeof(double), st));
+    if (x0) {
+        saa_k_scatter_to_internal<<<nblk(p->n_dof, 256), 256, 0, st>>>(p->n_dof, p->d_iperm, x0, w.x);
+        saa_k_cg_mask<<<nblk(n, 256), 256, 0, st>>>(n, w.free_mask, w.x);
+    }
+    const long long *gate = &S->done;
+    const unsigned gn = (unsigned)w.n_blk;
+    // r = b - A x, z = V r, p = z
+    if (cg_apply<SAA_APPLY_RES>(&w, 1, &CgWork::x, &CgWork::r, st, nullptr)) return -1;
+    cg_reduce<2>(&w, 1, true, rk, st, nullptr);
+    saa_k_cg_scalar<<<1, 32, 0, st>>>(S, rk, 1, SAA_CG_RES0, hist);
+    mg_vcycle(mg, 0, w.r, w.z, st, gate);
+    saa_k_mg_rz<true><<<gn, 256, 0, st>>>(w.n_nodes, S, w.r, w.z, w.pv, w.part, w.n_blk);
+    cg_reduce<2>(&w, 1, false, rk, st, nullptr);
+    saa_k_cg_scalar<<<1, 32, 0, st>>>(S, rk, 1, SAA_CG_INIT, hist);
+    CK(cudaGetLastError());
+    auto iteration = [&]() -> int {
+        if (cg_apply<SAA_APPLY_DOT>(&w, 1, &CgWork::pv, &CgWork::q, st, gate)) return -1;
+        cg_reduce<1>(&w, 1, true, rk, st, gate);
+        saa_k_cg_scalar<<<1, 32, 0, st>>>(S, rk, 1, SAA_CG_ALPHA, hist);
+        saa_k_mg_update<<<gn, 256, 0, st>>>(w.n_nodes, S, w.x, w.r, w.pv, w.q, w.free_mask, w.part, w.n_blk);
+        mg_vcycle(mg, 0, w.r, w.z, st, gate);
+        saa_k_mg_rz<false><<<gn, 256, 0, st>>>(w.n_nodes, S, w.r, w.z, nullptr, w.part, w.n_blk);
+        cg_reduce<2>(&w, 1, false, rk, st, gate);
+        saa_k_cg_scalar<<<1, 32, 0, st>>>(S, rk, 1, SAA_CG_BETA, hist);
+        saa_k_cg_direction<<<nblk(n, 256), 256, 0, st>>>(n, S, w.z, w.pv);
+        CK(cudaGetLastError());
+        return 0;
+    };
+    if (cg_iterate(iteration, name, st, S, hs, max_iter, check_every)) return -1;
+    // the true residual b - A x of the returned iterate, and x in local DOF order
+    if (cg_apply<SAA_APPLY_RES>(&w, 1, &CgWork::x, &CgWork::q, st, nullptr)) return -1;
+    cg_reduce<2>(&w, 1, true, rk, st, nullptr);
+    saa_k_cg_scalar<<<1, 32, 0, st>>>(S, rk, 1, SAA_CG_TRUE, hist);
+    saa_k_gather_to_external<<<nblk(p->n_dof, 256), 256, 0, st>>>(p->n_dof, p->d_iperm, w.x, xout);
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(&hs, S, sizeof hs, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    const double bn = std::sqrt(hs.bb);
+    if (iters) *iters = hs.it;
+    if (rel_res) *rel_res = bn > 0.0 ? std::sqrt(hs.rr) / bn : std::sqrt(hs.rr);
+    if (rel_res_true) *rel_res_true = bn > 0.0 ? std::sqrt(hs.rr_true) / bn : std::sqrt(hs.rr_true);
+    if (converged) *converged = (int)hs.converged;
+    return 0;
+}
+
+// ---- the hierarchy's operators one at a time, external order (tests) ----
+extern "C" int saa_mg_vcycle_dev(saa_mg *mg, const double *r_dev, double *z_dev)
+{
+    if (mg_check(mg, "saa_mg_vcycle_dev")) return -1;
+    if (!r_dev || !z_dev) return fail("saa_mg_vcycle_dev: null argument");
+    saa_plan *p = mg->L[0].p;
+    const cudaStream_t st = plan_stream(p);
+    const int64_t n = p->n_rows;
+    DevBuf t;
+    if (t.alloc(16 * n)) return -1;
+    double *b = t.as<double>(), *x = b + n;
+    CK(cudaMemsetAsync(b, 0, 8 * n, st));
+    saa_k_scatter_to_internal<<<nblk(p->n_dof, 256), 256, 0, st>>>(p->n_dof, p->d_iperm, r_dev, b);
+    saa_k_cg_mask<<<nblk(n, 256), 256, 0, st>>>(n, mg->L[0].w.free_mask, b);
+    mg_vcycle(mg, 0, b, x, st, nullptr);
+    saa_k_gather_to_external<<<nblk(p->n_dof, 256), 256, 0, st>>>(p->n_dof, p->d_iperm, x, z_dev);
+    CK(cudaGetLastError());
+    CK(cudaStreamSynchronize(st));
+    return 0;
+}
+
+static int mg_transfer(saa_mg *mg, int level, const double *in, double *out, bool prolong, const char *name)
+{
+    if (mg_check(mg, name)) return -1;
+    if (!in || !out) return fail("%s: null argument", name);
+    if (level < 0 || level + 1 >= mg->n) return fail("%s: level %d is not in [0, %d)", name, level, mg->n - 1);
+    MgLevel &F = mg->L[level], &C = mg->L[level + 1];
+    saa_plan *pi = prolong ? C.p : F.p, *po = prolong ? F.p : C.p;
+    const cudaStream_t st = plan_stream(F.p);
+    DevBuf t;
+    if (t.alloc(8 * (pi->n_rows + po->n_rows))) return -1;
+    double *vi = t.as<double>(), *vo = vi + pi->n_rows;
+    CK(cudaMemsetAsync(t.p, 0, 8 * (pi->n_rows + po->n_rows), st));
+    saa_k_scatter_to_internal<<<nblk(pi->n_dof, 256), 256, 0, st>>>(pi->n_dof, pi->d_iperm, in, vi);
+    if (prolong)
+        saa_k_mg_prolong<<<nblk(F.w.n_nodes, 256), 256, 0, st>>>(F.w.n_nodes, F.w.ext, F.p_ptr, F.p_cnode, F.p_w, vi, vo, F.w.free_mask,
+                                                                 nullptr);
+    else
+        saa_k_mg_restrict<<<nblk(C.w.n_nodes, 256), 256, 0, st>>>(C.w.n_nodes, C.w.ext, C.t_ptr, C.t_fnode, C.t_w, vi, vo,
+                                                                  C.w.free_mask, nullptr);
+    saa_k_gather_to_external<<<nblk(po->n_dof, 256), 256, 0, st>>>(po->n_dof, po->d_iperm, vo, out);
+    CK(cudaGetLastError());
+    CK(cudaStreamSynchronize(st));
+    return 0;
+}
+
+extern "C" int saa_mg_prolong_dev(saa_mg *mg, int level, const double *xc_dev, double *xf_dev)
+{
+    return mg_transfer(mg, level, xc_dev, xf_dev, true, "saa_mg_prolong_dev");
+}
+
+extern "C" int saa_mg_restrict_dev(saa_mg *mg, int level, const double *rf_dev, double *bc_dev)
+{
+    return mg_transfer(mg, level, rf_dev, bc_dev, false, "saa_mg_restrict_dev");
 }

@@ -66,6 +66,13 @@ ABI = {
     "saa_group_apply_stiffness_dev": (_int, [_vp, _vp, _vp]),
     "saa_plan_solve_static_dev": (_int, [_vp, _vp, _vp, _f64, _i64, _i64, _vp, _vp, _vp, _vp, _vp]),
     "saa_group_solve_static_dev": (_int, [_vp, _vp, _vp, _f64, _i64, _i64, _vp, _vp, _vp, _vp, _vp]),
+    "saa_mg_create": (_int, [_PP, _vp, _int, _vp, _vp, _vp, _vp, _int, _int, _i64]),
+    "saa_mg_destroy": (_int, [_vp]),
+    "saa_mg_info": (_int, [_vp, _vp, _vp]),
+    "saa_plan_solve_static_mg_dev": (_int, [_vp, _vp, _vp, _f64, _i64, _i64, _vp, _vp, _vp, _vp, _vp]),
+    "saa_mg_vcycle_dev": (_int, [_vp, _vp, _vp]),
+    "saa_mg_prolong_dev": (_int, [_vp, _int, _vp, _vp]),
+    "saa_mg_restrict_dev": (_int, [_vp, _int, _vp, _vp]),
     "saa_plan_stream": (_vp, [_vp]),
     "saa_step_host": (_int, [_vp, _vp, _vp, _f64, _int, _vp]),
     "saa_step_host_ex": (_int, [_vp, _vp, _vp, _f64, _int, _vp, _int]),
@@ -162,7 +169,11 @@ def _dev_vector(t, n, device, what):
 MAX_ITER_DEFAULT = 1_000_000
 
 
-def _solve_static(fn, handle, plans, rtol, max_iter, x0, check_every):
+# default iteration cap of the multigrid-preconditioned solve (its iteration count does not grow with the mesh)
+MG_MAX_ITER_DEFAULT = 1000
+
+
+def _solve_static(fn, handle, plans, rtol, max_iter, x0, check_every, single=False):
     import torch
     dev = torch.device("cuda", plans[0].device)
     max_iter = min(10 * sum(pl.n_dof for pl in plans), MAX_ITER_DEFAULT) if max_iter is None else int(max_iter)
@@ -177,11 +188,12 @@ def _solve_static(fn, handle, plans, rtol, max_iter, x0, check_every):
     torch.cuda.current_stream(dev).synchronize()              # torch's pending work on x0 precedes the plans' stream
     args = (float(rtol), max_iter, int(check_every), hist.data_ptr(), ctypes.byref(it), ctypes.byref(rel),
             ctypes.byref(rel_true), ctypes.byref(conv))
-    if handle is None:
-        _check(fn(plans[0].h, None if x0[0] is None else x0[0].data_ptr(), xs[0].data_ptr(), *args), "saa_plan_solve_static_dev")
+    if handle is None or single:
+        _check(fn(plans[0].h if handle is None else handle, None if x0[0] is None else x0[0].data_ptr(), xs[0].data_ptr(), *args),
+               "saa_plan_solve_static_dev" if handle is None else "saa_plan_solve_static_mg_dev")
     else:
         _check(fn(handle, ptrs(x0), ptrs(xs), *args), "saa_group_solve_static_dev")
-    return StaticResult(xs[0] if handle is None else xs, int(it.value), rel.value, rel_true.value, bool(conv.value),
+    return StaticResult(xs[0] if handle is None or single else xs, int(it.value), rel.value, rel_true.value, bool(conv.value),
                         hist[:int(it.value)].clone())        # the max_iter-long buffer is released
 
 
@@ -476,14 +488,22 @@ class StepPlan:
         _check(lib().saa_plan_apply_stiffness_dev(self.h, x.data_ptr(), y.data_ptr()), "saa_plan_apply_stiffness_dev")
         return y
 
-    def solve_static(self, rtol=1e-10, max_iter=None, x0=None, check_every=50):
+    def solve_static(self, rtol=1e-10, max_iter=None, x0=None, check_every=None, precond=None):
         """Solve the steady system of Steady_Elasticity_solver, (S K S + I - S) x = S F, on the device by block-Jacobi
         preconditioned CG (DESIGN.md §7c).  max_iter defaults to 10 n_dof, at most MAX_ITER_DEFAULT (CG in floating
         point needs more than n_dof iterations on an ill-conditioned system); x0: start tensor (None: 0).  Returns a
         StaticResult; not converging within max_iter is not an error (converged=False).  A plan of a partition with
-        size > 1 is solved through PlanGroup.solve_static."""
-        return _solve_static(lib().saa_plan_solve_static_dev, None, [self], rtol, max_iter, None if x0 is None else [x0],
-                             check_every)
+        size > 1 is solved through PlanGroup.solve_static.
+        precond: a multigrid.StructuredMultigrid built for this plan: one V-cycle per iteration instead of the
+        block-Jacobi step (DESIGN.md §7d); max_iter then defaults to 1000 and check_every to 10 (50 without)."""
+        if precond is None:
+            return _solve_static(lib().saa_plan_solve_static_dev, None, [self], rtol, max_iter, None if x0 is None else [x0],
+                                 50 if check_every is None else check_every)
+        if getattr(precond, "plan", None) is not self:
+            raise SaaError("solve_static: the multigrid hierarchy was built for another plan")
+        return _solve_static(lib().saa_plan_solve_static_mg_dev, precond.handle(), [self], rtol,
+                             MG_MAX_ITER_DEFAULT if max_iter is None else max_iter, None if x0 is None else [x0],
+                             10 if check_every is None else check_every, single=True)
 
     def _host_out(self):
         """The array a host call returns d1 in.  From 1 MiB per vector on it is a view of page-locked memory
@@ -696,9 +716,13 @@ class PlanGroup:
         _check(lib().saa_group_apply_stiffness_dev(self.h, ptrs(xs), ptrs(ys)), "saa_group_apply_stiffness_dev")
         return ys
 
-    def solve_static(self, rtol=1e-10, max_iter=None, x0=None, check_every=50):
+    def solve_static(self, rtol=1e-10, max_iter=None, x0=None, check_every=50, precond=None):
         """StepPlan.solve_static over all partitions of the group; x0 and the result's x are lists, one per plan.
-        max_iter defaults to 10 times the sum of the plans' n_dof, at most MAX_ITER_DEFAULT."""
+        max_iter defaults to 10 times the sum of the plans' n_dof, at most MAX_ITER_DEFAULT.  The multigrid
+        preconditioner is not available for a partitioned problem (precond must be None)."""
+        if precond is not None:
+            raise SaaError("PlanGroup.solve_static: the multigrid preconditioner (precond) works on a single-partition plan "
+                           "only; a partitioned problem is solved with block-Jacobi CG (precond=None)")
         return _solve_static(lib().saa_group_solve_static_dev, self.h, self.plans, rtol, max_iter, x0, check_every)
 
     def close(self):
