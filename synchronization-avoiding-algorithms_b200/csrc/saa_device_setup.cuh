@@ -136,52 +136,101 @@ __global__ void saa_k_fin_pmask(int64_t n_slices, const int64_t *__restrict__ sl
     }
     if (lane == 0) slice_vals[s] = 32 * planes;
 }
-// one warp per slice: every lane writes the stored planes of its blocks (stored order of each row kept), then pads with
-// blocks 0.0 * d0[own node]
-__global__ void saa_k_fin_fill(int64_t n_slices, const int64_t *__restrict__ slice_ptr, const int64_t *__restrict__ val_ptr,
-                               const uint16_t *__restrict__ pmask, const int32_t *__restrict__ permn,
-                               const int32_t *__restrict__ iperm, const int64_t *__restrict__ indptr,
-                               const int32_t *__restrict__ indices, const double *__restrict__ data, double *__restrict__ val,
-                               int32_t *__restrict__ col)
+// the lane's values of its next block (zeros past its last block or on a padding lane) and the block's column node
+// (INT32_MAX then)
+__device__ __forceinline__ int32_t saa_fin_next_block(SaaRowTriple &t, bool node, const int32_t *indices, const double *data, double (&a)[9])
+{
+    for (int k = 0; k < 9; ++k) a[k] = 0.0;
+    if (!node) return INT32_MAX;
+    const int32_t cn = t.next_col_node(indices);
+    if (cn != INT32_MAX)
+        for (int A = 0; A < 3; ++A)
+            while (t.q[A] < t.qe[A] && indices[t.q[A]] / 3 == cn) {
+                a[3 * A + indices[t.q[A]] % 3] = data[t.q[A]];
+                ++t.q[A];
+            }
+    return cn;
+}
+__device__ __forceinline__ long long saa_warp_min64(long long x)
+{
+    for (int o = 16; o > 0; o >>= 1) x = min(x, __shfl_xor_sync(0xffffffffu, x, o));
+    return x;
+}
+__device__ __forceinline__ long long saa_warp_max64(long long x)
+{
+    for (int o = 16; o > 0; o >>= 1) x = max(x, __shfl_xor_sync(0xffffffffu, x, o));
+    return x;
+}
+// one warp per slice: the coding decision of every block-row from the bits its stored planes will hold (padding lanes
+// and unstored entries of a stored plane are +0.0): coded iff every stored plane spans at most 65535 as int64.  Sets
+// bit 15 of the mask and gives the doubles the slice takes in val and its number of coded planes (same rule as the
+// host path in saa_plan_finalize).
+__global__ void saa_k_fin_code(int64_t n_slices, const int64_t *__restrict__ slice_ptr, const int32_t *__restrict__ permn,
+                               const int64_t *__restrict__ indptr, const int32_t *__restrict__ indices, const double *__restrict__ data,
+                               uint16_t *__restrict__ pmask, int64_t *__restrict__ slice_vals, int64_t *__restrict__ slice_coded)
 {
     const int lane = threadIdx.x & 31;
     const int64_t s = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (s >= n_slices) return;
     const int64_t beg = slice_ptr[s];
     const int L = (int)((slice_ptr[s + 1] - beg) >> 5);
-    double *vs = val + val_ptr[s] + lane;
+    const int32_t e = permn[s * 32 + lane];
+    SaaRowTriple t(indptr, e >= 0 ? e : 0);
+    int64_t vals = 0, coded = 0;
+    for (int j = 0; j < L; ++j) {
+        double a[9];
+        saa_fin_next_block(t, e >= 0, indices, data, a);
+        const unsigned m = pmask[(beg >> 5) + j];
+        bool code = m != 0u;
+        for (int k = 0; k < 9; ++k)
+            if (m & (1u << k)) {
+                const long long x = __double_as_longlong(a[k]);
+                code = code && (unsigned long long)saa_warp_max64(x) - (unsigned long long)saa_warp_min64(x) <= 65535ull;
+            }
+        if (code && lane == 0) pmask[(beg >> 5) + j] = (uint16_t)(m | SAA_CODED);
+        vals += (code ? 8 : 32) * __popc(m);
+        coded += code ? __popc(m) : 0;
+    }
+    if (lane == 0) { slice_vals[s] = vals; slice_coded[s] = coded; }
+}
+// one warp per slice: every lane writes the stored planes of its blocks (stored order of each row kept), raw or coded,
+// then pads with blocks 0.0 * d0[own node]
+__global__ void saa_k_fin_fill(int64_t n_slices, const int64_t *__restrict__ slice_ptr, const int64_t *__restrict__ val_ptr,
+                               const int64_t *__restrict__ vb_ptr, const uint16_t *__restrict__ pmask, const int32_t *__restrict__ permn,
+                               const int32_t *__restrict__ iperm, const int64_t *__restrict__ indptr,
+                               const int32_t *__restrict__ indices, const double *__restrict__ data, double *__restrict__ val,
+                               long long *__restrict__ vbase, int32_t *__restrict__ col)
+{
+    const int lane = threadIdx.x & 31;
+    const int64_t s = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (s >= n_slices) return;
+    const int64_t beg = slice_ptr[s];
+    const int L = (int)((slice_ptr[s + 1] - beg) >> 5);
+    char *v = (char *)(val + val_ptr[s]);
+    long long *vb = vbase + vb_ptr[s];
     const uint16_t *ms = pmask + (beg >> 5);
     int32_t *cs = col + beg + lane;
     const int64_t inode = s * 32 + lane;
     const int32_t e = permn[inode];
-    int64_t off = 0;                                   // planes stored for the blocks before j
-    auto store = [&](int j, const double (&a)[9]) {
+    SaaRowTriple t(indptr, e >= 0 ? e : 0);
+    for (int j = 0; j < L; ++j) {
+        double a[9];
+        const int32_t cn = saa_fin_next_block(t, e >= 0, indices, data, a);
+        cs[32 * (int64_t)j] = (cn != INT32_MAX) ? iperm[3 * (int64_t)cn] / 3 : (int32_t)inode;
         const unsigned m = ms[j];
+        int i = 0;
         for (int k = 0; k < 9; ++k)
-            if (m & (1u << k)) vs[32 * (off + __popc(m & ((1u << k) - 1u)))] = a[k];
-        off += __popc(m);
-    };
-    int j = 0;
-    if (e >= 0) {
-        SaaRowTriple t(indptr, e);
-        for (;; ++j) {
-            const int32_t cn = t.next_col_node(indices);
-            if (cn == INT32_MAX) break;
-            double a[9];
-            for (int k = 0; k < 9; ++k) a[k] = 0.0;
-            for (int A = 0; A < 3; ++A)
-                while (t.q[A] < t.qe[A] && indices[t.q[A]] / 3 == cn) {
-                    a[3 * A + indices[t.q[A]] % 3] = data[t.q[A]];
-                    ++t.q[A];
+            if (m & (1u << k)) {
+                if (m & SAA_CODED) {
+                    const long long x = __double_as_longlong(a[k]), lo = saa_warp_min64(x);
+                    ((uint16_t *)(v + 64 * i))[lane] = (uint16_t)((unsigned long long)x - (unsigned long long)lo);
+                    if (lane == 0) vb[i] = lo;
+                } else {
+                    ((double *)(v + 256 * i))[lane] = a[k];
                 }
-            store(j, a);
-            cs[32 * (int64_t)j] = iperm[3 * (int64_t)cn] / 3;
-        }
-    }
-    const double z[9] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
-    for (; j < L; ++j) {
-        store(j, z);
-        cs[32 * (int64_t)j] = (int32_t)inode;
+                ++i;
+            }
+        if (m & SAA_CODED) { v += 64 * i; vb += i; } else { v += 256 * i; }
     }
 }
 __global__ void saa_k_fin_vectors(int64_t n_rows, const int32_t *__restrict__ permn, const double *__restrict__ M_ext,
@@ -335,10 +384,25 @@ static int finalize_device(saa_plan *p)
     int64_t n_val = 0;
     CK(cudaMemcpy(&n_val, p->d_val_ptr + p->n_slices, sizeof(int64_t), cudaMemcpyDeviceToHost));
     p->value_planes = n_val / 32;
+    //    coding decision per block-row (bit 15), then the offsets of the coded layout: val in doubles, vbase in bases
+    DevBuf b_cc;
+    if (b_cc.alloc((p->n_slices + 1) * sizeof(int64_t))) return -1;
+    int64_t *ccnt = b_cc.as<int64_t>();
+    CK(cudaMemset(ccnt, 0, (p->n_slices + 1) * sizeof(int64_t)));
+    CK(cudaMalloc((void **)&p->d_vb_ptr, (p->n_slices + 1) * sizeof(int64_t)));
+    if (p->value_code) {
+        saa_k_fin_code<<<nblk(p->n_slices, 8), 256>>>(p->n_slices, p->d_slice_ptr, permn, p->in_indptr, p->in_indices, p->in_data,
+                                                      p->d_pmask, cnt, ccnt);
+        thrust::exclusive_scan(thrust::device, cnt, cnt + p->n_slices + 1, p->d_val_ptr);
+        CK(cudaMemcpy(&n_val, p->d_val_ptr + p->n_slices, sizeof(int64_t), cudaMemcpyDeviceToHost));
+    }
+    thrust::exclusive_scan(thrust::device, ccnt, ccnt + p->n_slices + 1, p->d_vb_ptr);
+    CK(cudaMemcpy(&p->coded_planes, p->d_vb_ptr + p->n_slices, sizeof(int64_t), cudaMemcpyDeviceToHost));
+    CK(cudaMalloc((void **)&p->d_vbase, std::max<int64_t>(p->coded_planes, 1) * sizeof(long long)));
     CK(cudaMalloc((void **)&p->d_val, std::max<int64_t>(n_val, 1) * sizeof(double)));
     CK(cudaMalloc((void **)&p->d_col, std::max<int64_t>(lanes, 1) * sizeof(int32_t)));
-    saa_k_fin_fill<<<nblk(p->n_slices, 8), 256>>>(p->n_slices, p->d_slice_ptr, p->d_val_ptr, p->d_pmask, permn, p->d_iperm,
-                                                  p->in_indptr, p->in_indices, p->in_data, p->d_val, p->d_col);
+    saa_k_fin_fill<<<nblk(p->n_slices, 8), 256>>>(p->n_slices, p->d_slice_ptr, p->d_val_ptr, p->d_vb_ptr, p->d_pmask, permn, p->d_iperm,
+                                                  p->in_indptr, p->in_indices, p->in_data, p->d_val, p->d_vbase, p->d_col);
     CK(cudaMalloc((void **)&p->d_M, p->n_rows * sizeof(double)));
     CK(cudaMalloc((void **)&p->d_F, p->n_rows * sizeof(double)));
     saa_k_fin_vectors<<<nblk(p->n_rows, 256), 256>>>(p->n_rows, permn, p->in_M, p->in_F, p->d_M, p->d_F);

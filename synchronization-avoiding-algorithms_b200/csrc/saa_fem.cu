@@ -116,15 +116,18 @@ struct saa_plan {
     std::vector<int32_t> nb_rank, holders_rank;
     // layout
     int64_t nnz = 0, padded_entries = 0, n_rows = 0, n_slices = 0, sh_slices = 0;
-    int64_t value_planes = 0;              // stored value planes (32 fp64 each)
+    int64_t value_planes = 0;              // stored value planes (raw and coded)
+    int64_t coded_planes = 0;              // of which coded (int64 base + 32 16-bit offsets)
     bool plane_mask = true;                // false: all nine planes of every block stored (SAA_PLANE_MASK=0, or the cp.async variant)
+    bool value_code = true;                // false: every block-row raw (SAA_VALUE_CODE=0, or plane_mask false)
     std::vector<int32_t> iperm_h;          // external local DOF -> internal row
     std::vector<int32_t> node_order;       // optional base order of the nodes (saa_plan_set_node_order); empty = ascending
     // device
     SaaDev D{};
     SaaHaloDev H{};
-    int64_t *d_slice_ptr = nullptr, *d_val_ptr = nullptr;
+    int64_t *d_slice_ptr = nullptr, *d_val_ptr = nullptr, *d_vb_ptr = nullptr;
     uint16_t *d_pmask = nullptr;
+    long long *d_vbase = nullptr;
     double *d_val = nullptr, *d_M = nullptr, *d_F = nullptr;
     int32_t *d_col = nullptr, *d_iperm = nullptr;
     uint32_t *d_dir = nullptr;
@@ -350,6 +353,9 @@ extern "C" int saa_plan_finalize(saa_plan *p)
         // cp.async variant walks the values by block-row arithmetic and gets the full-plane layout
         const char *pm = getenv("SAA_PLANE_MASK");
         p->plane_mask = !(pm && pm[0] == '0') && p->kvariant < 6;
+        // block-rows whose planes span at most 65535 ulps are stored as base + 16-bit offsets (SAA_VALUE_CODE=0: all raw)
+        const char *vc = getenv("SAA_VALUE_CODE");
+        p->value_code = p->plane_mask && !(vc && vc[0] == '0');
     }
     if (p->dev_input) return finalize_device(p);
     CK(cudaSetDevice(p->device));
@@ -460,20 +466,21 @@ extern "C" int saa_plan_finalize(saa_plan *p)
             for (int64_t j = cnt; j < L; ++j) cs[32 * j + l] = (int32_t)inode;
         }
     }
-    std::vector<int64_t> val_ptr(p->n_slices + 1, 0);
+    // raw planes of every slice, then the coding decision of every block-row from their bits and the final layout
+    std::vector<int64_t> raw_ptr(p->n_slices + 1, 0);
     for (int64_t s = 0; s < p->n_slices; ++s) {
         int64_t planes = 0;
         for (int64_t r = slice_ptr[s] / 32; r < slice_ptr[s + 1] / 32; ++r) planes += __builtin_popcount(pmask[r]);
-        val_ptr[s + 1] = val_ptr[s] + 32 * planes;
+        raw_ptr[s + 1] = raw_ptr[s] + 32 * planes;
     }
-    p->value_planes = val_ptr[p->n_slices] / 32;
-    std::vector<double> val((size_t)val_ptr[p->n_slices], 0.0);
+    p->value_planes = raw_ptr[p->n_slices] / 32;
+    std::vector<double> raw((size_t)raw_ptr[p->n_slices], 0.0);
     for (int64_t s = 0; s < p->n_slices; ++s) {
         const int64_t L = (slice_ptr[s + 1] - slice_ptr[s]) / 32;
         const uint16_t *ms = pmask.data() + slice_ptr[s] / 32;
         std::vector<int64_t> off(L + 1, 0);              // planes stored for the blocks before j
         for (int64_t j = 0; j < L; ++j) off[j + 1] = off[j] + __builtin_popcount(ms[j]);
-        double *vs = val.data() + val_ptr[s];
+        double *vs = raw.data() + raw_ptr[s];
         for (int l = 0; l < 32; ++l) {
             const int64_t e = permn[s * 32 + l];
             if (e >= 0)
@@ -482,6 +489,54 @@ extern "C" int saa_plan_finalize(saa_plan *p)
                 });
         }
     }
+    auto bits = [](double x) { int64_t b; std::memcpy(&b, &x, 8); return b; };
+    std::vector<int64_t> val_ptr(p->n_slices + 1, 0), vb_ptr(p->n_slices + 1, 0);
+    for (int64_t s = 0; s < p->n_slices; ++s) {
+        const double *pl = raw.data() + raw_ptr[s];     // next raw plane of the slice
+        int64_t vals = 0, coded = 0;
+        for (int64_t r = slice_ptr[s] / 32; r < slice_ptr[s + 1] / 32; ++r) {
+            const int n = __builtin_popcount(pmask[r]);
+            bool code = p->value_code && n > 0;
+            for (int i = 0; i < n && code; ++i) {
+                int64_t lo = INT64_MAX, hi = INT64_MIN;
+                for (int l = 0; l < 32; ++l) { lo = std::min(lo, bits(pl[32 * i + l])); hi = std::max(hi, bits(pl[32 * i + l])); }
+                code = (uint64_t)hi - (uint64_t)lo <= 65535u;
+            }
+            if (code) pmask[r] |= SAA_CODED;
+            vals += (code ? 8 : 32) * n;
+            coded += code ? n : 0;
+            pl += 32 * n;
+        }
+        val_ptr[s + 1] = val_ptr[s] + vals;
+        vb_ptr[s + 1] = vb_ptr[s] + coded;
+    }
+    p->coded_planes = vb_ptr[p->n_slices];
+    std::vector<double> val((size_t)val_ptr[p->n_slices], 0.0);
+    std::vector<long long> vbase((size_t)vb_ptr[p->n_slices], 0);
+    for (int64_t s = 0; s < p->n_slices; ++s) {
+        const double *pl = raw.data() + raw_ptr[s];
+        char *v = (char *)(val.data() + val_ptr[s]);
+        long long *vb = vbase.data() + vb_ptr[s];
+        for (int64_t r = slice_ptr[s] / 32; r < slice_ptr[s + 1] / 32; ++r) {
+            const int n = __builtin_popcount(pmask[r] & SAA_PLANES);
+            for (int i = 0; i < n; ++i, pl += 32) {
+                if (pmask[r] & SAA_CODED) {
+                    int64_t lo = INT64_MAX;
+                    for (int l = 0; l < 32; ++l) lo = std::min(lo, bits(pl[l]));
+                    *vb++ = lo;
+                    for (int l = 0; l < 32; ++l) {
+                        const uint16_t o = (uint16_t)((uint64_t)bits(pl[l]) - (uint64_t)lo);
+                        std::memcpy(v + 2 * l, &o, 2);
+                    }
+                    v += 64;
+                } else {
+                    std::memcpy(v, pl, 256);
+                    v += 256;
+                }
+            }
+        }
+    }
+    std::vector<double>().swap(raw);
     std::vector<double> M(p->n_rows, 1.0), F(p->n_rows, 0.0);
     for (int64_t r = 0; r < n; ++r) { M[p->iperm_h[r]] = p->M[r]; F[p->iperm_h[r]] = p->F[r]; }
     std::vector<uint32_t> dir(p->n_rows / 32, 0u);
@@ -491,7 +546,7 @@ extern "C" int saa_plan_finalize(saa_plan *p)
     }
 
     if (upload(&p->d_slice_ptr, slice_ptr) || upload(&p->d_val_ptr, val_ptr) || upload(&p->d_pmask, pmask) ||
-        upload(&p->d_val, val) || upload(&p->d_col, col) ||
+        upload(&p->d_vb_ptr, vb_ptr) || upload(&p->d_vbase, vbase) || upload(&p->d_val, val) || upload(&p->d_col, col) ||
         upload(&p->d_M, M) || upload(&p->d_F, F) || upload(&p->d_dir, dir) || upload(&p->d_iperm, p->iperm_h))
         return -1;
     const int64_t sh_pad = 3 * sh_padn;
@@ -518,6 +573,7 @@ static int finalize_tail(saa_plan *p, int64_t sh_pad)
 
     p->D.n_rows = p->n_rows; p->D.n_slices = p->n_slices; p->D.sh_slices = p->sh_slices;
     p->D.slice_ptr = p->d_slice_ptr; p->D.val_ptr = p->d_val_ptr; p->D.pmask = p->d_pmask; p->D.val = p->d_val; p->D.col = p->d_col; p->D.dir_mask = p->d_dir;
+    p->D.vb_ptr = p->d_vb_ptr; p->D.vbase = p->d_vbase;
     p->D.M = p->d_M; p->D.F = p->d_F;
     {   // one mass value per node when every node's three DOFs hold the same bits (SAA_NODE_MASS=0 keeps the per-DOF stream)
         const char *nm = getenv("SAA_NODE_MASS");
@@ -617,10 +673,10 @@ static int finalize_tail(saa_plan *p, int64_t sh_pad)
     std::vector<int32_t>().swap(p->indptr); std::vector<int32_t>().swap(p->indices);
     std::vector<double>().swap(p->data); std::vector<double>().swap(p->F); std::vector<double>().swap(p->M);
     CK(cudaDeviceSynchronize());   // set-up work ran on the default stream; the plan's stream is non-blocking
-    // measured on B200 (profiles/r1/kernel_variants.md, profiles/r2/kernel_variants_r2.md, and after the plane-masked
-    // layout profiles/plane_mask/variants.md): the column-prefetching schedule with 3 blocks per SM (85-register cap; the
-    // predicated value loads spill under the 64-register cap of 4 blocks per SM) wins at 1.1 M and 104 M DOF
-    if (p->kvariant < 0) p->kvariant = 5;
+    // measured on B200 (profiles/r1/kernel_variants.md, profiles/r2/kernel_variants_r2.md, profiles/plane_mask/variants.md
+    // and, with the coded values, profiles/value_coding/value_coding_probe.json): the plain schedule with 3 blocks per SM
+    // (85-register cap, no spills; the 64-register cap of 4 blocks per SM spills) wins at 1.1 M and 104 M DOF, coded or raw
+    if (p->kvariant < 0) p->kvariant = 2;
     p->finalized = true;
     return prepare_graphs(p, false);
 }
@@ -637,7 +693,7 @@ extern "C" int saa_plan_destroy(saa_plan *p)
         }
         for (void *m : p->peer_mapped) cudaIpcCloseMemHandle(m);
         for (auto &g : p->step_graphs) cudaGraphExecDestroy(g.exec);
-        void *ptrs[] = {p->d_slice_ptr, p->d_val_ptr, p->d_pmask, p->d_val, p->d_col, p->d_M, p->d_F, p->d_dir, p->d_iperm, p->d_buf[0], p->d_buf[1],
+        void *ptrs[] = {p->d_slice_ptr, p->d_val_ptr, p->d_vb_ptr, p->d_pmask, p->d_val, p->d_vbase, p->d_col, p->d_M, p->d_F, p->d_dir, p->d_iperm, p->d_buf[0], p->d_buf[1],
                         p->d_clk, p->d_stage, p->d_xbuf, p->d_send, p->d_dst_ptr, p->d_dst_pos, p->d_src_ptr, p->d_src_pos,
                         p->d_recv, p->d_done, p->d_own_ready, p->d_dst_nb, p->d_dst_pos_peer, p->d_peer_recv, p->d_peer_stride, p->d_peer_flag,
                         p->d_hist_rows, p->d_hist, p->d_pred_rows, p->d_force, p->d_hook,
@@ -667,13 +723,23 @@ extern "C" int64_t saa_plan_vector_bytes(const saa_plan *p)
     return p ? 4 * 8 * p->n_rows + 8 * (p->D.node_mass ? p->n_rows / 3 : p->n_rows) : -1;
 }
 extern "C" int64_t saa_plan_value_planes(const saa_plan *p) { return p ? p->value_planes : -1; }
+extern "C" int64_t saa_plan_coded_planes(const saa_plan *p) { return p ? p->coded_planes : -1; }
 extern "C" int64_t saa_plan_matrix_bytes(const saa_plan *p)
 {
-    // stored value planes (32 fp64 each), one column-node id per block-lane, one plane mask per block-row, slice and
-    // value offsets, Dirichlet mask words
+    // the plane-masked layout without value coding: stored value planes (32 fp64 each), one column-node id per
+    // block-lane, one plane mask per block-row, slice and value offsets, Dirichlet mask words
     if (!p) return -1;
     const int64_t lanes = p->padded_entries / 9;
     return p->value_planes * 256 + lanes * 4 + (lanes / 32) * 2 + 2 * (p->n_slices + 1) * 8 + (p->n_rows / 32) * 4;
+}
+extern "C" int64_t saa_plan_streamed_matrix_bytes(const saa_plan *p)
+{
+    // what a matrix pass reads: raw planes 256 B, coded planes 64 B of offsets + an 8-B base, the ids, masks, the
+    // slice, value and base offsets and the Dirichlet mask words
+    if (!p) return -1;
+    const int64_t lanes = p->padded_entries / 9;
+    return (p->value_planes - p->coded_planes) * 256 + p->coded_planes * (64 + 8) + lanes * 4 + (lanes / 32) * 2 +
+           3 * (p->n_slices + 1) * 8 + (p->n_rows / 32) * 4;
 }
 extern "C" void *saa_plan_stream(saa_plan *p) { return p ? (void *)plan_stream(p) : nullptr; }
 
@@ -1344,8 +1410,8 @@ extern "C" int saa_plan_set_option(saa_plan *p, int option, int value)
         if (!value && !p->d_val) return fail("saa_plan_set_option: the assembled matrix of this plan was released (SAA_OPT_MATFREE = 2)");
         if (value == 2 && p->d_val) {                    // release the assembled matrix: the plan is matrix-free for good
             if (p->size > 1) return fail("saa_plan_set_option: SAA_OPT_MATFREE = 2 is for single-partition plans (synchronised steps stream the matrix)");
-            cudaFree(p->d_val); cudaFree(p->d_col);
-            p->d_val = nullptr; p->d_col = nullptr; p->D.val = nullptr; p->D.col = nullptr;
+            cudaFree(p->d_val); cudaFree(p->d_col); cudaFree(p->d_vbase);
+            p->d_val = nullptr; p->d_col = nullptr; p->d_vbase = nullptr; p->D.val = nullptr; p->D.col = nullptr; p->D.vbase = nullptr;
         }
         if ((value != 0) == p->matfree) return 0;
         p->matfree = value != 0;

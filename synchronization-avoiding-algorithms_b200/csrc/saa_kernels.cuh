@@ -10,23 +10,30 @@
 // which nvcc never contracts into FMA, and the row sum runs over the stored entries in order starting
 // from 0.0 — the same sequence of roundings scipy/numpy perform, hence bit-identical results.
 //
-// Storage (HBM): plane-masked node-block sliced ELL.  The stiffness of 3-D elasticity is made of 3x3 node blocks, so
-// one thread owns one NODE (its three DOF rows) and one warp owns a slice of 32 nodes.  Block j of the node of lane l in
-// slice s has one column-node id and up to nine value planes (plane (A,B) = entry (A,B) of block j in all 32 lanes);
-// slice_ptr counts block-lanes, the block-row of block j is r = slice_ptr[s]/32 + j:
+// Storage (HBM): plane-masked node-block sliced ELL with value coding.  The stiffness of 3-D elasticity is made of 3x3
+// node blocks, so one thread owns one NODE (its three DOF rows) and one warp owns a slice of 32 nodes.  Block j of the
+// node of lane l in slice s has one column-node id and up to nine value planes (plane (A,B) = entry (A,B) of block j in
+// all 32 lanes); slice_ptr counts block-lanes, the block-row of block j is r = slice_ptr[s]/32 + j:
 //     column node of block j  :  col[slice_ptr[s] + j*32 + l]
-//     stored planes of block j:  bit 3A+B of pmask[r]
-//     value (A,B) of block j  :  val[val_ptr[s] + 32*(off_j + popc(pmask[r] & ((1 << (3A+B)) - 1))) + l]  if that bit is set
-// where off_j is the number of planes stored for blocks 0..j-1 of the slice.  A plane is stored iff at least one lane
-// of the slice has a stored CSR entry there; a plane that is not stored is 0.0 in every lane, and the kernel puts 0.0
-// in the register instead of loading it, so the arithmetic is the same as with all nine planes.  On structured meshes
-// the 32 nodes of a slice share their stencil, so whole planes are zero in every lane (DESIGN.md §3).  Every warp-wide
-// load stays a fully coalesced, aligned 256-B (values) or 128-B (ids) request, and the column id is shared by the
-// entries of a block.  Entries the reference dropped as exact zeros (csr_matrix(dense), Mat_construction.py:150) in a
-// stored plane are 0.0; adding 0.0*x leaves a finite row sum bit-identical (the sum starts at +0.0 and can never
-// become -0.0).  Within a row the blocks are in ascending column order and inside a block B = 0,1,2, i.e. exactly the
-// stored order of the CSR row, which is the summation order of csr_matvec.  SAA_PLANE_MASK=0 at finalisation stores
-// all nine planes of every block (pmask = 0x1FF, val_ptr[s] = 9*slice_ptr[s]).
+//     stored planes of block j:  bit 3A+B of pmask[r] (bits 0-8, SAA_PLANES)
+//     coded block-row         :  bit 15 of pmask[r] (SAA_CODED)
+//     plane (A,B) of block j  :  the (off_j + popc(pmask[r] & ((1 << (3A+B)) - 1)))-th plane of the slice, if that bit is set
+// where off_j is the number of planes stored for blocks 0..j-1 of the slice.  The planes of a slice follow each other
+// from byte 8*val_ptr[s] of val on: a raw plane is 32 fp64 (256 B); a plane of a coded block-row is 32 uint16 lane
+// offsets (64 B) from a per-plane int64 base, vbase[vb_ptr[s] + number of coded planes of the slice before it], and
+// lane l's value is the double whose bits are base + offset[l] (pure integer, bit-exact).  A block-row is coded iff
+// every one of its stored planes spans at most 65535 between the smallest and the largest bit pattern of its 32
+// lanes read as int64 (finalisation decides from the stored bits, padding lanes included).
+// A plane is stored iff at least one lane of the slice has a stored CSR entry there; a plane that is not stored is 0.0
+// in every lane, and the kernel puts 0.0 in the register instead of loading it, so the arithmetic is the same as with
+// all nine planes.  On structured meshes the 32 nodes of a slice share their stencil, so whole planes are zero in every
+// lane, and the lanes of a stored plane differ only by the rounding of the coordinates (DESIGN.md §3).  Every plane is
+// a multiple of 64 B, so every warp-wide load stays one aligned request, and the column id is shared by the entries of
+// a block.  Entries the reference dropped as exact zeros (csr_matrix(dense), Mat_construction.py:150) in a stored plane
+// are 0.0; adding 0.0*x leaves a finite row sum bit-identical (the sum starts at +0.0 and can never become -0.0).
+// Within a row the blocks are in ascending column order and inside a block B = 0,1,2, i.e. exactly the stored order of
+// the CSR row, which is the summation order of csr_matvec.  SAA_PLANE_MASK=0 at finalisation stores all nine raw planes
+// of every block (pmask = 0x1FF, val_ptr[s] = 9*slice_ptr[s]); SAA_VALUE_CODE=0 keeps every block-row raw.
 // Nodes are ordered boundary-first (nodes of the partition interface, then interior) and, inside windows of
 // SIGMA nodes, by decreasing block count, so slices are almost padding-free; all vectors (d0, dn, M, F) live
 // in that internal order (row = 3*node + component) and are streamed.  The only non-streaming access is the
@@ -42,7 +49,7 @@ namespace cg = cooperative_groups;
 #define SAA_DOT_MODE 0
 #endif
 #ifndef SAA_UNROLL
-#define SAA_UNROLL 2          // blocks whose loads are in flight together per thread (2 x at most 76 B x 32 lanes per warp)
+#define SAA_UNROLL 2          // blocks whose loads are in flight together per thread
 #endif
 
 struct SaaDev {
@@ -50,9 +57,11 @@ struct SaaDev {
     int64_t n_slices;          // slices of 32 nodes
     int64_t sh_slices;         // slices [0, sh_slices) hold the shared (interface) nodes
     const int64_t *slice_ptr;  // [n_slices + 1] offsets in block-lanes (multiples of 32)
-    const int64_t *val_ptr;    // [n_slices + 1] offsets of the slices in val, in doubles
-    const uint16_t *pmask;     // [block-rows] stored value planes of each block-row (see above)
-    const double *val;         // stored value planes
+    const int64_t *val_ptr;    // [n_slices + 1] offsets of the slices in val, in doubles (8 B)
+    const int64_t *vb_ptr;     // [n_slices + 1] offsets of the slices in vbase (coded planes before the slice)
+    const uint16_t *pmask;     // [block-rows] stored value planes and coding flag of each block-row (see above)
+    const double *val;         // stored value planes: raw (256 B) or coded (64 B of 16-bit lane offsets)
+    const long long *vbase;    // bases of the coded planes, in plane order
     const int32_t *col;        // internal column NODE ids
     const uint32_t *dir_mask;  // bit (row & 31) of word (row >> 5) set: row is a Dirichlet DOF
     const double *M;           // lumped mass, internal row order — or one value per NODE when node_mass is set (all three
@@ -174,7 +183,6 @@ __device__ __forceinline__ double saa_ramp(double t) { return (t <= 1.0) ? t : 1
 // and nothing after it may be hoisted above it.  Used to make ALL loads of a batch issue back to back (the
 // compiler otherwise interleaves each dependent multiply-add right behind its own load, which stalls the warp on
 // the first outstanding load and leaves only 3-4 requests in flight).
-#define SAA_FENCE9(a) asm volatile("" : "+d"(a[0]), "+d"(a[1]), "+d"(a[2]), "+d"(a[3]), "+d"(a[4]), "+d"(a[5]), "+d"(a[6]), "+d"(a[7]), "+d"(a[8]))
 #define SAA_FENCE3(x) asm volatile("" : "+d"(x[0]), "+d"(x[1]), "+d"(x[2]))
 
 template <bool NC_X>
@@ -193,60 +201,191 @@ __device__ __forceinline__ void saa_block_madd(const double (&a)[9], const doubl
         for (int b = 0; b < 3; ++b) s[A] = __dadd_rn(s[A], __dmul_rn(a[3 * A + b], xv[b]));
 }
 
-// Value planes of one block: plane e is loaded iff bit e of the block's plane mask m is set (m is warp-uniform, so the
-// predicate is too); otherwise a[e] = 0.0, the value every lane would have loaded from a full-plane layout.  v points
-// at the block's first stored plane (of this lane); the stored planes follow each other in bit order.
-__device__ __forceinline__ double ld_stream_f64_if(const double *p, unsigned pred)
+#define SAA_PLANES 0x1FFu      // bits 0-8 of a plane mask: the stored planes of the block-row
+#define SAA_CODED 0x8000u      // bit 15: the block-row's planes are coded (int64 base + 16-bit lane offsets)
+
+// Predicated loads: 0 (the bits of 0.0) when pred is 0.  pred is warp-uniform.  Each destination register is written
+// by one load only, so that ptxas never has to order two loads of the same register.
+__device__ __forceinline__ unsigned long long ld_b64_if(const char *p, unsigned pred)
 {
-    double v;
-    asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %2, 0;\n\tmov.b64 %0, 0d0000000000000000;\n\t"
-                 "@q ld.global.nc.L1::no_allocate.f64 %0, [%1];\n\t}"
-                 : "=&d"(v) : "l"(p), "r"(pred));
+    unsigned long long v;
+    asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %2, 0;\n\tmov.b64 %0, 0;\n\t"
+                 "@q ld.global.nc.L1::no_allocate.b64 %0, [%1];\n\t}"
+                 : "=&l"(v) : "l"(p), "r"(pred));
     return v;
 }
-__device__ __forceinline__ void saa_load_block(const double *v, unsigned m, double (&a)[9])
+// bases of coded planes go through L1: the block's bases share one or two sectors
+__device__ __forceinline__ long long ld_base_if(const long long *p, unsigned pred)
+{
+    long long v;
+    asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %2, 0;\n\tmov.b64 %0, 0;\n\t"
+                 "@q ld.global.nc.s64 %0, [%1];\n\t}"
+                 : "=&l"(v) : "l"(p), "r"(pred));
+    return v;
+}
+__device__ __forceinline__ void prefetch_l2_if(const char *p, unsigned pred)
+{
+    asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %1, 0;\n\t@q prefetch.global.L2 [%0];\n\t}" ::"l"(p), "r"(pred));
+}
+__device__ __forceinline__ uint4 ld_v4_if(const char *p, unsigned pred)
+{
+    uint4 v;
+    asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %5, 0;\n\tmov.b32 %0, 0;\n\tmov.b32 %1, 0;\n\tmov.b32 %2, 0;\n\tmov.b32 %3, 0;\n\t"
+                 "@q ld.global.nc.L1::no_allocate.v4.u32 {%0, %1, %2, %3}, [%4];\n\t}"
+                 : "=&r"(v.x), "=&r"(v.y), "=&r"(v.z), "=&r"(v.w) : "l"(p), "r"(pred));
+    return v;
+}
+__device__ __forceinline__ unsigned ld_u32_if(const char *p, unsigned pred)
+{
+    unsigned v;
+    asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %2, 0;\n\tmov.b32 %0, 0;\n\t"
+                 "@q ld.global.nc.L1::no_allocate.u32 %0, [%1];\n\t}"
+                 : "=&r"(v) : "l"(p), "r"(pred));
+    return v;
+}
+// A block in flight.  The coded planes of a block are contiguous (n planes x 64 B, at most 576 B), so the warp loads
+// them as one region with wide loads, two requests instead of one per plane: lane l gets bytes [16 l, 16 l + 16) in
+// q and lanes l < 16 bytes [512 + 4 l, 512 + 4 l + 4) in r.  Lane i < n also loads (the low word of) the base of the
+// block's i-th plane.  A raw
+// block-row only has its stored planes prefetched into L2 (no register is held for them); 96 % of the planes of the
+// structured beam at 104 M DOF are coded (DESIGN.md §4).  saa_decode_block, once the loads of the batch have arrived, passes the region
+// and the bases through the warp's staging area in shared memory to hand every lane its offsets and bases, and forms
+// base + offset, or loads the raw planes now (from L2).
+struct SaaBlk {
+    uint4 q;
+    unsigned r;
+    long long bl;         // base of the block's (lane)-th plane
+    unsigned m;           // plane mask
+    int vo, bo;           // byte offset of the block's first plane in the slice's values, index of its first base
+};
+__device__ __forceinline__ void saa_load_block(const char *vs, const long long *bs, int lane, unsigned m, int vo, int bo, SaaBlk &k)
+{
+    k.m = m; k.vo = vo; k.bo = bo; k.bl = 0; k.r = 0;
+    k.q = make_uint4(0u, 0u, 0u, 0u);
+    const char *v = vs + vo;
+    const int n = __popc(m & SAA_PLANES);
+    if (m & SAA_CODED) {
+        k.q = ld_v4_if(v + 16 * lane, 16 * lane < 64 * n);
+        k.r = ld_u32_if(v + 512 + 4 * lane, 512 + 4 * lane < 64 * n);
+        k.bl = ld_base_if(bs + bo + lane, lane < n);
+    } else {
+#pragma unroll
+        for (int e = 0; e < 9; ++e) prefetch_l2_if(v + 256 * __popc(m & ((1u << e) - 1u)) + 8 * lane, m & (1u << e));
+    }
+}
+// stage: this warp's staging area in shared memory (576 B of offsets, 72 B of bases; 16-B aligned)
+__device__ __forceinline__ void saa_decode_block(const char *vs, const long long *bs, int lane, const SaaBlk &k, unsigned char *stage,
+                                                 double (&a)[9])
+{
+    const unsigned m = k.m;
+    if (m & SAA_CODED) {
+        __syncwarp();                                  // every lane has read the previous block's offsets
+        *(uint4 *)(stage + 16 * lane) = k.q;
+        if (lane < 16) *(unsigned *)(stage + 512 + 4 * lane) = k.r;
+        if (lane < 9) *(long long *)(stage + 576 + 8 * lane) = k.bl;
+        __syncwarp();
+#pragma unroll
+        for (int e = 0; e < 9; ++e) {
+            const int i = __popc(m & ((1u << e) - 1u));
+            long long bits = 0;
+            if (m & (1u << e)) bits = *(const long long *)(stage + 576 + 8 * i) + *(const uint16_t *)(stage + 64 * i + 2 * lane);
+            a[e] = __longlong_as_double(bits);
+        }
+    } else {
+        const char *v = vs + k.vo;
+#pragma unroll
+        for (int e = 0; e < 9; ++e)
+            a[e] = __longlong_as_double((long long)ld_b64_if(v + 256 * __popc(m & ((1u << e) - 1u)) + 8 * lane, m & (1u << e)));
+    }
+}
+// the staging area of the calling warp (every kernel that reads the matrix runs blocks of at most 8 warps)
+__device__ __forceinline__ unsigned char *saa_stage()
+{
+    __shared__ __align__(16) unsigned char stage[8][656];
+    return stage[(threadIdx.x >> 5) & 7];
+}
+#define SAA_FENCE_BLK(k) asm volatile("" : "+r"(k.q.x), "+r"(k.q.y), "+r"(k.q.z), "+r"(k.q.w), "+r"(k.r), "+l"(k.bl))
+// one lane's values of one block, for lanes that do not walk the slice together
+__device__ __forceinline__ void saa_load_block_lane(const char *v, const long long *b, int lane, unsigned m, double (&a)[9])
 {
 #pragma unroll
-    for (int e = 0; e < 9; ++e) a[e] = ld_stream_f64_if(v + 32 * __popc(m & ((1u << e) - 1u)), m & (1u << e));
+    for (int e = 0; e < 9; ++e) {
+        const int i = __popc(m & ((1u << e) - 1u));
+        long long bits = 0;
+        if (m & (1u << e)) {
+            if (m & SAA_CODED) bits = __ldg(b + i) + ((const uint16_t *)(v + 64 * i))[lane];
+            else bits = ((const long long *)(v + 256 * i))[lane];
+        }
+        a[e] = __longlong_as_double(bits);
+    }
+}
+// moves the cursors past a block with mask m
+__device__ __forceinline__ void saa_next_block(const char *&v, const long long *&b, unsigned m)
+{
+    const int n = __popc(m & SAA_PLANES);
+    if (m & SAA_CODED) { v += 64 * n; b += n; } else { v += 256 * n; }
+}
+__device__ __forceinline__ void saa_next_block(int &vo, int &bo, unsigned m)
+{
+    const int n = __popc(m & SAA_PLANES);
+    if (m & SAA_CODED) { vo += 64 * n; bo += n; } else { vo += 256 * n; }
 }
 
+// column ids and plane masks run one batch ahead of the values, so that the gathers of a batch are issued together
+// with its value loads instead of after a first round trip
 template <int UNROLL, bool NC_X>
 __device__ __forceinline__ void saa_node_dot_pipe(const SaaDev &P, int64_t slice, int lane, const double *x, double (&s)[3])
 {
-    static_assert(UNROLL == 2, "the software pipeline below is written for two blocks per batch");
     const int64_t beg = P.slice_ptr[slice];
     const int len = (int)((P.slice_ptr[slice + 1] - beg) >> 5);
-    const double *v = P.val + P.val_ptr[slice] + lane;
+    const char *vs = (const char *)(P.val + P.val_ptr[slice]);
+    const long long *bs = P.vbase + P.vb_ptr[slice];
+    unsigned char *stage = saa_stage();
     const int32_t *c = P.col + beg + lane;
     const uint16_t *mk = P.pmask + (beg >> 5);
     s[0] = 0.0; s[1] = 0.0; s[2] = 0.0;
-    // column ids and plane masks run one batch ahead of the values, so that the gathers of a batch are issued together
-    // with its value loads instead of after a first round trip
-    int32_t k0 = 0, k1 = 0;
-    unsigned m0 = 0, m1 = 0;
-    if (len > 0) { k0 = ld_stream_s32(c); m0 = __ldg(mk); }
-    if (len > 1) { k1 = ld_stream_s32(c + 32); m1 = __ldg(mk + 1); }
-    int j = 0;
-    for (; j + 2 <= len; j += 2) {
-        double a0[9], a1[9], x0[3], x1[3];
-        saa_load_block(v, m0, a0);
-        v += 32 * __popc(m0);
-        saa_load_block(v, m1, a1);
-        v += 32 * __popc(m1);
-        saa_gather3<NC_X>(x, k0, x0);
-        saa_gather3<NC_X>(x, k1, x1);
-        if (j + 2 < len) { k0 = ld_stream_s32(c + 32 * (j + 2)); m0 = __ldg(mk + j + 2); }
-        if (j + 3 < len) { k1 = ld_stream_s32(c + 32 * (j + 3)); m1 = __ldg(mk + j + 3); }
-        SAA_FENCE9(a0); SAA_FENCE9(a1); SAA_FENCE3(x0); SAA_FENCE3(x1);
-        saa_block_madd(a0, x0, s);              // blocks in ascending column order: the order of the CSR row
-        saa_block_madd(a1, x1, s);
+    int32_t k[UNROLL];
+    unsigned m[UNROLL];
+#pragma unroll
+    for (int u = 0; u < UNROLL; ++u) {
+        k[u] = 0; m[u] = 0;
+        if (u < len) { k[u] = ld_stream_s32(c + 32 * u); m[u] = __ldg(mk + u); }
     }
-    if (j < len) {
-        double a0[9], x0[3];
-        saa_load_block(v, m0, a0);
-        saa_gather3<NC_X>(x, k0, x0);
-        saa_block_madd(a0, x0, s);
+    int vo = 0, bo = 0, j = 0;
+    for (; j + UNROLL <= len; j += UNROLL) {
+        SaaBlk blk[UNROLL];
+        double xv[UNROLL][3];
+#pragma unroll
+        for (int u = 0; u < UNROLL; ++u) {
+            saa_load_block(vs, bs, lane, m[u], vo, bo, blk[u]);
+            saa_next_block(vo, bo, m[u]);
+        }
+#pragma unroll
+        for (int u = 0; u < UNROLL; ++u) saa_gather3<NC_X>(x, k[u], xv[u]);
+#pragma unroll
+        for (int u = 0; u < UNROLL; ++u)
+            if (j + UNROLL + u < len) { k[u] = ld_stream_s32(c + 32 * (j + UNROLL + u)); m[u] = __ldg(mk + j + UNROLL + u); }
+#pragma unroll
+        for (int u = 0; u < UNROLL; ++u) { SAA_FENCE_BLK(blk[u]); SAA_FENCE3(xv[u]); }
+#pragma unroll
+        for (int u = 0; u < UNROLL; ++u) {              // blocks in ascending column order: the order of the CSR row
+            double a[9];
+            saa_decode_block(vs, bs, lane, blk[u], stage, a);
+            saa_block_madd(a, xv[u], s);
+        }
     }
+#pragma unroll
+    for (int u = 0; u + 1 < UNROLL; ++u)                // the last len - j < UNROLL blocks, ids and masks already loaded
+        if (j + u < len) {
+            SaaBlk blk;
+            double a[9], xv[3];
+            saa_load_block(vs, bs, lane, m[u], vo, bo, blk);
+            saa_next_block(vo, bo, m[u]);
+            saa_gather3<NC_X>(x, k[u], xv);
+            SAA_FENCE_BLK(blk);
+            saa_decode_block(vs, bs, lane, blk, stage, a);
+            saa_block_madd(a, xv, s);
+        }
 }
 
 // plain form: the compiler schedules the loads of UNROLL blocks against the dependent add chains
@@ -255,53 +394,46 @@ __device__ __forceinline__ void saa_node_dot_simple(const SaaDev &P, int64_t sli
 {
     const int64_t beg = P.slice_ptr[slice];
     const int len = (int)((P.slice_ptr[slice + 1] - beg) >> 5);
-    const double *v = P.val + P.val_ptr[slice] + lane;
+    const char *vs = (const char *)(P.val + P.val_ptr[slice]);
+    const long long *bs = P.vbase + P.vb_ptr[slice];
+    unsigned char *stage = saa_stage();
     const int32_t *c = P.col + beg + lane;
     const uint16_t *mk = P.pmask + (beg >> 5);
     s[0] = 0.0; s[1] = 0.0; s[2] = 0.0;
-    int j = 0;
+    int vo = 0, bo = 0, j = 0;
     for (; j + UNROLL <= len; j += UNROLL) {
-        double a[UNROLL][9];
+        SaaBlk blk[UNROLL];
         int32_t k[UNROLL];
-        unsigned m[UNROLL];
         double xv[UNROLL][3];
 #pragma unroll
-        for (int u = 0; u < UNROLL; ++u) {
-            k[u] = ld_stream_s32(c + 32 * (j + u));
-            m[u] = __ldg(mk + j + u);
-        }
+        for (int u = 0; u < UNROLL; ++u) k[u] = ld_stream_s32(c + 32 * (j + u));
 #pragma unroll
         for (int u = 0; u < UNROLL; ++u) {
-            saa_load_block(v, m[u], a[u]);
-            v += 32 * __popc(m[u]);
+            const unsigned m = __ldg(mk + j + u);
+            saa_load_block(vs, bs, lane, m, vo, bo, blk[u]);
+            saa_next_block(vo, bo, m);
         }
+#pragma unroll
+        for (int u = 0; u < UNROLL; ++u) saa_gather3<NC_X>(x, k[u], xv[u]);
 #pragma unroll
         for (int u = 0; u < UNROLL; ++u) {
-            const double *xp = x + 3 * (int64_t)k[u];
-#pragma unroll
-            for (int b = 0; b < 3; ++b) xv[u][b] = NC_X ? __ldg(xp + b) : xp[b];
+            double a[9];
+            SAA_FENCE_BLK(blk[u]);
+            saa_decode_block(vs, bs, lane, blk[u], stage, a);
+            saa_block_madd(a, xv[u], s);
         }
-#pragma unroll
-        for (int u = 0; u < UNROLL; ++u)
-#pragma unroll
-            for (int A = 0; A < 3; ++A)
-#pragma unroll
-                for (int b = 0; b < 3; ++b) s[A] = __dadd_rn(s[A], __dmul_rn(a[u][3 * A + b], xv[u][b]));
     }
     for (; j < len; ++j) {
         const int32_t k = ld_stream_s32(c + 32 * j);
         const unsigned m = __ldg(mk + j);
-        double a[9];
-        saa_load_block(v, m, a);
-        v += 32 * __popc(m);
-        const double *xp = x + 3 * (int64_t)k;
-        double xv[3];
-#pragma unroll
-        for (int b = 0; b < 3; ++b) xv[b] = NC_X ? __ldg(xp + b) : xp[b];
-#pragma unroll
-        for (int A = 0; A < 3; ++A)
-#pragma unroll
-            for (int b = 0; b < 3; ++b) s[A] = __dadd_rn(s[A], __dmul_rn(a[3 * A + b], xv[b]));
+        SaaBlk blk;
+        double a[9], xv[3];
+        saa_load_block(vs, bs, lane, m, vo, bo, blk);
+        saa_next_block(vo, bo, m);
+        saa_gather3<NC_X>(x, k, xv);
+        SAA_FENCE_BLK(blk);
+        saa_decode_block(vs, bs, lane, blk, stage, a);
+        saa_block_madd(a, xv, s);
     }
 }
 

@@ -312,15 +312,16 @@ __global__ void __launch_bounds__(256) saa_k_cg_diag(SaaDev P, double *__restric
     if (slice >= P.n_slices) return;
     const int64_t node = slice * 32 + lane, beg = P.slice_ptr[slice];
     const int len = (int)((P.slice_ptr[slice + 1] - beg) >> 5);
-    const double *v = P.val + P.val_ptr[slice] + lane;
+    const char *v = (const char *)(P.val + P.val_ptr[slice]);
+    const long long *b = P.vbase + P.vb_ptr[slice];
     double a[9] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
     for (int j = 0; j < len; ++j) {
         const unsigned m = P.pmask[(beg >> 5) + j];
         if (P.col[beg + 32 * j + lane] == (int32_t)node) {
-            saa_load_block(v, m, a);
+            saa_load_block_lane(v, b, lane, m, a);
             break;
         }
-        v += 32 * __popc(m);
+        saa_next_block(v, b, m);
     }
 #pragma unroll
     for (int A = 0; A < 3; ++A) {

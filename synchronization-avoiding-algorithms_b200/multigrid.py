@@ -153,7 +153,7 @@ class StructuredMultigrid:
         _check(lib().saa_mg_info(self.h, lam.ctypes.data_as(ctypes.c_void_p), ctypes.byref(own)), "saa_mg_info")
         self.lambda_max = [float(v) for v in lam]
         # the hierarchy's own vectors, tables and coarsest inverse, plus the coarse plans' matrices and vectors
-        self.bytes = int(own.value) + sum(p.matrix_bytes + p.vector_bytes for p in self._plans)
+        self.bytes = int(own.value) + sum(p.streamed_matrix_bytes + p.vector_bytes for p in self._plans)
 
     def handle(self):
         if not self.h:

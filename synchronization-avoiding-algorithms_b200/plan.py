@@ -48,8 +48,10 @@ ABI = {
     "saa_plan_nnz": (_i64, [_vp]),
     "saa_plan_padded_entries": (_i64, [_vp]),
     "saa_plan_value_planes": (_i64, [_vp]),
+    "saa_plan_coded_planes": (_i64, [_vp]),
     "saa_plan_kernel_launches": (_i64, [_vp]),
     "saa_plan_matrix_bytes": (_i64, [_vp]),
+    "saa_plan_streamed_matrix_bytes": (_i64, [_vp]),
     "saa_plan_vector_bytes": (_i64, [_vp]),
     "saa_plan_set_state": (_int, [_vp, _vp, _vp, _f64]),
     "saa_plan_get_state": (_int, [_vp, _vp, _vp, _vp]),
@@ -361,13 +363,23 @@ class StepPlan:
 
     @property
     def value_planes(self):
-        """value planes the step kernel streams (32 fp64 each); padded_entries / 32 when every plane is stored"""
+        """value planes the step kernel streams, raw or coded; padded_entries / 32 when every plane is stored"""
         return int(lib().saa_plan_value_planes(self.h))
 
     @property
+    def coded_planes(self):
+        """value planes stored as an int64 base + 32 16-bit lane offsets (64 B instead of 256 B)"""
+        return int(lib().saa_plan_coded_planes(self.h))
+
+    @property
     def matrix_bytes(self):
-        """bytes of matrix storage the step kernel streams per time step"""
+        """bytes of the plane-masked matrix layout without value coding (256 B per value plane)"""
         return int(lib().saa_plan_matrix_bytes(self.h))
+
+    @property
+    def streamed_matrix_bytes(self):
+        """bytes of matrix storage the step kernel streams per time step (coded planes at their coded size)"""
+        return int(lib().saa_plan_streamed_matrix_bytes(self.h))
 
     @property
     def vector_bytes(self):
