@@ -218,12 +218,13 @@ __global__ void saa_k_fin_fill(int64_t n_slices, const int64_t *__restrict__ sli
         const int32_t cn = saa_fin_next_block(t, e >= 0, indices, data, a);
         cs[32 * (int64_t)j] = (cn != INT32_MAX) ? iperm[3 * (int64_t)cn] / 3 : (int32_t)inode;
         const unsigned m = ms[j];
+        const int n = __popc(m & SAA_PLANES);
         int i = 0;
         for (int k = 0; k < 9; ++k)
             if (m & (1u << k)) {
-                if (m & SAA_CODED) {
+                if (m & SAA_CODED) {                       // lane-major offsets (saa_coded_off)
                     const long long x = __double_as_longlong(a[k]), lo = saa_warp_min64(x);
-                    ((uint16_t *)(v + 64 * i))[lane] = (uint16_t)((unsigned long long)x - (unsigned long long)lo);
+                    *(uint16_t *)(v + saa_coded_off(n, i, lane)) = (uint16_t)((unsigned long long)x - (unsigned long long)lo);
                     if (lane == 0) vb[i] = lo;
                 } else {
                     ((double *)(v + 256 * i))[lane] = a[k];

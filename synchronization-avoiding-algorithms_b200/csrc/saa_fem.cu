@@ -520,20 +520,19 @@ extern "C" int saa_plan_finalize(saa_plan *p)
         for (int64_t r = slice_ptr[s] / 32; r < slice_ptr[s + 1] / 32; ++r) {
             const int n = __builtin_popcount(pmask[r] & SAA_PLANES);
             for (int i = 0; i < n; ++i, pl += 32) {
-                if (pmask[r] & SAA_CODED) {
+                if (pmask[r] & SAA_CODED) {                // lane-major offsets (saa_coded_off)
                     int64_t lo = INT64_MAX;
                     for (int l = 0; l < 32; ++l) lo = std::min(lo, bits(pl[l]));
                     *vb++ = lo;
                     for (int l = 0; l < 32; ++l) {
                         const uint16_t o = (uint16_t)((uint64_t)bits(pl[l]) - (uint64_t)lo);
-                        std::memcpy(v + 2 * l, &o, 2);
+                        std::memcpy(v + saa_coded_off(n, i, l), &o, 2);
                     }
-                    v += 64;
                 } else {
-                    std::memcpy(v, pl, 256);
-                    v += 256;
+                    std::memcpy(v + 256 * i, pl, 256);
                 }
             }
+            v += ((pmask[r] & SAA_CODED) ? 64 : 256) * n;
         }
     }
     std::vector<double>().swap(raw);

@@ -20,7 +20,8 @@
 //     plane (A,B) of block j  :  the (off_j + popc(pmask[r] & ((1 << (3A+B)) - 1)))-th plane of the slice, if that bit is set
 // where off_j is the number of planes stored for blocks 0..j-1 of the slice.  The planes of a slice follow each other
 // from byte 8*val_ptr[s] of val on: a raw plane is 32 fp64 (256 B); a plane of a coded block-row is 32 uint16 lane
-// offsets (64 B) from a per-plane int64 base, vbase[vb_ptr[s] + number of coded planes of the slice before it], and
+// offsets (64 B, stored lane-major across the block-row's planes, saa_coded_off) from a per-plane int64 base,
+// vbase[vb_ptr[s] + number of coded planes of the slice before it], and
 // lane l's value is the double whose bits are base + offset[l] (pure integer, bit-exact).  A block-row is coded iff
 // every one of its stored planes spans at most 65535 between the smallest and the largest bit pattern of its 32
 // lanes read as int64 (finalisation decides from the stored bits, padding lanes included).
@@ -227,14 +228,6 @@ __device__ __forceinline__ void prefetch_l2_if(const char *p, unsigned pred)
 {
     asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %1, 0;\n\t@q prefetch.global.L2 [%0];\n\t}" ::"l"(p), "r"(pred));
 }
-__device__ __forceinline__ uint4 ld_v4_if(const char *p, unsigned pred)
-{
-    uint4 v;
-    asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %5, 0;\n\tmov.b32 %0, 0;\n\tmov.b32 %1, 0;\n\tmov.b32 %2, 0;\n\tmov.b32 %3, 0;\n\t"
-                 "@q ld.global.nc.L1::no_allocate.v4.u32 {%0, %1, %2, %3}, [%4];\n\t}"
-                 : "=&r"(v.x), "=&r"(v.y), "=&r"(v.z), "=&r"(v.w) : "l"(p), "r"(pred));
-    return v;
-}
 __device__ __forceinline__ unsigned ld_u32_if(const char *p, unsigned pred)
 {
     unsigned v;
@@ -243,77 +236,137 @@ __device__ __forceinline__ unsigned ld_u32_if(const char *p, unsigned pred)
                  : "=&r"(v) : "l"(p), "r"(pred));
     return v;
 }
-// A block in flight.  The coded planes of a block are contiguous (n planes x 64 B, at most 576 B), so the warp loads
-// them as one region with wide loads, two requests instead of one per plane: lane l gets bytes [16 l, 16 l + 16) in
-// q and lanes l < 16 bytes [512 + 4 l, 512 + 4 l + 4) in r.  Lane i < n also loads (the low word of) the base of the
-// block's i-th plane.  A raw
-// block-row only has its stored planes prefetched into L2 (no register is held for them); 96 % of the planes of the
-// structured beam at 104 M DOF are coded (DESIGN.md §4).  saa_decode_block, once the loads of the batch have arrived, passes the region
-// and the bases through the warp's staging area in shared memory to hand every lane its offsets and bases, and forms
-// base + offset, or loads the raw planes now (from L2).
+__device__ __forceinline__ unsigned short ld_u16_if(const char *p, unsigned pred)
+{
+    unsigned short v;
+    asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.u32 q, %2, 0;\n\tmov.b16 %0, 0;\n\t"
+                 "@q ld.global.nc.L1::no_allocate.u16 %0, [%1];\n\t}"
+                 : "=&h"(v) : "l"(p), "r"(pred));
+    return v;
+}
+// Lane-major offsets of a coded block-row with n stored planes, n = 4a + 2b + c (b, c in {0, 1}): a chunks of 256 B,
+// where lane l's 8 bytes at 8 l hold its offsets of stored planes 4g .. 4g+3 (chunk g); then, if b, a chunk of 128 B
+// with lane l's offsets of planes 4a, 4a+1 at 4 l; then, if c, a chunk of 64 B with lane l's offset of plane n-1 at
+// 2 l.  Byte offset of lane l's offset of stored plane i from the block-row's first offset:
+__host__ __device__ __forceinline__ int saa_coded_off(int n, int i, int lane)
+{
+    const int a4 = n & ~3, n2 = n & ~1;
+    if (i < a4) return 256 * (i >> 2) + 8 * lane + 2 * (i & 3);
+    if (i < n2) return 64 * a4 + 4 * lane + 2 * (i - a4);
+    return 64 * n2 + 2 * lane;
+}
+// A block in flight.  Every lane loads its own offsets of a coded block-row straight into registers, with at most four
+// aligned warp-wide loads predicated on the warp-uniform n: chunk 0 -> q0, chunk 1 -> q1 (64 bit), the 128-B chunk -> h,
+// the 64-B chunk -> t.  Lane i < n also loads the base of the block's i-th stored plane; the decode broadcasts it with
+// two shuffles.  A raw block-row only has its stored planes prefetched into L2 (no register is held for them); 96 % of
+// the planes of the structured beam at 104 M DOF are coded (DESIGN.md §4), and the raw planes are loaded at decode time.
 struct SaaBlk {
-    uint4 q;
-    unsigned r;
-    long long bl;         // base of the block's (lane)-th plane
-    unsigned m;           // plane mask
+    unsigned long long q0, q1;
+    unsigned h;
+    unsigned short t;
+    long long bl;         // base of the block's (lane)-th stored plane
+    unsigned m;           // plane mask, warp-uniform
     int vo, bo;           // byte offset of the block's first plane in the slice's values, index of its first base
 };
 __device__ __forceinline__ void saa_load_block(const char *vs, const long long *bs, int lane, unsigned m, int vo, int bo, SaaBlk &k)
 {
-    k.m = m; k.vo = vo; k.bo = bo; k.bl = 0; k.r = 0;
-    k.q = make_uint4(0u, 0u, 0u, 0u);
+    k.m = m; k.vo = vo; k.bo = bo; k.bl = 0; k.q0 = 0; k.q1 = 0; k.h = 0; k.t = 0;
     const char *v = vs + vo;
     const int n = __popc(m & SAA_PLANES);
     if (m & SAA_CODED) {
-        k.q = ld_v4_if(v + 16 * lane, 16 * lane < 64 * n);
-        k.r = ld_u32_if(v + 512 + 4 * lane, 512 + 4 * lane < 64 * n);
+        k.q0 = ld_b64_if(v + 8 * lane, n >= 4);
+        k.q1 = ld_b64_if(v + 256 + 8 * lane, n >= 8);
+        k.h = ld_u32_if(v + 64 * (n & ~3) + 4 * lane, n & 2);
+        k.t = ld_u16_if(v + 64 * (n & ~1) + 2 * lane, n & 1);
         k.bl = ld_base_if(bs + bo + lane, lane < n);
     } else {
 #pragma unroll
-        for (int e = 0; e < 9; ++e) prefetch_l2_if(v + 256 * __popc(m & ((1u << e) - 1u)) + 8 * lane, m & (1u << e));
+        for (int i = 0; i < 9; ++i) prefetch_l2_if(v + 256 * i + 8 * lane, i < n);      // the n stored planes follow each other
     }
 }
-// stage: this warp's staging area in shared memory (576 B of offsets, 72 B of bases; 16-B aligned)
-__device__ __forceinline__ void saa_decode_block(const char *vs, const long long *bs, int lane, const SaaBlk &k, unsigned char *stage,
-                                                 double (&a)[9])
+// lane's offset of stored plane I of a coded block with N stored planes (compile-time register and half-word)
+template <int N, int I>
+__device__ __forceinline__ unsigned saa_slot(const SaaBlk &k)
+{
+    if (I < (N & ~3)) return (unsigned)((I < 4 ? k.q0 : k.q1) >> (16 * (I & 3))) & 0xFFFFu;
+    if (I < (N & ~1)) return (I == (N & ~3)) ? (k.h & 0xFFFFu) : (k.h >> 16);
+    return k.t;
+}
+__device__ __forceinline__ long long saa_base(const SaaBlk &k, int i) { return __shfl_sync(0xFFFFFFFFu, k.bl, i); }
+template <unsigned MASK, int E = 0, int I = 0>
+__device__ __forceinline__ void saa_decode_fixed(const SaaBlk &k, double (&a)[9])
+{
+    if constexpr (E < 9) {
+        if constexpr ((MASK >> E) & 1u) {
+            a[E] = __longlong_as_double(saa_base(k, I) + saa_slot<__builtin_popcount(MASK), I>(k));
+            saa_decode_fixed<MASK, E + 1, I + 1>(k, a);
+        } else {
+            a[E] = 0.0;
+            saa_decode_fixed<MASK, E + 1, I>(k, a);
+        }
+    }
+}
+// a raw block with a mask known at compile time: the planes' addresses need no popcounts
+template <unsigned MASK, int E = 0, int I = 0>
+__device__ __forceinline__ void saa_decode_raw_fixed(const char *v, double (&a)[9])
+{
+    if constexpr (E < 9) {
+        if constexpr ((MASK >> E) & 1u) {
+            a[E] = __longlong_as_double((long long)ld_b64_if(v + 256 * I, 1u));
+            saa_decode_raw_fixed<MASK, E + 1, I + 1>(v, a);
+        } else {
+            a[E] = 0.0;
+            saa_decode_raw_fixed<MASK, E + 1, I>(v, a);
+        }
+    }
+}
+// Every lane forms base + offset of the block's planes, 0.0 for a plane that is not stored.  The masks of the coded
+// block-rows of the structured beam (DESIGN.md §3) get a decode with compile-time registers, and raw block-rows with
+// those masks compile-time plane addresses; any other mask takes the generic path, which lines the offsets up as
+// slots 0-3 of lo, 4-7 of hi and 8 of t (slot i = stored plane i).
+__device__ __forceinline__ void saa_decode_block(const char *vs, int lane, const SaaBlk &k, double (&a)[9])
 {
     const unsigned m = k.m;
     if (m & SAA_CODED) {
-        __syncwarp();                                  // every lane has read the previous block's offsets
-        *(uint4 *)(stage + 16 * lane) = k.q;
-        if (lane < 16) *(unsigned *)(stage + 512 + 4 * lane) = k.r;
-        if (lane < 9) *(long long *)(stage + 576 + 8 * lane) = k.bl;
-        __syncwarp();
+        switch (m & SAA_PLANES) {
+        case 0x1FFu: saa_decode_fixed<0x1FFu>(k, a); break;
+        case 0x0EEu: saa_decode_fixed<0x0EEu>(k, a); break;
+        default: {
+            const int n = __popc(m & SAA_PLANES);
+            const unsigned long long tail = (n & 2) ? (k.h | ((unsigned long long)k.t << 32)) : k.t;
+            const unsigned long long lo = (n < 4) ? tail : k.q0, hi = (n < 4) ? 0ull : (n < 8) ? tail : k.q1;
 #pragma unroll
-        for (int e = 0; e < 9; ++e) {
-            const int i = __popc(m & ((1u << e) - 1u));
-            long long bits = 0;
-            if (m & (1u << e)) bits = *(const long long *)(stage + 576 + 8 * i) + *(const uint16_t *)(stage + 64 * i + 2 * lane);
-            a[e] = __longlong_as_double(bits);
+            for (int e = 0; e < 9; ++e) {
+                const int i = __popc(m & ((1u << e) - 1u));
+                long long bits = 0;
+                if (m & (1u << e)) bits = saa_base(k, i) + (long long)(((i < 4 ? lo : i < 8 ? hi : k.t) >> (16 * (i & 3))) & 0xFFFFull);
+                a[e] = __longlong_as_double(bits);
+            }
+        }
         }
     } else {
-        const char *v = vs + k.vo;
+        const char *v = vs + k.vo + 8 * lane;
+        switch (m & SAA_PLANES) {
+        case 0x1FFu: saa_decode_raw_fixed<0x1FFu>(v, a); break;
+        case 0x0EEu: saa_decode_raw_fixed<0x0EEu>(v, a); break;
+        default:
 #pragma unroll
-        for (int e = 0; e < 9; ++e)
-            a[e] = __longlong_as_double((long long)ld_b64_if(v + 256 * __popc(m & ((1u << e) - 1u)) + 8 * lane, m & (1u << e)));
+            for (int e = 0; e < 9; ++e)
+                a[e] = __longlong_as_double((long long)ld_b64_if(v + 256 * __popc(m & ((1u << e) - 1u)), m & (1u << e)));
+        }
     }
 }
-// the staging area of the calling warp (every kernel that reads the matrix runs blocks of at most 8 warps)
-__device__ __forceinline__ unsigned char *saa_stage()
-{
-    __shared__ __align__(16) unsigned char stage[8][656];
-    return stage[(threadIdx.x >> 5) & 7];
-}
-#define SAA_FENCE_BLK(k) asm volatile("" : "+r"(k.q.x), "+r"(k.q.y), "+r"(k.q.z), "+r"(k.q.w), "+r"(k.r), "+l"(k.bl))
+#define SAA_FENCE_BLK(k) asm volatile("" : "+l"(k.q0), "+l"(k.q1), "+r"(k.h), "+h"(k.t), "+l"(k.bl))
 // one lane's values of one block, for lanes that do not walk the slice together
 __device__ __forceinline__ void saa_load_block_lane(const char *v, const long long *b, int lane, unsigned m, double (&a)[9])
 {
+    const int n = __popc(m & SAA_PLANES);
 #pragma unroll
     for (int e = 0; e < 9; ++e) {
         const int i = __popc(m & ((1u << e) - 1u));
         long long bits = 0;
         if (m & (1u << e)) {
-            if (m & SAA_CODED) bits = __ldg(b + i) + ((const uint16_t *)(v + 64 * i))[lane];
+            if (m & SAA_CODED) bits = __ldg(b + i) + *(const uint16_t *)(v + saa_coded_off(n, i, lane));
             else bits = ((const long long *)(v + 256 * i))[lane];
         }
         a[e] = __longlong_as_double(bits);
@@ -340,7 +393,6 @@ __device__ __forceinline__ void saa_node_dot_pipe(const SaaDev &P, int64_t slice
     const int len = (int)((P.slice_ptr[slice + 1] - beg) >> 5);
     const char *vs = (const char *)(P.val + P.val_ptr[slice]);
     const long long *bs = P.vbase + P.vb_ptr[slice];
-    unsigned char *stage = saa_stage();
     const int32_t *c = P.col + beg + lane;
     const uint16_t *mk = P.pmask + (beg >> 5);
     s[0] = 0.0; s[1] = 0.0; s[2] = 0.0;
@@ -370,7 +422,7 @@ __device__ __forceinline__ void saa_node_dot_pipe(const SaaDev &P, int64_t slice
 #pragma unroll
         for (int u = 0; u < UNROLL; ++u) {              // blocks in ascending column order: the order of the CSR row
             double a[9];
-            saa_decode_block(vs, bs, lane, blk[u], stage, a);
+            saa_decode_block(vs, lane, blk[u], a);
             saa_block_madd(a, xv[u], s);
         }
     }
@@ -383,7 +435,7 @@ __device__ __forceinline__ void saa_node_dot_pipe(const SaaDev &P, int64_t slice
             saa_next_block(vo, bo, m[u]);
             saa_gather3<NC_X>(x, k[u], xv);
             SAA_FENCE_BLK(blk);
-            saa_decode_block(vs, bs, lane, blk, stage, a);
+            saa_decode_block(vs, lane, blk, a);
             saa_block_madd(a, xv, s);
         }
 }
@@ -396,7 +448,6 @@ __device__ __forceinline__ void saa_node_dot_simple(const SaaDev &P, int64_t sli
     const int len = (int)((P.slice_ptr[slice + 1] - beg) >> 5);
     const char *vs = (const char *)(P.val + P.val_ptr[slice]);
     const long long *bs = P.vbase + P.vb_ptr[slice];
-    unsigned char *stage = saa_stage();
     const int32_t *c = P.col + beg + lane;
     const uint16_t *mk = P.pmask + (beg >> 5);
     s[0] = 0.0; s[1] = 0.0; s[2] = 0.0;
@@ -419,7 +470,7 @@ __device__ __forceinline__ void saa_node_dot_simple(const SaaDev &P, int64_t sli
         for (int u = 0; u < UNROLL; ++u) {
             double a[9];
             SAA_FENCE_BLK(blk[u]);
-            saa_decode_block(vs, bs, lane, blk[u], stage, a);
+            saa_decode_block(vs, lane, blk[u], a);
             saa_block_madd(a, xv[u], s);
         }
     }
@@ -432,7 +483,7 @@ __device__ __forceinline__ void saa_node_dot_simple(const SaaDev &P, int64_t sli
         saa_next_block(vo, bo, m);
         saa_gather3<NC_X>(x, k, xv);
         SAA_FENCE_BLK(blk);
-        saa_decode_block(vs, bs, lane, blk, stage, a);
+        saa_decode_block(vs, lane, blk, a);
         saa_block_madd(a, xv, s);
     }
 }
