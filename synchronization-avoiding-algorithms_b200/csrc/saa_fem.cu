@@ -1643,7 +1643,7 @@ extern "C" int saa_plan_host_pipe_info(saa_plan *p, int mode, int *n_chunks, int
     const int table = (mode == SAA_MODE_SYNC && p->size > 1) ? 1 : 0;
     if (p->hp[table].state == 0 && host_pipe_build(p, table)) return -1;
     const saa_plan::HostPipe &h = p->hp[table];
-    const int K = h.state == 1 ? (int)h.slice_end.size() : 0;
+    const int K = (h.state == 1 && !p->matfree) ? (int)h.slice_end.size() : 0;   // K5 steps take the plain sequence
     *n_chunks = K;
     if (K > 0 && slice_end && need_upload) {
         if (cap < K) return fail("saa_plan_host_pipe_info: capacity %d < %d chunks", cap, K);
@@ -1987,6 +1987,21 @@ extern "C" int saa_plan_set_matfree_dev(saa_plan *p, int64_t n_elem, const int32
     if (p->d_mf_inc) return fail("saa_plan_set_matfree_dev: already set");
     CK(cudaSetDevice(p->device));
     const int64_t nn_ext = p->n_dof / 3, nn_int = p->n_rows / 3;
+    {   // every kernel below indexes by the node ids and K5 divides by 6 detJ: refuse bad cells before anything changes
+        DevBuf b_first;
+        if (b_first.alloc(2 * sizeof(unsigned long long))) return -1;
+        unsigned long long *first_d = b_first.as<unsigned long long>();
+        CK(cudaMemset(first_d, 0xff, 2 * sizeof(unsigned long long)));
+        saa_k_mf_check_cells<<<nblk(n_elem, 256), 256>>>(n_elem, nn_ext, cells_dev, coords_dev, first_d);
+        CK(cudaGetLastError());
+        unsigned long long first[2] = {0, 0};
+        CK(cudaMemcpy(first, first_d, sizeof first, cudaMemcpyDeviceToHost));
+        if (first[0] != ~0ull)
+            return fail("saa_plan_set_matfree_dev: element %llu has a node id outside [0, %lld)", first[0], (long long)nn_ext);
+        if (first[1] != ~0ull)
+            return fail("saa_plan_set_matfree_dev: element %llu has zero volume (a repeated corner, or 6 detJ of a corner "
+                        "rounds to 0)", first[1]);
+    }
     CK(cudaMalloc((void **)&p->d_mf_cells, 4 * n_elem * sizeof(int32_t)));
     CK(cudaMalloc((void **)&p->d_mf_X, 3 * nn_int * sizeof(double)));
     CK(cudaMemset(p->d_mf_X, 0, 3 * nn_int * sizeof(double)));

@@ -16,10 +16,12 @@
 // is therefore evaluated four times (once per corner); the gathers of the other three corners (coordinates and
 // displacements, 2 x 24 B each) are served by L1/L2.
 //
-// Arithmetic differs from the assembled path by association (K u is summed per element here, per matrix entry there)
-// and uses FMA: results agree with the parity path to ~1e-13 relative per step and drift apart as SURVEY.md §0.5
+// Arithmetic differs from the assembled path by association (K u is summed per element here, per matrix entry there;
+// the library is built with -fmad=false): results agree with the parity path to ~1e-13 relative per step and drift apart as SURVEY.md §0.5
 // describes (measured: tests/test_gpu_matfree.py, bench.py --kernel matfree).  It can therefore not meet the 1e-12
 // history criterion over 10^4 steps and is never used by the parity tests or the default bench line.
+// Accuracy: every row of the force is within a bound counted from the operation sequence below of the exact rational
+// value (oracle/matfree_ref.py, tests/test_gpu_matfree_reference.py); keep a rewrite of this arithmetic inside it.
 #pragma once
 
 struct SaaMatFreeDev {
@@ -122,6 +124,50 @@ __global__ void __launch_bounds__(256, MINB) saa_k_step_matfree(SaaDev P, SaaMat
 }
 
 // ---- set-up kernels -----------------------------------------------------------------------------------------------
+// 6 detJ of the tetrahedron (x0; x1, x2, x3) in the operations of saa_mf_corner_force (the library is built with
+// -fmad=false, so neither side contracts to FMA)
+__device__ __forceinline__ double saa_mf_six_detJ(const double *__restrict__ X, int32_t n0, int32_t n1, int32_t n2, int32_t n3)
+{
+    const int32_t nb[3] = {n1, n2, n3};
+    double e[3][3];
+#pragma unroll
+    for (int b = 0; b < 3; ++b)
+#pragma unroll
+        for (int i = 0; i < 3; ++i) e[b][i] = __dsub_rn(X[3 * (int64_t)nb[b] + i], X[3 * (int64_t)n0 + i]);
+    const double c0 = __dsub_rn(__dmul_rn(e[1][1], e[2][2]), __dmul_rn(e[1][2], e[2][1]));
+    const double c1 = __dsub_rn(__dmul_rn(e[1][2], e[2][0]), __dmul_rn(e[1][0], e[2][2]));
+    const double c2 = __dsub_rn(__dmul_rn(e[1][0], e[2][1]), __dmul_rn(e[1][1], e[2][0]));
+    return __dmul_rn(6.0, __dadd_rn(__dadd_rn(__dmul_rn(e[0][0], c0), __dmul_rn(e[0][1], c1)), __dmul_rn(e[0][2], c2)));
+}
+// the check saa_plan_set_matfree_dev makes before it allocates or indexes anything, one thread per element; keeps the
+// lowest offending element per kind:  first[0] a node id outside [0, n_nodes) (nothing else of that element is read),
+// first[1] zero volume: a repeated corner, or a corner whose factor -1/(6 detJ) in K5 (the four even rotations of
+// saa_k_step_matfree, each with its own rounding of detJ) is not finite.  Negative detJ is accepted: V = detJ/6 is
+// signed in the reference.
+__global__ void saa_k_mf_check_cells(int64_t n_elem, int64_t n_nodes, const int32_t *__restrict__ cells, const double *__restrict__ X,
+                                     unsigned long long *__restrict__ first)
+{
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n_elem) return;
+    int32_t n[4];
+    bool bad_id = false;
+#pragma unroll
+    for (int a = 0; a < 4; ++a) {
+        n[a] = cells[4 * e + a];
+        if (n[a] < 0 || n[a] >= n_nodes) bad_id = true;
+    }
+    if (bad_id) {
+        atomicMin(first, (unsigned long long)e);
+        return;
+    }
+    bool zero = n[0] == n[1] || n[0] == n[2] || n[0] == n[3] || n[1] == n[2] || n[1] == n[3] || n[2] == n[3];
+    // own corner first, by an even permutation: (0123) (1032) (2301) (3210), as saa_k_step_matfree rotates them
+    const double d[4] = {saa_mf_six_detJ(X, n[0], n[1], n[2], n[3]), saa_mf_six_detJ(X, n[1], n[0], n[3], n[2]),
+                         saa_mf_six_detJ(X, n[2], n[3], n[0], n[1]), saa_mf_six_detJ(X, n[3], n[2], n[1], n[0])};
+#pragma unroll
+    for (int a = 0; a < 4; ++a) zero = zero || !isfinite(__ddiv_rn(-1.0, d[a]));
+    if (zero) atomicMin(first + 1, (unsigned long long)e);
+}
 __global__ void saa_k_mf_cells_to_internal(int64_t n4, const int32_t *__restrict__ cells_ext, const int32_t *__restrict__ iperm,
                                            int32_t *__restrict__ cells_int)
 {

@@ -435,10 +435,25 @@ class StepPlan:
     def set_matfree(self, cells_local, coords_local, lmd, mu):
         """Hand the element connectivity (nE,4; local node ids) and the local node coordinates (n,3) to the plan for the
         matrix-free kernel K5 (torch CUDA tensors, or host arrays which are uploaded through torch); enable it with
-        set_option(OPT_MATFREE, 1)."""
+        set_option(OPT_MATFREE, 1).  Refused (SaaError, the plan unchanged): a node id outside [0, n_dof/3), an element with
+        a repeated corner or detJ == 0; negative detJ is accepted (the reference's volume is signed)."""
         import torch
         dev = torch.device("cuda", self.device)
-        c = cells_local if isinstance(cells_local, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(cells_local, dtype=np.int32))
+        nn = self.n_dof // 3
+        # node ids are checked in their own type: the int32 cast below would wrap an id >= 2^31 into range
+        if isinstance(cells_local, torch.Tensor):
+            c = cells_local
+            if c.is_floating_point() or c.is_complex() or c.dtype == torch.bool:
+                raise SaaError(f"set_matfree: cells must hold integer node ids, not {c.dtype}")
+            lo, hi = (int(c.min()), int(c.max())) if c.numel() else (0, 0)
+        else:
+            a = np.asarray(cells_local)
+            if not np.issubdtype(a.dtype, np.integer):
+                raise SaaError(f"set_matfree: cells must hold integer node ids, not {a.dtype}")
+            lo, hi = (int(a.min()), int(a.max())) if a.size else (0, 0)
+            c = torch.from_numpy(np.ascontiguousarray(a.astype(np.int64)))
+        if lo < 0 or hi >= nn:
+            raise SaaError(f"set_matfree: node id {lo if lo < 0 else hi} outside [0, {nn})")
         x = coords_local if isinstance(coords_local, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(coords_local, dtype=np.float64))
         c = c.to(device=dev, dtype=torch.int32).contiguous()
         x = x.to(device=dev, dtype=torch.float64).contiguous()
